@@ -2,6 +2,7 @@
 """bench.py -- throughput of the fused ramp + format-convert path on N B200s (one process per GPU).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                         # + what the last timed step computed, as DIR/*.npy
     python bench.py --impl reference [--gpus N] --steps K --warmup W  # the reference's own CPU code (oracle/_ref)
 
 A "step" is one pass of the hot path over one batch: BASELINE.json configs[1] by default (1024 streams, stereo,
@@ -388,6 +389,23 @@ class DeviceRun:
         ok = bool(ok_sizes and np.array_equal(sums[picks], want))
         return sums, ok, len(picks), kind
 
+    def dump_outputs(self, out_dir, sums, n_windows=256, window=4096):
+        """Write what the last step left in the output arena, so that two builds can be compared output for output:
+        output_sample.npy          n_windows x window output bytes (float32) at offsets drawn with a fixed seed,
+        output_sample_offsets.npy  those offsets (float64),
+        stream_checksums.npy       every stream's checksum of its whole output range, as (high, low) 32-bit halves
+                                   (float64 holds both exactly).
+        A few MB in all, whatever the workload's size."""
+        os.makedirs(out_dir, exist_ok=True)
+        n = self.w.out_bytes
+        window = min(window, n)
+        offs = np.sort(np.random.default_rng(0).integers(0, n - window + 1, size=n_windows))
+        sample = self.torch.stack([self.d_out[o:o + window] for o in offs.tolist()]).cpu().numpy()
+        np.save(os.path.join(out_dir, "output_sample.npy"), sample.astype(np.float32))
+        np.save(os.path.join(out_dir, "output_sample_offsets.npy"), offs.astype(np.float64))
+        halves = np.stack([sums >> np.uint64(32), sums & np.uint64(0xFFFFFFFF)], axis=1)
+        np.save(os.path.join(out_dir, "stream_checksums.npy"), halves.astype(np.float64))
+
     def free(self):
         for name in ("d_specs", "d_events", "d_in", "d_out", "d_begin", "d_outb", "d_desc", "d_off"):
             if hasattr(self, name):
@@ -399,7 +417,7 @@ def main():
     claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of the headline measurement (at least 1)")
     ap.add_argument("--warmup", type=int, default=4)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="", help="experiments: run this workload alone as the timed one (default: config2 + the configs array)")
@@ -413,7 +431,14 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=0, help="default: min(steps, 5)")
     ap.add_argument("--e2e-api", default="run_streams_host", choices=["run_streams_host", "process_host"])
     ap.add_argument("--chunk-frames", type=int, default=0, help="experiment: override the workload's frames per message")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write a seeded sample of the last step's output and every stream's "
+                         "checksum to DIR/*.npy (rank 0's batch)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; the reference arm has nothing of it to write")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -522,6 +547,8 @@ def main():
 
     # what was just computed, on every rank, against the reference's own code on the same bytes
     sums, ok, n_checked, check_kind = (run.checksums(), None, 0, "skipped") if args.no_check else run.check_against_reference(args.check_streams, check_threads)
+    if args.dump_outputs and rank == 0:
+        run.dump_outputs(args.dump_outputs, sums)  # before the from-specs leg below writes the arena again
     all_sums = sharding.gather_checksums(sums, len(sums) * world, world, rank, dist)
     checksum_of_checksums = int(np.bitwise_xor.reduce(all_sums)) if len(all_sums) else 0
     main_bit_exact = None if args.no_check else all_ranks(ok)

@@ -41,6 +41,45 @@ def test_our_arm_refuses_to_run_without_a_gpu():
     assert "no CUDA device" in r.stderr or "no CPU fallback" in r.stderr
 
 
+@pytest.mark.gpu
+def test_dump_outputs_holds_what_the_timed_step_computed(tmp_path):
+    """--steps sets the number of timed launches, and --dump-outputs writes float arrays that a second run with the same
+    arguments reproduces exactly: a sample of the output arena that is the C port's output at the same offsets, and
+    every stream's checksum."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from oracle import pyoracle
+    dumps = []
+    for i in range(2):
+        d = tmp_path / str(i)
+        r = run_bench("--steps", "3", "--warmup", "4", "--streams", "8", "--seconds", "0.1", "--no-configs", "--no-e2e",
+                      "--no-cpu-baseline", "--dump-outputs", str(d))
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads(r.stdout)
+        assert line["steps"] == 3 and line["gpu_launches"] == 3 and line["bit_exact"] is True
+        files = sorted(d.glob("*.npy"))
+        assert sum(f.stat().st_size for f in files) <= 64 << 20
+        dumps.append({f.name: np.load(f) for f in files})
+    assert sorted(dumps[0]) == ["output_sample.npy", "output_sample_offsets.npy", "stream_checksums.npy"]
+    for name, a in dumps[0].items():
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, dumps[1][name]), name
+    w = bench.build_workload("config2", 8, 0.1)
+    port = pyoracle.Port()
+    inp = port.fill_streams(w.streams, w.in_bytes, bench.seed_base("config2"), 0)
+    rc, want = port.run(w.streams, w.events, inp, w.out_bytes)[:2]
+    assert rc == 0
+    # a stream's checksum covers its range of the arena: from its dst_base to the next stream's
+    edges = np.concatenate([w.streams["dst_base"], [w.out_bytes]]).astype(np.int64)
+    halves = dumps[0]["stream_checksums.npy"].astype(np.uint64)
+    assert halves.shape == (len(w.streams), 2)
+    got = (halves[:, 0] << np.uint64(32)) | halves[:, 1]
+    assert [int(x) for x in got] == [port.checksum(want[edges[s]:edges[s + 1]]) for s in range(len(w.streams))]
+    sample, offs = dumps[0]["output_sample.npy"], dumps[0]["output_sample_offsets.npy"].astype(np.int64)
+    for row, o in zip(sample, offs):
+        assert np.array_equal(row, want[o:o + len(row)]), o
+
+
 def test_the_bench_check_agrees_with_the_port_on_a_mixed_batch():
     """bench.py compares each rank's per-stream checksums with the reference's own code run on a sample of streams fed the
     per-stream seeded bytes.  Here the C port stands in for the GPU (same arena layout, same fill, same checksum ranges):
