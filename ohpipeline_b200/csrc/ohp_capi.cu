@@ -175,6 +175,7 @@ class RangeSet
 {
 public:
     static constexpr uint64_t kBridge = 4096;
+    explicit RangeSet(uint64_t bridge = kBridge) : iBridge(bridge) {} // 0: no hole is bridged
     void Add(uint64_t off, uint64_t len)
     {
         if (len == 0) return;
@@ -182,8 +183,8 @@ public:
         if (!iRanges.empty() && off < iRanges.back().hi) iSorted = false;
         iRanges.push_back(Range{off, off + len});
     }
-    // Sort and merge what was added; f(lo, hi) for every maximal covered range, g(lo, hi) for every hole <= kBridge
-    // between two of them (which is then bridged: the ranges either side reach f as one).
+    // Sort and merge what was added; f(lo, hi) for every maximal covered range, g(lo, hi) for every hole <= the bridge
+    // limit between two of them (which is then bridged: the ranges either side reach f as one).
     template <class F, class G>
     void Merge(F f, G g)
     {
@@ -193,7 +194,7 @@ public:
         for (size_t i = 1; i < iRanges.size(); i++) {
             const Range& r = iRanges[i];
             if (r.lo <= hi) { hi = r.hi > hi ? r.hi : hi; continue; }
-            if (r.lo - hi <= kBridge) { g(hi, r.lo); hi = r.hi; continue; }
+            if (r.lo - hi <= iBridge) { g(hi, r.lo); hi = r.hi; continue; }
             f(lo, hi);
             lo = r.lo; hi = r.hi;
         }
@@ -205,12 +206,13 @@ private:
     struct Range { uint64_t lo, hi; };
     std::vector<Range> iRanges;
     bool iSorted = true;
+    uint64_t iBridge;
 };
 
 class CopyBackPlan
 {
 public:
-    explicit CopyBackPlan(uint8_t* h_out) : iOut(h_out) {}
+    explicit CopyBackPlan(uint8_t* h_out, uint64_t bridge = RangeSet::kBridge) : iOut(h_out), iBatch(bridge), iSlice(bridge) {}
     ~CopyBackPlan() { Restore(); }
     RangeSet& Batch() { return iBatch; }   // every range the whole call covers ...
     void SaveHoles()                       // ... then, before the first copy is issued
@@ -967,11 +969,17 @@ int ohp_schedule_emit_device(ohp_context* ctx, const ohp_stream_spec* d_streams,
     return OHP_OK;
 }
 
-// The whole stage for a batch of streams in HOST memory (include/ohp_schedule_device.h).
-int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, size_t n_streams,
-                         const ohp_ramp_event* h_events, size_t n_events,
-                         const uint8_t* h_in, uint64_t in_bytes, uint8_t* h_out, uint64_t out_bytes,
-                         uint64_t* h_stream_out_bytes, uint64_t* total_chunks)
+} // extern "C"
+
+namespace ohp {
+
+// The whole stage for a batch of streams in HOST memory (include/ohp_schedule_device.h).  Holes of up to `bridge` bytes
+// between the streams' output ranges go back with the ranges around them and get the caller's bytes back at the end
+// (CopyBackPlan): that is only right where nothing else writes into h_out while the call runs.
+static int run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, size_t n_streams,
+                            const ohp_ramp_event* h_events, size_t n_events,
+                            const uint8_t* h_in, uint64_t in_bytes, uint8_t* h_out, uint64_t out_bytes,
+                            uint64_t* h_stream_out_bytes, uint64_t* total_chunks, uint64_t bridge)
 {
     if (!ctx) return OHP_E_INVALID_ARG;
     if (total_chunks) *total_chunks = 0;
@@ -1027,7 +1035,7 @@ int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, siz
         return cudaSuccess;
     };
     const SliceMode slice_mode(ctx);
-    CopyBackPlan plan(h_out); // a stream's chunks tile [dst_base, dst_base + its output bytes): one range per stream
+    CopyBackPlan plan(h_out, bridge); // a stream's chunks tile [dst_base, dst_base + its output bytes): one range per stream
     const DrainOnExit drain(ctx, st);
     for (size_t s = 0; s < n_streams; s++) plan.Batch().Add(h_streams[s].dst_base, ctx->h_outb[s]);
     plan.SaveHoles();
@@ -1069,6 +1077,19 @@ int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, siz
     OHP_CUDA(ctx, cudaStreamSynchronize(st));
     if (rc != OHP_OK) return rc;
     return read_status(ctx, st);
+}
+
+} // namespace ohp
+
+extern "C" {
+
+int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, size_t n_streams,
+                         const ohp_ramp_event* h_events, size_t n_events,
+                         const uint8_t* h_in, uint64_t in_bytes, uint8_t* h_out, uint64_t out_bytes,
+                         uint64_t* h_stream_out_bytes, uint64_t* total_chunks)
+{
+    return run_streams_host(ctx, h_streams, n_streams, h_events, n_events, h_in, in_bytes, h_out, out_bytes,
+                            h_stream_out_bytes, total_chunks, RangeSet::kBridge);
 }
 
 // The whole stage for a batch resident in HBM (include/ohp_schedule_device.h).

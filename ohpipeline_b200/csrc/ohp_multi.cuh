@@ -120,11 +120,21 @@ static int multi_run_block(MultiWorker& w, const MultiJob& j, size_t n_devices)
         const uint64_t at = j.streams[s].dst_base;
         if (at > out_last && at < out_hi) out_hi = at;
     }
+    // The host call bridges small holes between the block's output ranges: it copies the device's bytes over them and
+    // puts back, when it ends, what they held when it began.  Where another block's stream begins inside the block's
+    // span, that stream may be written into such a hole in the meantime, and putting the hole back would undo it: such a
+    // block copies its ranges back one by one.
+    bool foreign_inside = false;
+    for (size_t s = 0; s < j.n_streams && !foreign_inside; s++) {
+        if (s >= first && s < first + count) continue;
+        const uint64_t at = j.streams[s].dst_base;
+        foreign_inside = at >= out_lo && at < out_hi;
+    }
     w.outb.assign(count, 0);
     uint64_t chunks = 0;
-    const int rc = ohp_run_streams_host(w.ctx, w.specs.data(), count, j.events ? j.events + ev_lo : nullptr, (size_t)(ev_hi - ev_lo),
-                                        j.h_in + in_lo, in_hi - in_lo, j.h_out + out_lo, out_hi - out_lo,
-                                        w.outb.data(), &chunks);
+    const int rc = run_streams_host(w.ctx, w.specs.data(), count, j.events ? j.events + ev_lo : nullptr, (size_t)(ev_hi - ev_lo),
+                                    j.h_in + in_lo, in_hi - in_lo, j.h_out + out_lo, out_hi - out_lo,
+                                    w.outb.data(), &chunks, foreign_inside ? 0 : RangeSet::kBridge);
     if (rc != OHP_OK) {
         // the call names streams by their place in the block
         return multi_fail(w, rc, std::string(ohp_last_error(w.ctx)) + " (streams counted from " + std::to_string(first) + ")");

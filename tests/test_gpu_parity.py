@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 from ohpipeline_b200 import abi, capi, workloads as W
-from util import covered_mask, describe_first_diff, make_desc, pack_chunks
+from util import alignment_specs, covered_mask, describe_first_diff, make_desc, pack_chunks
 
 pytestmark = pytest.mark.gpu
 
@@ -130,17 +130,7 @@ def test_mixed_covers_the_interesting_chunk_kinds(port):
 @pytest.mark.parametrize("le", [False, True])
 def test_every_alignment_of_source_and_destination(ctx, port, bits, le):
     """Chunks at every src/dst byte offset mod 16 (a split playable starts wherever the ramp ended)."""
-    b = bits // 8
-    specs = []
-    rng = np.random.default_rng(bits + le)
-    for k in range(64):
-        ch = int(rng.integers(1, 9))
-        frames = int(rng.integers(1, 40))
-        specs.append(dict(bytes=frames * ch * b, bit_depth=bits, channels=ch,
-                          flags=(abi.F_RAMP_ENABLED if k % 3 else 0) | (abi.F_IN_LITTLE_ENDIAN if le else 0),
-                          ramp_start=int(rng.integers(0, 16385)), ramp_end=int(rng.integers(0, 16385)),
-                          src_pad=int(rng.integers(0, 5)), dst_pad=int(rng.integers(0, 5))))
-    descs, in_bytes, out_bytes = pack_chunks(specs)
+    descs, in_bytes, out_bytes = pack_chunks(alignment_specs(bits, le))
     inp = port.fill_pcm(in_bytes, 99 + bits)
     want = oracle_out(port, descs, inp, out_bytes)
     got = run_device(ctx, descs, inp, out_bytes)
@@ -515,28 +505,34 @@ def test_converting_sinks_reject_what_the_reference_asserts_on(ctx):
 
 def test_inflight_tuning_never_changes_results(ctx, port):
     """Large batches are tuned: the first launches of a batch shape each keep a different number of chunks in flight
-    (ohp_inflight_cap).  Every launch must produce the same bytes, and those are the oracle's."""
+    (ohp_inflight_cap).  Every launch must produce the same bytes, and those are the oracle's.  Two batch shapes: uniform
+    stereo 24-bit, and mixed formats shaped like a pipeline's output."""
+    for w in (W.config5(n_streams=1024, seconds=0.4), W.config4(n_streams=760, seconds=0.25, seed=7)):
+        check_tuned_launches(ctx, port, w)
+
+
+def check_tuned_launches(ctx, port, w):
     import torch
-    w = W.config5(n_streams=1024, seconds=0.4)
     sched = capi.schedule_build(w.streams, w.events)
-    assert len(sched.chunks) >= 65536 and w.in_bytes + w.out_bytes >= (256 << 20)
+    assert len(sched.chunks) >= 65536 and w.in_bytes + w.out_bytes >= (256 << 20), w.name
     inp = port.fill_pcm(w.in_bytes, w.seed)
     d_desc = torch.from_numpy(sched.chunks.view(np.uint8).copy()).cuda()
     d_in = torch.from_numpy(inp).cuda()
     stream = torch.cuda.Stream()
     st = stream.cuda_stream
-    caps, outs = [], []
-    for _ in range(7):
+    caps, first = [], None
+    for launch in range(7):
         d_out = torch.zeros(w.out_bytes, dtype=torch.uint8, device="cuda")
         torch.cuda.synchronize()
         ctx.process_device(d_desc.data_ptr(), len(sched.chunks), d_in.data_ptr(), w.in_bytes, d_out.data_ptr(), w.out_bytes, st)
         ctx.sync(st)
         caps.append(ctx.inflight_cap())
-        outs.append(d_out)
-    assert len(set(caps[:3])) == 3, caps           # three candidates explored ...
-    assert caps[4] == caps[5] == caps[6]           # ... (the first one again, warm, if it was close) then the fastest is kept
-    for o in outs[1:]:
-        assert torch.equal(o, outs[0])
+        if first is None:
+            first = d_out
+        else:
+            assert torch.equal(d_out, first), (w.name, launch, caps)
+    assert len(set(caps[:3])) == 3, (w.name, caps)           # three candidates explored ...
+    assert caps[4] == caps[5] == caps[6], (w.name, caps)     # ... (the first one again, warm, if it was close) then the fastest is kept
     # the first 24 streams against the oracle
     k = int(sched.stream_chunk_begin[24])
     sub = sched.chunks[:k]
@@ -544,4 +540,4 @@ def test_inflight_tuning_never_changes_results(ctx, port):
     rc, want = port.process_chunks(sub, inp, hi)
     assert rc == 0
     mask = covered_mask(sub, hi)
-    assert np.array_equal(outs[0][:hi].cpu().numpy()[mask], want[mask])
+    assert np.array_equal(first[:hi].cpu().numpy()[mask], want[mask]), w.name

@@ -52,6 +52,22 @@ def pack_chunks(chunk_specs, align=1, rng=None):
     return descs, src + 64, dst + 64
 
 
+def alignment_specs(bits, le):
+    """64 chunks of `bits`-bit audio, 1-8 channels, 1-39 frames, ramped or not, at every src/dst byte offset mod 16
+    (pack_chunks specs: a split playable starts wherever the ramp ended)."""
+    b = bits // 8
+    specs = []
+    rng = np.random.default_rng(bits + le)
+    for k in range(64):
+        ch = int(rng.integers(1, 9))
+        frames = int(rng.integers(1, 40))
+        specs.append(dict(bytes=frames * ch * b, bit_depth=bits, channels=ch,
+                          flags=(abi.F_RAMP_ENABLED if k % 3 else 0) | (abi.F_IN_LITTLE_ENDIAN if le else 0),
+                          ramp_start=int(rng.integers(0, 16385)), ramp_end=int(rng.integers(0, 16385)),
+                          src_pad=int(rng.integers(0, 5)), dst_pad=int(rng.integers(0, 5))))
+    return specs
+
+
 def covered_mask(descs, out_bytes):
     """Boolean mask of the output bytes some chunk writes (planar output is strided per channel)."""
     mask = np.zeros(out_bytes, dtype=bool)
