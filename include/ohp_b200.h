@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define OHP_ABI_VERSION 2u
+#define OHP_ABI_VERSION 3u
 
 /* Ramp::kMax / Ramp::kMin (Msg.h:257-258) */
 #define OHP_RAMP_MAX 16384u

@@ -113,11 +113,6 @@ int    ohp_schedule_build(const ohp_stream_spec* streams, size_t n_streams,
 int    ohp_schedule_build_walk(const ohp_stream_spec* streams, size_t n_streams,
                                const ohp_ramp_event* events, size_t n_events,
                                int threads, ohp_schedule** out);
-/* The same walk taken in n_stretches stretches per stream, stopping and resuming where ohp_run_streams_device does
- * (it walks a stretch while ramp_convert_kernel works on the one before): the result must not depend on n_stretches. */
-int    ohp_schedule_build_walk_stretches(const ohp_stream_spec* streams, size_t n_streams,
-                                         const ohp_ramp_event* events, size_t n_events,
-                                         int threads, uint32_t n_stretches, ohp_schedule** out);
 /* The closed-form upper bound on each stream's playables that ohp_run_streams_device sizes its descriptor regions with
  * (one walk per stream instead of count + emit); bounds[s] = 0 for a stream the walk refuses.  Exported so that the CPU
  * suite can hold it against the exact counts. */

@@ -73,8 +73,7 @@ int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, siz
  *     stream ever have more playables than its region holds (none of this repo's generators produces one; the bound is
  *     held against exact counts in the tests) -- redo the batch through count + emit.  Without it that case is an
  *     OHP_E_NO_MEMORY from the next ohp_sync.
- * One call at a time per context.  Environment (experiments, tests): OHP_STRETCHES=k walks every stream in k stretches of
- * time, resumable (the form for audio that arrives a window at a time; DESIGN 4.2); OHP_ONE_WALK=0 takes count + scan + emit.
+ * One call at a time per context.  Environment (tests): OHP_ONE_WALK=0 takes count + scan + emit.
  * Errors as ohp_run_streams_host.
  */
 int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,

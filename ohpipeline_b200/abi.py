@@ -5,7 +5,7 @@ headers exactly -- tests/test_abi.py checks sizeof/offsetof against the built li
 """
 import numpy as np
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 RAMP_MAX = 16384          # Ramp::kMax, OpenHome/Media/Pipeline/Msg.h:257
 RAMP_MIN = 0

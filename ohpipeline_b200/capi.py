@@ -170,9 +170,6 @@ def host_lib():
         L.ohp_flywheel_batch_arena_bytes.argtypes = [C.c_void_p, C.POINTER(C.c_uint64)]
         L.ohp_flywheel_batch_free.restype = None
         L.ohp_flywheel_batch_free.argtypes = [C.c_void_p]
-        L.ohp_schedule_build_walk_stretches.restype = C.c_int
-        L.ohp_schedule_build_walk_stretches.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_int, C.c_uint32,
-                                                        C.POINTER(C.c_void_p)]
         L.ohp_flywheel_ramp_chunks.restype = C.c_int
         L.ohp_flywheel_ramp_chunks.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint64, C.c_void_p, C.c_size_t,
                                                C.POINTER(C.c_uint32)]
@@ -368,20 +365,16 @@ class Schedule:
         return self.recent[int(self.recent_begin[k]):int(self.recent_begin[k + 1])]
 
 
-def schedule_build(streams, events, threads=0, walk=False, stretches=None):
+def schedule_build(streams, events, threads=0, walk=False):
     """Run the ramp events of every stream through the stage chain; returns a Schedule.
     Raises OhpError(E_INVALID_DESC) where the reference would ASSERT.
-    walk=True: the class-free walk (ohp_schedule_build_walk), the source the GPU schedule kernels compile;
-    stretches=k: that walk stopped and resumed k - 1 times per stream (ohp_schedule_build_walk_stretches)."""
+    walk=True: the class-free walk (ohp_schedule_build_walk), the source the GPU schedule kernels compile."""
     L = host_lib()
     streams = np.ascontiguousarray(streams, dtype=abi.STREAM_SPEC)
     events = np.ascontiguousarray(events, dtype=abi.RAMP_EVENT)
     h = C.c_void_p()
-    if stretches is not None:
-        rc = L.ohp_schedule_build_walk_stretches(_ptr(streams), len(streams), _ptr(events), len(events), threads, int(stretches), C.byref(h))
-    else:
-        build = L.ohp_schedule_build_walk if walk else L.ohp_schedule_build
-        rc = build(_ptr(streams), len(streams), _ptr(events), len(events), threads, C.byref(h))
+    build = L.ohp_schedule_build_walk if walk else L.ohp_schedule_build
+    rc = build(_ptr(streams), len(streams), _ptr(events), len(events), threads, C.byref(h))
     if rc != 0:
         raise OhpError(rc, L.ohp_schedule_last_error().decode())
     try:

@@ -82,12 +82,8 @@ struct ohp_context
     uint64_t* d_begin = nullptr; uint64_t d_begin_cap = 0;
     uint64_t* d_outb = nullptr; uint64_t d_outb_cap = 0;
     uint64_t* d_counts = nullptr; uint64_t d_counts_cap = 0;  // ohp_run_streams_device: exact playables per stream
-    cudaStream_t sched_stream = nullptr;                         // ... the walks run here, beside ramp_convert_kernel
-    std::vector<cudaEvent_t> sched_events;
-    ohp::sched::WalkState* d_walk[2] = {nullptr, nullptr};       // ... where every stream's walk stopped, ping-pong between stretches
-    uint64_t d_walk_cap[2] = {0, 0};
-    uint64_t* d_bases = nullptr;                                 // ... [kMaxStretches + 1] descriptors in front of each stretch
-    uint64_t* h_bases = nullptr;                                 // pinned copy
+    cudaEvent_t sched_event = nullptr;                           // ... recorded behind a copy the host waits for
+    uint64_t* h_regions = nullptr;                               // ... the regions' total (pinned)
     std::vector<uint64_t> h_begin, h_outb;
     cudaEvent_t ev_start = nullptr, ev_stop = nullptr;
     bool timing = false;
@@ -114,8 +110,6 @@ namespace ohp {
 // per stream beyond: with more warps than that the walks go in waves and the 32-fold redundant general path is paid in
 // issue slots (round 2, configs[2]: 2.97 -> 2.80 ms specs-to-bytes, configs[3]: 5.96 -> 4.47 ms; profiles/README.md).
 constexpr size_t kScheduleWarpTeamMaxStreams = 2048;
-constexpr uint32_t kMaxStretches = 16;
-constexpr uint32_t kDefaultStretches = 0; // the one-walk path; see run_streams_device_stretched for why
 
 static int fail(ohp_context* ctx, int status, const char* what, cudaError_t e = cudaSuccess)
 {
@@ -593,10 +587,7 @@ int ohp_create(int device, ohp_context** out_ctx)
     } while (0)
     OHP_CREATE(cudaSetDevice(device));
     {
-        // the compute stream outranks the schedule stream (created on first use, lowest priority): when a stretch's
-        // ramp_convert_kernel and the next stretch's walk become runnable together, the persistent kernel's CTAs are placed
-        // first and the walk takes the registers that are left (one of its CTAs per SM) -- the other way round two walk CTAs
-        // per SM leave room for only one of ramp_convert_kernel's, for as long as there are walks (ohp_run_streams_device)
+        // the compute stream at the device's greatest priority: the walk and kernel times of DESIGN 4 were measured so
         int least = 0, greatest = 0;
         OHP_CREATE(cudaDeviceGetStreamPriorityRange(&least, &greatest));
         OHP_CREATE(cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, greatest));
@@ -622,10 +613,9 @@ int ohp_create(int device, ohp_context** out_ctx)
         int per_sm = 0;
         OHP_CREATE(cudaFuncSetAttribute(ramp_convert_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SharedStorage)));
         OHP_CREATE(cudaFuncSetAttribute(ramp_convert_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SharedStorage)));
-        // The schedule kernels run BESIDE ramp_convert_kernel (ohp_run_streams_device walks stretch k + 1 while stretch k is
-        // being converted).  They use no shared memory, and by default ask for the L1-heavy split of an SM's 256 KB; an SM
-        // cannot change its split while CTAs are resident, so their CTAs would wait for ramp_convert_kernel's persistent
-        // CTAs to finish -- for the whole kernel.  Asking for the same split lets them in.
+        // The schedule and scan kernels need (next to) no shared memory and would get the L1-heavy split of an SM's 256 KB;
+        // they ask for ramp_convert_kernel's split instead (an SM cannot change its split while CTAs are resident).  The
+        // walk times of DESIGN 4.2 were measured so.
         OHP_CREATE(cudaFuncSetAttribute(sched::schedule_kernel<false, 32>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(sched::schedule_kernel<true, 32>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(sched::schedule_kernel<false, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -659,12 +649,8 @@ int ohp_destroy(ohp_context* ctx)
     if (ctx->d_begin) (void)cudaFree(ctx->d_begin);
     if (ctx->d_outb) (void)cudaFree(ctx->d_outb);
     if (ctx->d_counts) (void)cudaFree(ctx->d_counts);
-    if (ctx->d_walk[0]) (void)cudaFree(ctx->d_walk[0]);
-    if (ctx->d_walk[1]) (void)cudaFree(ctx->d_walk[1]);
-    if (ctx->d_bases) (void)cudaFree(ctx->d_bases);
-    if (ctx->h_bases) (void)cudaFreeHost(ctx->h_bases);
-    if (ctx->sched_stream) { (void)cudaStreamSynchronize(ctx->sched_stream); (void)cudaStreamDestroy(ctx->sched_stream); }
-    for (cudaEvent_t e : ctx->sched_events) (void)cudaEventDestroy(e);
+    if (ctx->h_regions) (void)cudaFreeHost(ctx->h_regions);
+    if (ctx->sched_event) (void)cudaEventDestroy(ctx->sched_event);
     if (ctx->h_status) (void)cudaFreeHost(ctx->h_status);
     if (ctx->ev_start) (void)cudaEventDestroy(ctx->ev_start);
     if (ctx->ev_stop) (void)cudaEventDestroy(ctx->ev_stop);
@@ -1098,11 +1084,6 @@ int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, siz
 // descriptor buffer, the walk writes what the stream has and zero-fills the rest of its region (a zero-byte descriptor is
 // a playable MsgPlayable::Read does nothing for, and costs ramp_convert_kernel a record and a ticket).  No count pass, and
 // the only host round trip is for the regions' total (bound + scan are a few microseconds of GPU time).
-// The batch CAN go in slices of streams (OHP_SLICE_CHUNKS=<descriptors per slice>): ramp_convert_kernel on slice k on the
-// caller's stream while the walk of slice k + 1 runs beside it on the context's schedule stream.  Measured (round 2,
-// profiles/README.md) that loses: a walk takes as long as its longest stream whatever the number of streams (the ramp
-// recurrence is sequential; 1024 or 256 streams of configs[1] both take 0.65 ms), so slicing by streams multiplies the
-// walk time it was meant to hide (configs[1]: 5.07 ms in 4 slices against 4.3 in one).  Default: one slice.
 // A stream that outgrows its region (none of the shapes this repo generates does, the bound is held against the exact
 // counts in tests/test_schedule_walk.py) sends the whole call through the two-pass path.
 static int run_streams_device_two_pass(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
@@ -1121,167 +1102,6 @@ static int run_streams_device_two_pass(ohp_context* ctx, const ohp_stream_spec* 
     }
     if ((rc = ohp_schedule_emit_device(ctx, d_streams, n_streams, d_events, n_events, ctx->d_begin, ctx->d_descs, nullptr, st)) != OHP_OK) return rc;
     return launch(ctx, ctx->d_descs, (size_t)total, d_in, in_bytes, d_out, out_bytes, st);
-}
-
-// THE WALK IN STRETCHES (OHP_STRETCHES=k; not the default).  A stream's walk is a chain of dependent steps -- it takes as
-// long as the stream is long however many streams there are -- so the way to hide it behind ramp_convert_kernel is not to
-// slice the batch by streams but by TIME: every stream is walked a stretch of its length at a time
-// (sched::stretch_stop_frame), the walks leave their state in HBM between stretches (sched::WalkState), and
-// ramp_convert_kernel runs on stretch k while stretch k + 1 is walked on the schedule stream.  Each stretch is count +
-// scan + emit (the exact two passes: descriptors compact, no padding), laid out behind the previous stretch's by a base
-// the scan carries forward on the device; the host only waits for each stretch's total to size the launch.
-//
-// It works -- same bytes for any number of stretches (tests/test_gpu_schedule.py), and a caller that gets its audio a
-// window at a time can use the resumable walk for exactly that -- but it does NOT overlap, and so it is slower than the
-// one-walk path (configs[1]: 4.6 ms in 4 stretches, 4.8 in 8, against 4.1).  OHP_STRETCH_TRACE=1 prints the device
-// timeline that shows why (profiles/README.md, GPU calls 16-18): every CTA of a walk enqueued beside ramp_convert_kernel
-// starts within 27 us of the others, AFTER that kernel has ended.  The walk's CTAs find no room: an SM's register file is
-// four sub-partition files of 16 K registers, ramp_convert_kernel's two persistent CTAs put 18 warps of 2304 registers
-// on them (6 + 4 + 4 + 4 or 5 + 5 + 4 + 4), and a 168-register walk warp (5376) does not fit the fuller ones, so a
-// four-warp CTA can not be placed (the SM-wide sum, 41472 + 21504 of 65536, would fit).  Neither the shared-memory split,
-// nor stream priorities, nor a 96-register walk (spills; and 6 warps of 2304 leave 2560) changed that.  What would: eight
-// or twelve warps per ramp_convert CTA (an even load on the sub-partitions), at a cost on the hot path this repo has measured
-// before (0.92 against 0.99 on configs[1]); or a walk of 80 registers.
-static int run_streams_device_stretched(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
-                                        const ohp_ramp_event* d_events, size_t n_events,
-                                        const uint8_t* d_in, uint64_t in_bytes, uint8_t* d_out, uint64_t out_bytes,
-                                        uint64_t* d_stream_out_bytes, uint64_t* total_chunks, uint32_t n_stretches, cudaStream_t st,
-                                        bool* overflowed)
-{
-    int rc;
-    *overflowed = false;
-    // room for the descriptors: the closed-form bound, summed on the device (the one host round trip up front)
-    sched::bound_kernel<<<(unsigned)((n_streams + 127) / 128), 128, 0, st>>>(d_streams, n_streams, d_events, n_events, ctx->d_begin);
-    OHP_CUDA(ctx, cudaGetLastError());
-    sched::scan_kernel<<<1, sched::kScanThreads, 0, st>>>(ctx->d_begin, n_streams);
-    OHP_CUDA(ctx, cudaGetLastError());
-    ctx->launches += 2;
-    if (!ctx->h_bases) OHP_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void**>(&ctx->h_bases), (kMaxStretches + 2) * sizeof(uint64_t), cudaHostAllocDefault));
-    if (!ctx->d_bases) OHP_CUDA(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->d_bases), (kMaxStretches + 1) * sizeof(uint64_t)));
-    OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_bases + kMaxStretches + 1, ctx->d_begin + n_streams, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    OHP_CUDA(ctx, cudaMemsetAsync(ctx->d_bases, 0, sizeof(uint64_t), st));
-    OHP_CUDA(ctx, cudaStreamSynchronize(st));
-    const uint64_t room = ctx->h_bases[kMaxStretches + 1];
-    if (room > ctx->d_descs_cap / sizeof(ohp_chunk_desc)) {
-        OHP_CUDA(ctx, cudaDeviceSynchronize()); // the buffer may still be read by a launch enqueued earlier on another stream
-        if ((rc = grow(ctx, ctx->d_descs, ctx->d_descs_cap, room * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
-    }
-    for (int k = 0; k < 2; k++) {
-        if ((rc = grow(ctx, ctx->d_walk[k], ctx->d_walk_cap[k], (uint64_t)n_streams * sizeof(sched::WalkState))) != OHP_OK) return rc;
-    }
-    while (ctx->sched_events.size() < 2 * (size_t)n_stretches + 1) {
-        cudaEvent_t e;
-        OHP_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        ctx->sched_events.push_back(e);
-    }
-    if (!ctx->sched_stream) {
-        int least = 0, greatest = 0;
-        OHP_CUDA(ctx, cudaDeviceGetStreamPriorityRange(&least, &greatest));
-        OHP_CUDA(ctx, cudaStreamCreateWithPriority(&ctx->sched_stream, cudaStreamNonBlocking, least));
-    }
-    // the schedule stream starts behind whatever the caller's stream holds so far (specs, events and PCM may just have arrived)
-    OHP_CUDA(ctx, cudaEventRecord(ctx->sched_events[2 * n_stretches], st));
-    OHP_CUDA(ctx, cudaStreamWaitEvent(ctx->sched_stream, ctx->sched_events[2 * n_stretches], 0));
-    const int team = schedule_team(n_streams);
-    const unsigned grid = sched::schedule_grid(n_streams, team);
-    // OHP_STRETCH_TRACE=1 (experiments): when each piece started and ended on the device, printed to stderr
-    static const bool trace = std::getenv("OHP_STRETCH_TRACE") != nullptr;
-    std::vector<std::pair<std::string, cudaEvent_t>> marks;
-    auto mark = [&](const char* what, uint32_t j, cudaStream_t on) {
-        if (!trace) return;
-        cudaEvent_t e;
-        if (cudaEventCreate(&e) != cudaSuccess) return;
-        (void)cudaEventRecord(e, on);
-        marks.emplace_back(std::string(what) + " " + std::to_string(j), e);
-    };
-    mark("start", 0, st);
-    uint64_t* d_timeline = nullptr; // of stretch 1's count pass, the first walk that runs beside ramp_convert_kernel
-    if (trace && n_stretches > 1) {
-        if (cudaMalloc(reinterpret_cast<void**>(&d_timeline), (size_t)grid * 3 * sizeof(uint64_t)) != cudaSuccess) d_timeline = nullptr;
-        else (void)cudaMemset(d_timeline, 0, (size_t)grid * 3 * sizeof(uint64_t));
-    }
-    // count + scan + total to the host + emit of stretch j, on the schedule stream
-    auto enqueue_walk = [&](uint32_t j) -> int {
-        sched::ScheduleParams p{};
-        p.streams = d_streams; p.n_streams = n_streams; p.events = d_events; p.n_events = n_events;
-        p.status = ctx->d_status + 2;
-        p.state_in = j ? ctx->d_walk[j & 1] : nullptr;
-        p.state_out = ctx->d_walk[(j + 1) & 1];
-        p.stretch = j; p.n_stretches = n_stretches;
-        p.chunk_count = ctx->d_begin; p.out_bytes = d_stream_out_bytes;
-        p.timeline = j == 1 ? d_timeline : nullptr;
-        mark("count begins", j, ctx->sched_stream);
-        if (team == 32) sched::schedule_kernel<false, 32><<<grid, sched::kScheduleBlock, 0, ctx->sched_stream>>>(p);
-        else sched::schedule_kernel<false, 1><<<grid, sched::kScheduleBlock, 0, ctx->sched_stream>>>(p);
-        OHP_CUDA(ctx, cudaGetLastError());
-        mark("count ends", j, ctx->sched_stream);
-        sched::scan_kernel<<<1, sched::kScanThreads, 0, ctx->sched_stream>>>(ctx->d_begin, n_streams, ctx->d_bases + j);
-        OHP_CUDA(ctx, cudaGetLastError());
-        OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_bases + j + 1, ctx->d_bases + j + 1, sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->sched_stream));
-        OHP_CUDA(ctx, cudaEventRecord(ctx->sched_events[2 * j], ctx->sched_stream));
-        mark("emit begins", j, ctx->sched_stream);
-        p.chunk_count = nullptr; p.out_bytes = nullptr; p.state_out = nullptr; p.timeline = nullptr;
-        p.chunk_begin = ctx->d_begin; p.descs = ctx->d_descs; p.info = nullptr;
-        p.descs_cap = ctx->d_descs_cap / sizeof(ohp_chunk_desc);
-        if (team == 32) sched::schedule_kernel<true, 32><<<grid, sched::kScheduleBlock, 0, ctx->sched_stream>>>(p);
-        else sched::schedule_kernel<true, 1><<<grid, sched::kScheduleBlock, 0, ctx->sched_stream>>>(p);
-        OHP_CUDA(ctx, cudaGetLastError());
-        OHP_CUDA(ctx, cudaEventRecord(ctx->sched_events[2 * j + 1], ctx->sched_stream));
-        mark("emit ends", j, ctx->sched_stream);
-        ctx->launches += 3;
-        return OHP_OK;
-    };
-    // two stretches ahead of ramp_convert_kernel, no more: the host is not in the way of the first launch, and the GPU always
-    // has the next walk queued
-    for (uint32_t j = 0; j < n_stretches && j < 2; j++) {
-        if ((rc = enqueue_walk(j)) != OHP_OK) return rc;
-    }
-    ctx->h_bases[0] = 0;
-    for (uint32_t j = 0; j < n_stretches; j++) {
-        OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_events[2 * j]));
-        const uint64_t lo = ctx->h_bases[j], hi = ctx->h_bases[j + 1];
-        if (hi > ctx->d_descs_cap / sizeof(ohp_chunk_desc)) { // more playables than the bound allowed for: nothing was written for them
-            *overflowed = true;
-            break;
-        }
-        if (hi != lo) {
-            OHP_CUDA(ctx, cudaStreamWaitEvent(st, ctx->sched_events[2 * j + 1], 0));
-            mark("ramp_convert begins", j, st);
-            if ((rc = launch(ctx, ctx->d_descs + lo, (size_t)(hi - lo), d_in, in_bytes, d_out, out_bytes, st)) != OHP_OK) return rc;
-            mark("ramp_convert ends", j, st);
-        }
-        if (j + 2 < n_stretches && (rc = enqueue_walk(j + 2)) != OHP_OK) return rc;
-    }
-    if (trace) {
-        (void)cudaStreamSynchronize(st);
-        (void)cudaStreamSynchronize(ctx->sched_stream);
-        for (auto& m : marks) {
-            float ms = 0.f;
-            (void)cudaEventElapsedTime(&ms, marks[0].second, m.second);
-            std::fprintf(stderr, "[stretch trace] %8.3f ms  %s\n", ms, m.first.c_str());
-            if (&m != &marks[0]) (void)cudaEventDestroy(m.second);
-        }
-        (void)cudaEventDestroy(marks[0].second);
-        if (d_timeline) {
-            std::vector<uint64_t> tl((size_t)grid * 3);
-            (void)cudaMemcpy(tl.data(), d_timeline, tl.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost);
-            (void)cudaFree(d_timeline);
-            uint64_t t0 = ~0ull;
-            for (unsigned b = 0; b < grid; b++) if (tl[3 * b] && tl[3 * b] < t0) t0 = tl[3 * b];
-            for (unsigned b = 0; b < grid; b += (grid > 64 ? grid / 64 : 1)) {
-                std::fprintf(stderr, "[stretch trace] count 1, CTA %4u on SM %3u: started %8.1f us after the first, ran %8.1f us\n", b,
-                             (unsigned)tl[3 * b + 2], (tl[3 * b] - t0) / 1e3, (tl[3 * b + 1] - tl[3 * b]) / 1e3);
-            }
-        }
-    }
-    // a stream the walk refused (spec, ASSERT, stack depth) fails the call
-    const int src = schedule_status(ctx, ctx->sched_stream);
-    if (src != OHP_OK || *overflowed) {
-        OHP_CUDA(ctx, cudaStreamSynchronize(st));
-        return src;
-    }
-    if (total_chunks) *total_chunks = ctx->h_bases[n_stretches];
-    return OHP_OK;
 }
 
 int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
@@ -1304,166 +1124,70 @@ int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, s
         return run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
                                            d_stream_out_bytes, total_chunks, st);
     }
-    uint32_t n_stretches = kDefaultStretches; // OHP_STRETCHES=k: the walk in k stretches; 0 (default): the one-walk-into-regions path below
-    if (const char* e = std::getenv("OHP_STRETCHES")) {
-        const long v = std::atol(e);
-        n_stretches = v < 0 ? 0u : (v > (long)kMaxStretches ? kMaxStretches : (uint32_t)v);
-    }
-    if (n_stretches != 0) {
-        bool overflowed = false;
-        rc = run_streams_device_stretched(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
-                                          d_stream_out_bytes, total_chunks, n_stretches, st, &overflowed);
-        if (!overflowed) return rc;
-        if (rc != OHP_OK) return rc;
-        return run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
-                                           d_stream_out_bytes, total_chunks, st);
-    }
     // 1. regions: bound per stream, exclusive scan
     sched::bound_kernel<<<(unsigned)((n_streams + 127) / 128), 128, 0, st>>>(d_streams, n_streams, d_events, n_events, ctx->d_begin);
     OHP_CUDA(ctx, cudaGetLastError());
     sched::scan_kernel<<<1, sched::kScanThreads, 0, st>>>(ctx->d_begin, n_streams);
     OHP_CUDA(ctx, cudaGetLastError());
     ctx->launches += 2;
-    if (!std::getenv("OHP_SLICE_CHUNKS")) {
-        // THE DEFAULT: everything on the caller's stream, and the walk is launched BEFORE the host knows how many
-        // descriptors the regions add up to -- the total (8 bytes, pinned) comes back while the walk runs, so the host's
-        // round trip costs the GPU nothing.  The walk writes nothing for a stream whose region would end beyond the
-        // buffer; if the total says the buffer was too small (first call of a shape), it grows and the walk runs again.
-        if (!ctx->h_bases) OHP_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void**>(&ctx->h_bases), (kMaxStretches + 2) * sizeof(uint64_t), cudaHostAllocDefault));
-        if (ctx->sched_events.empty()) {
-            cudaEvent_t e;
-            OHP_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            ctx->sched_events.push_back(e);
-        }
-        OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_bases, ctx->d_begin + n_streams, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        OHP_CUDA(ctx, cudaEventRecord(ctx->sched_events[0], st));
-        const int team = schedule_team(n_streams);
-        auto walk = [&]() -> int {
-            sched::ScheduleParams p{};
-            p.streams = d_streams; p.n_streams = n_streams; p.events = d_events; p.n_events = n_events;
-            p.chunk_begin = ctx->d_begin; p.descs = ctx->d_descs; p.info = nullptr;
-            p.descs_cap = ctx->d_descs_cap / sizeof(ohp_chunk_desc);
-            p.status = ctx->d_status + 2;
-            p.first_stream = 0; p.counts_out = ctx->d_counts; p.out_bytes = d_stream_out_bytes;
-            p.lanes_per_warp = schedule_lanes(ctx, n_streams);
-            if (team == 32) sched::schedule_kernel<true, 32><<<sched::schedule_grid(n_streams, 32), sched::kScheduleBlock, 0, st>>>(p);
-            else sched::schedule_kernel<true, 1><<<sched::schedule_grid(n_streams, 1, p.lanes_per_warp), sched::kScheduleBlock, 0, st>>>(p);
-            OHP_CUDA(ctx, cudaGetLastError());
-            ctx->launches++;
-            return OHP_OK;
-        };
-        if (ctx->d_descs_cap >= sizeof(ohp_chunk_desc) && (rc = walk()) != OHP_OK) return rc; // (no buffer yet: after the total)
-        OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_events[0]));
-        const uint64_t regions = ctx->h_bases[0];
-        if (regions > ctx->d_descs_cap / sizeof(ohp_chunk_desc)) {
-            OHP_CUDA(ctx, cudaDeviceSynchronize()); // the buffer may still be read by a launch enqueued earlier on another stream
-            if ((rc = grow(ctx, ctx->d_descs, ctx->d_descs_cap, regions * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
-            if ((rc = walk()) != OHP_OK) return rc;
-        }
-        if (total_chunks) {
-            // the exact number of playables, and what the walk refused: in front of ramp_convert_kernel in the stream, so the
-            // host waits for the walk only
-            ctx->h_outb.resize(n_streams);
-            OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_outb.data(), ctx->d_counts, n_streams * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-            OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_status, ctx->d_status, 16 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-            OHP_CUDA(ctx, cudaEventRecord(ctx->sched_events[0], st));
-        }
-        if ((rc = launch(ctx, ctx->d_descs, (size_t)regions, d_in, in_bytes, d_out, out_bytes, st)) != OHP_OK) return rc;
-        if (total_chunks) {
-            OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_events[0]));
-            if (ctx->h_status[2] != 0) {
-                const int src = schedule_status(ctx, st); // waits for ramp_convert_kernel too: the call has failed anyway
-                if (src == OHP_E_NO_MEMORY && ctx->error.find("region") != std::string::npos) {
-                    // a stream outgrew its region: nothing wrong with the batch, take the exact two-pass path
-                    (void)read_status(ctx, st);
-                    return run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
-                                                       d_stream_out_bytes, total_chunks, st);
-                }
-                if (src != OHP_OK) return src;
-            }
-            uint64_t total = 0;
-            for (size_t s2 = 0; s2 < n_streams; s2++) total += ctx->h_outb[s2];
-            *total_chunks = total;
-        }
-        return OHP_OK;
-    }
-    // 1b. (OHP_SLICE_CHUNKS: slices of streams) the regions' offsets to the host
-    ctx->h_begin.resize(n_streams + 1);
-    OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_begin.data(), ctx->d_begin, (n_streams + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    OHP_CUDA(ctx, cudaStreamSynchronize(st));
-    const uint64_t regions = ctx->h_begin[n_streams];
-    if (regions > ctx->d_descs_cap / sizeof(ohp_chunk_desc)) {
-        OHP_CUDA(ctx, cudaDeviceSynchronize());
-        if ((rc = grow(ctx, ctx->d_descs, ctx->d_descs_cap, regions * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
-    }
-    // 2. slices of streams, about equal in descriptors; the walk of each on the schedule stream, its ramp_convert launch on
-    //    the caller's stream behind it
-    uint64_t kSliceChunks = ~0ull;
-    if (const char* e = std::getenv("OHP_SLICE_CHUNKS")) { // experiments and tests
-        const long v = std::atol(e);
-        if (v > 0) kSliceChunks = (uint64_t)v;
-    }
-    size_t n_slices = (size_t)((regions + kSliceChunks - 1) / kSliceChunks);
-    if (n_slices > 8) n_slices = 8;
-    if (n_slices < 1) n_slices = 1;
-    if (ctx->sched_events.size() < n_slices + 1) {
-        while (ctx->sched_events.size() < n_slices + 1) {
-            cudaEvent_t e;
-            OHP_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            ctx->sched_events.push_back(e);
-        }
-    }
-    if (!ctx->sched_stream) {
-        int least = 0, greatest = 0;
-        OHP_CUDA(ctx, cudaDeviceGetStreamPriorityRange(&least, &greatest));
-        OHP_CUDA(ctx, cudaStreamCreateWithPriority(&ctx->sched_stream, cudaStreamNonBlocking, least));
-    }
-    // the schedule stream starts behind whatever the caller's stream holds so far (specs, events and PCM may just have arrived)
-    OHP_CUDA(ctx, cudaEventRecord(ctx->sched_events[n_slices], st));
-    OHP_CUDA(ctx, cudaStreamWaitEvent(ctx->sched_stream, ctx->sched_events[n_slices], 0));
+    // 2. everything on the caller's stream, and the walk is launched BEFORE the host knows how many descriptors the
+    //    regions add up to -- the total (8 bytes, pinned) comes back while the walk runs, so the host's round trip costs
+    //    the GPU nothing.  The walk writes nothing for a stream whose region would end beyond the buffer; if the total says
+    //    the buffer was too small (first call of a shape), it grows and the walk runs again.
+    if (!ctx->h_regions) OHP_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void**>(&ctx->h_regions), sizeof(uint64_t), cudaHostAllocDefault));
+    if (!ctx->sched_event) OHP_CUDA(ctx, cudaEventCreateWithFlags(&ctx->sched_event, cudaEventDisableTiming));
+    OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_regions, ctx->d_begin + n_streams, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    OHP_CUDA(ctx, cudaEventRecord(ctx->sched_event, st));
     const int team = schedule_team(n_streams);
-    size_t lo = 0;
-    for (size_t k = 0; k < n_slices; k++) {
-        // streams [lo, hi): up to the next multiple of regions / n_slices descriptors
-        const uint64_t want = regions * (k + 1) / n_slices;
-        size_t hi = (size_t)(std::upper_bound(ctx->h_begin.begin() + lo, ctx->h_begin.begin() + n_streams, want) - ctx->h_begin.begin());
-        if (hi <= lo) hi = lo + 1;
-        if (hi > n_streams || k + 1 == n_slices) hi = n_streams;
+    auto walk = [&]() -> int {
         sched::ScheduleParams p{};
-        p.streams = d_streams; p.n_streams = hi - lo; p.events = d_events; p.n_events = n_events;
+        p.streams = d_streams; p.n_streams = n_streams; p.events = d_events; p.n_events = n_events;
         p.chunk_begin = ctx->d_begin; p.descs = ctx->d_descs; p.info = nullptr;
+        p.descs_cap = ctx->d_descs_cap / sizeof(ohp_chunk_desc);
         p.status = ctx->d_status + 2;
-        p.first_stream = lo; p.counts_out = ctx->d_counts; p.out_bytes = d_stream_out_bytes;
-        if (team == 32) sched::schedule_kernel<true, 32><<<sched::schedule_grid(hi - lo, 32), sched::kScheduleBlock, 0, ctx->sched_stream>>>(p);
-        else sched::schedule_kernel<true, 1><<<sched::schedule_grid(hi - lo, 1), sched::kScheduleBlock, 0, ctx->sched_stream>>>(p);
+        p.counts_out = ctx->d_counts; p.out_bytes = d_stream_out_bytes;
+        p.lanes_per_warp = schedule_lanes(ctx, n_streams);
+        if (team == 32) sched::schedule_kernel<true, 32><<<sched::schedule_grid(n_streams, 32), sched::kScheduleBlock, 0, st>>>(p);
+        else sched::schedule_kernel<true, 1><<<sched::schedule_grid(n_streams, 1, p.lanes_per_warp), sched::kScheduleBlock, 0, st>>>(p);
         OHP_CUDA(ctx, cudaGetLastError());
         ctx->launches++;
-        OHP_CUDA(ctx, cudaEventRecord(ctx->sched_events[k], ctx->sched_stream));
-        OHP_CUDA(ctx, cudaStreamWaitEvent(st, ctx->sched_events[k], 0));
-        const uint64_t c_lo = ctx->h_begin[lo], c_hi = ctx->h_begin[hi];
-        if ((rc = launch(ctx, ctx->d_descs + c_lo, (size_t)(c_hi - c_lo), d_in, in_bytes, d_out, out_bytes, st)) != OHP_OK) return rc;
-        lo = hi;
-        if (lo == n_streams) break;
+        return OHP_OK;
+    };
+    if (ctx->d_descs_cap >= sizeof(ohp_chunk_desc) && (rc = walk()) != OHP_OK) return rc; // (no buffer yet: after the total)
+    OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_event));
+    const uint64_t regions = *ctx->h_regions;
+    if (regions > ctx->d_descs_cap / sizeof(ohp_chunk_desc)) {
+        OHP_CUDA(ctx, cudaDeviceSynchronize()); // the buffer may still be read by a launch enqueued earlier on another stream
+        if ((rc = grow(ctx, ctx->d_descs, ctx->d_descs_cap, regions * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
+        if ((rc = walk()) != OHP_OK) return rc;
     }
     if (total_chunks) {
-        // the exact number of playables: wait for the walks (not for ramp_convert_kernel), add the streams' counts up
-        OHP_CUDA(ctx, cudaStreamSynchronize(ctx->sched_stream));
+        // the exact number of playables, and what the walk refused: in front of ramp_convert_kernel in the stream, so the
+        // host waits for the walk only
         ctx->h_outb.resize(n_streams);
-        OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_outb.data(), ctx->d_counts, n_streams * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->sched_stream));
-        OHP_CUDA(ctx, cudaStreamSynchronize(ctx->sched_stream));
-        const int src = schedule_status(ctx, ctx->sched_stream);
-        if (src == OHP_E_NO_MEMORY && ctx->error.find("region") != std::string::npos) {
-            // a stream outgrew its region: nothing wrong with the batch, take the exact two-pass path
-            OHP_CUDA(ctx, cudaStreamSynchronize(st));
+        OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_outb.data(), ctx->d_counts, n_streams * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_status, ctx->d_status, 16 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        OHP_CUDA(ctx, cudaEventRecord(ctx->sched_event, st));
+    }
+    if ((rc = launch(ctx, ctx->d_descs, (size_t)regions, d_in, in_bytes, d_out, out_bytes, st)) != OHP_OK) return rc;
+    if (!total_chunks) return OHP_OK;
+    OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_event));
+    const uint32_t bits = ctx->h_status[2];
+    if (bits != 0) {
+        const int src = schedule_status(ctx, st); // waits for ramp_convert_kernel too: the call has failed anyway
+        // a stream outgrew its region and none was refused for what it is (schedule_status reports those first): nothing
+        // wrong with the batch, take the exact two-pass path
+        const uint32_t refused = (1u << sched::kErrSpec) | (1u << sched::kErrAssert);
+        if ((bits & (1u << sched::kErrBound)) && !(bits & refused)) {
             (void)read_status(ctx, st);
             return run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
                                                d_stream_out_bytes, total_chunks, st);
         }
         if (src != OHP_OK) return src;
-        uint64_t total = 0;
-        for (size_t s2 = 0; s2 < n_streams; s2++) total += ctx->h_outb[s2];
-        *total_chunks = total;
     }
+    uint64_t total = 0;
+    for (size_t s = 0; s < n_streams; s++) total += ctx->h_outb[s];
+    *total_chunks = total;
     return OHP_OK;
 }
 

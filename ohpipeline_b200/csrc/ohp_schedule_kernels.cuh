@@ -29,16 +29,8 @@ struct ScheduleParams
     ohp_chunk_info* info;      // EMIT, may be null
     uint32_t* status;          // [0] error bits (1 << code), [1] 0xffffffff - lowest failing stream (atomicMax; 0 = none)
     // ONE-WALK mode (regions from stream_chunk_bound): EMIT also reports what COUNT would have, and fills each region's tail
-    uint64_t first_stream;     // the slice [first_stream, first_stream + n_streams) of the batch is walked
-    uint64_t* counts_out;      // [all streams] exact playables per stream (null: two-pass mode)
-    // STRETCH mode (n_stretches != 0): every stream is walked from where stretch - 1 stopped to stretch_stop_frame();
-    // COUNT leaves the state for the next stretch in state_out, EMIT re-walks the stretch from state_in.  chunk_count /
-    // chunk_begin are per stretch: descriptors come out compact, stretch after stretch, streams in order inside each.
-    const WalkState* state_in; // [n_streams], null for stretch 0
-    WalkState* state_out;      // [n_streams], COUNT only
-    uint32_t stretch, n_stretches;
-    uint64_t descs_cap;        // EMIT: descriptors the buffer holds; a stream whose stretch would end beyond writes nothing
-    uint64_t* timeline;        // experiments (OHP_STRETCH_TRACE): [3 * CTAs] globaltimer at a CTA's start and end, its SM; else null
+    uint64_t* counts_out;      // [n_streams] exact playables per stream (null: two-pass mode)
+    uint64_t descs_cap;        // descriptors the buffer holds; a stream whose region would end beyond writes nothing (0: no check)
     uint32_t lanes_per_warp;   // TEAM = 1: streams a warp walks (its first lanes, one each; the others idle); 0 = 32
 };
 
@@ -58,49 +50,31 @@ __global__ void __launch_bounds__(128) bound_kernel(const ohp_stream_spec* __res
 // step written side by side) when streams are few enough for that to fill the GPU, TEAM = 1 (a thread per stream) when
 // there are so many streams that they alone do.  All lanes of a team hold the same state; see schedule_walk.h.
 #ifndef OHP_SCHED_MIN_BLOCKS
-#define OHP_SCHED_MIN_BLOCKS 3 /* <= 168 registers: a 128-thread CTA of the walk must fit into the 24064 registers that two of ramp_convert_kernel's
-                                  persistent CTAs leave on an SM, or the walks of ohp_run_streams_device wait for that kernel to end
-                                  (measured: at 200 registers they did).  5 (96 registers, 7 warps beside it) spills and loses. */
+#define OHP_SCHED_MIN_BLOCKS 3 /* <= 168 registers.  The walk times of DESIGN 4.2 were measured with this bound; 5 (96 registers) spills. */
 #endif
 template <bool EMIT, int TEAM>
 __global__ void __launch_bounds__(128, OHP_SCHED_MIN_BLOCKS) schedule_kernel(const ScheduleParams p)
 {
     const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    uint64_t local = t / TEAM;
+    uint64_t s = t / TEAM;
     const uint32_t lane = (uint32_t)(t % TEAM);
     if (TEAM == 1 && p.lanes_per_warp != 0) {
         // a thread per stream, but fewer streams than lanes in a warp: threads of a warp walk different streams and
         // take turns wherever their paths differ, so a warp takes about as long as its streams take one after the other
         if ((t & 31u) >= p.lanes_per_warp) return;
-        local = (t >> 5) * p.lanes_per_warp + (t & 31u);
+        s = (t >> 5) * p.lanes_per_warp + (t & 31u);
     }
-    if (p.timeline != nullptr && threadIdx.x == 0) {
-        uint64_t now; uint32_t sm;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(sm));
-        p.timeline[3 * blockIdx.x] = now; p.timeline[3 * blockIdx.x + 2] = sm;
-    }
-    if (local >= p.n_streams) return;
-    const uint64_t s = p.first_stream + local;
+    if (s >= p.n_streams) return;
     const ohp_stream_spec sp = p.streams[s];
     uint64_t nChunks, outBytes;
-    const bool stretched = p.n_stretches != 0;
-    const WalkState* in = (stretched && p.state_in != nullptr) ? p.state_in + s : nullptr;
-    WalkState* out = (stretched && !EMIT) ? p.state_out + s : nullptr;
-    const uint64_t stop = stretched ? stretch_stop_frame(sp.total_frames, p.stretch, p.n_stretches) : ~0ull;
-    const uint64_t before = (in != nullptr && in->phase != 0) ? in->nChunks : 0; // playables of the stretches in front
-    // EMIT: the walk indexes a stream's playables from its start; this stretch's first one goes to chunk_begin[s]
-    ohp_chunk_desc* descs = EMIT ? p.descs + p.chunk_begin[s] - before : nullptr;
-    ohp_chunk_info* info = (EMIT && p.info) ? p.info + p.chunk_begin[s] - before : nullptr;
+    ohp_chunk_desc* descs = EMIT ? p.descs + p.chunk_begin[s] : nullptr;
+    ohp_chunk_info* info = (EMIT && p.info) ? p.info + p.chunk_begin[s] : nullptr;
     const bool regions = EMIT && p.counts_out != nullptr;
     // (regions: launched before the host has sized the buffer -- a stream whose region would end beyond it is left for the
     //  second launch that follows when that turns out to be the case)
     if (regions && p.descs_cap != 0 && p.chunk_begin[s + 1] > p.descs_cap) return;
-    uint64_t limit = regions ? p.chunk_begin[s + 1] - p.chunk_begin[s] : ~0ull;
-    if (EMIT && stretched) { // a refused stream counted 0: it writes nothing
-        limit = p.chunk_begin[s + 1] <= p.descs_cap ? before + (p.chunk_begin[s + 1] - p.chunk_begin[s]) : before;
-    }
-    uint32_t rc = run_stream<EMIT, TEAM, true>(sp, p.events, p.n_events, descs, info, nChunks, outBytes, lane, limit, in, out, stop);
+    const uint64_t limit = regions ? p.chunk_begin[s + 1] - p.chunk_begin[s] : ~0ull;
+    uint32_t rc = run_stream<EMIT, TEAM, true>(sp, p.events, p.n_events, descs, info, nChunks, outBytes, lane, limit);
     if (regions) {
         if (rc == kOk && nChunks > limit) rc = kErrBound;
         // the rest of the region: zero-byte descriptors (all lanes of the team, two 128-bit stores each)
@@ -108,21 +82,13 @@ __global__ void __launch_bounds__(128, OHP_SCHED_MIN_BLOCKS) schedule_kernel(con
         uint4* d4 = reinterpret_cast<uint4*>(descs);
         for (uint64_t i = 2 * from + lane; i < 2 * limit; i += TEAM) d4[i] = make_uint4(0, 0, 0, 0);
     }
-    if (p.timeline != nullptr && threadIdx.x == 0) { // warp 0's end stands for the CTA's (streams of a batch are of a length)
-        uint64_t now;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-        p.timeline[3 * blockIdx.x + 1] = now;
-    }
     if (lane != 0) return;
     if (rc != kOk) {
         atomicOr(&p.status[0], 1u << rc);
         atomicMax(&p.status[1], 0xffffffffu - (uint32_t)(s > 0xfffffffeull ? 0xfffffffeull : s));
-        if (out != nullptr) { // the call fails; later stretches find this stream over
-            out->phase = 2; out->nChunks = before; out->outBytes = 0;
-        }
     }
     if (!EMIT) {
-        p.chunk_count[s] = (stretched && rc == kOk) ? nChunks - before : nChunks;
+        p.chunk_count[s] = nChunks;
         if (p.out_bytes) p.out_bytes[s] = outBytes;
     }
     else if (regions) {
@@ -143,17 +109,13 @@ inline unsigned schedule_grid(uint64_t n_streams, int team, uint32_t lanes_per_w
 }
 
 // In-place exclusive scan of counts[0..n) into begin[0..n] (begin has n+1 entries; begin[n] = total).  One CTA.
-// base (may be null): base[0] is added to every entry and base[1] = base[0] + total is left for the next scan -- how the
-// stretches of ohp_run_streams_device lay their descriptors out one after the other without the host in between.
-// 256 threads, not 1024: the stretches' scans run while ramp_convert_kernel's persistent CTAs hold two thirds of every
-// SM's registers, and a 1024-thread CTA finds no SM to run on until that kernel ends (measured: the walk of stretch
-// k + 1 then waits for ramp_convert_kernel on stretch k, and the overlap is gone).
+// 256 threads: the walk times of DESIGN 4.2 were measured with this scan.
 constexpr unsigned kScanThreads = 256;
-__global__ void __launch_bounds__(kScanThreads) scan_kernel(uint64_t* begin, uint64_t n, uint64_t* base = nullptr)
+__global__ void __launch_bounds__(kScanThreads) scan_kernel(uint64_t* begin, uint64_t n)
 {
     __shared__ uint64_t warp_sum[kScanThreads / 32];
     __shared__ uint64_t carry;
-    if (threadIdx.x == 0) carry = base ? base[0] : 0;
+    if (threadIdx.x == 0) carry = 0;
     __syncthreads();
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (uint64_t first = 0; first < n; first += kScanThreads) {
@@ -181,10 +143,7 @@ __global__ void __launch_bounds__(kScanThreads) scan_kernel(uint64_t* begin, uin
         if (threadIdx.x == kScanThreads - 1) carry = before + v;
         __syncthreads();
     }
-    if (threadIdx.x == 0) {
-        begin[n] = carry;
-        if (base) base[1] = carry;
-    }
+    if (threadIdx.x == 0) begin[n] = carry;
 }
 
 } // namespace sched

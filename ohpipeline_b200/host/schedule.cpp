@@ -211,13 +211,6 @@ int ohp_schedule_build(const ohp_stream_spec* streams, size_t n_streams, const o
 int ohp_schedule_build_walk(const ohp_stream_spec* streams, size_t n_streams, const ohp_ramp_event* events, size_t n_events,
                             int threads, ohp_schedule** out)
 {
-    return ohp_schedule_build_walk_stretches(streams, n_streams, events, n_events, threads, 1, out);
-}
-
-int ohp_schedule_build_walk_stretches(const ohp_stream_spec* streams, size_t n_streams, const ohp_ramp_event* events, size_t n_events,
-                                      int threads, uint32_t n_stretches, ohp_schedule** out)
-{
-    if (n_stretches == 0) n_stretches = 1;
     if (!out || (!streams && n_streams) || (!events && n_events)) {
         g_error = "null argument";
         return OHP_E_INVALID_ARG;
@@ -236,23 +229,12 @@ int ohp_schedule_build_walk_stretches(const ohp_stream_spec* streams, size_t n_s
             const size_t hi = n_streams * (size_t)(t + 1) / (size_t)threads;
             for (size_t s = lo; s < hi; s++) {
                 uint64_t n = 0, bytes = 0;
-                // in stretches: each starts from the state the one before left (as the device's COUNT pass does; its
-                // EMIT pass re-walks a stretch from the same state, which is what the emit run here does too)
-                sched::WalkState state[2];
-                state[0].phase = 0;
-                for (uint32_t j = 0; j < n_stretches && rcs[s] == sched::kOk; j++) {
-                    const sched::WalkState* in = j ? &state[j & 1] : nullptr;
-                    sched::WalkState* next = &state[(j + 1) & 1];
-                    const uint64_t stop = sched::stretch_stop_frame(streams[s].total_frames, j, n_stretches);
-                    if (emit) {
-                        rcs[s] = sched::run_stream<true>(streams[s], events, n_events, sch->chunks.data() + sch->chunkBegin[s],
-                                                         sch->info.data() + sch->chunkBegin[s], n, bytes, 0, ~0ull, in, next, stop);
-                    }
-                    else {
-                        rcs[s] = sched::run_stream<false>(streams[s], events, n_events, nullptr, nullptr, n, bytes, 0, ~0ull, in, next, stop);
-                    }
+                if (emit) {
+                    rcs[s] = sched::run_stream<true>(streams[s], events, n_events, sch->chunks.data() + sch->chunkBegin[s],
+                                                     sch->info.data() + sch->chunkBegin[s], n, bytes);
                 }
-                if (!emit) {
+                else {
+                    rcs[s] = sched::run_stream<false>(streams[s], events, n_events, nullptr, nullptr, n, bytes);
                     sch->chunkBegin[s + 1] = n; // scanned below
                     sch->outBytes[s] = bytes;
                 }

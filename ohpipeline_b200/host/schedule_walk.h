@@ -562,21 +562,6 @@ struct Lookahead
     uint32_t head, count;
 };
 
-// A walk can stop between two messages and go on later (ohp_run_streams_device walks every stream a stretch of its
-// length at a time, so that ramp_convert_kernel can start on the first stretch while the rest is still being walked):
-// everything walk_stream keeps between messages.  The stages' stacks are not in here -- they are empty whenever a message
-// has been fed through (see walk_stream).
-struct WalkState
-{
-    Stage st[kStages];
-    Cursor cur;
-    core::CodecSource source;
-    Lookahead la;
-    uint64_t nChunks, outBytes;
-    uint32_t blockFill;
-    uint32_t phase;        // 0: not started, 1: stopped at aStopFrame, 2: the stream is over
-};
-
 OHP_HD void lookahead_fill(core::CodecSource& src, Lookahead& la)
 {
     if (la.head != la.count) return;
@@ -874,42 +859,20 @@ OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[
     return n;
 }
 
-// Where stretch aIndex of aCount ends, as a frame of the source: stretches of equal length; the last one runs to the end
-// of the stream.
-OHP_HD uint64_t stretch_stop_frame(uint64_t aTotalFrames, uint32_t aIndex, uint32_t aCount)
-{
-    if (aIndex + 1 >= aCount) return ~0ull;
-    return (aTotalFrames / aCount) * (aIndex + 1); // total_frames < 2^64 / aCount is not assumed
-}
-
 // One stream's walk.  The per-stage queues of stage_chain.h only ever grow at the front while a stage is being served
 // and are drained before the stage returns, so each is a stack; Feed()'s recursion becomes: carry the message down
 // the remaining stages (in registers), hand it to the driver, then resume with the top of the deepest non-empty stack.
 // A team of STRIDE threads (device: a warp, or 1; host: 1) walks the stream holding identical state; they differ only
 // in cx.lane, i.e. in which messages of a bulk step they emit.  BULK = false is the message-at-a-time walk alone.
-// aIn / aOut / aStopFrame: the walk in stretches.  aIn (phase 1) is where an earlier call stopped; the walk stops in front
-// of the first message that starts at or after frame aStopFrame of the source and leaves its state in aOut (may be null:
-// a pass that only re-walks a stretch).  The playables' indices and output offsets run on across stretches.
 template <bool EMIT, int STRIDE, bool BULK>
-OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx, const WalkState* aIn = nullptr, WalkState* aOut = nullptr,
-                            uint64_t aStopFrame = ~0ull)
+OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
 {
     Packed stack[kStages][kStackDepth];
     Stage st[kStages];
-    const bool resume = aIn != nullptr && aIn->phase != 0;
-    if (resume && aIn->phase == 2) { // nothing left of this stream
-        cx.nChunks = aIn->nChunks; cx.outBytes = aIn->outBytes;
-        if (aOut != nullptr && cx.lane == 0 && aOut != aIn) *aOut = *aIn;
-        return kOk;
-    }
 #if defined(__CUDA_ARCH__)
 #pragma unroll
 #endif
     for (int i = 0; i < kStages; i++) {
-        if (resume) {
-            st[i] = aIn->st[i];
-            continue;
-        }
         st[i].pos = 0; st[i].mode = Running; st[i].current = core::kRampMax; st[i].remaining = 0; st[i].maxMsg = 0;
         st[i].attenuation = OHP_UNITY_ATTENUATION; st[i].depth = 0;
         st[i].elem = stage_element(cx, (uint32_t)i);
@@ -958,34 +921,14 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx, const Walk
 
     // stage_chain.h Run()
     Cursor cur;
+    cur.frame = 0;
+    cur.srcJiffies = 0;
+    seek_silence(cx, cur, 0);
     core::CodecSource source;
+    core::codec_source_init(source, sp.chunk_frames, sp.codec_read_frames, cx.frameBytes, cx.jps, sp.total_frames);
     Lookahead la;
-    if (resume) {
-        cur = aIn->cur; source = aIn->source; la = aIn->la;
-        cx.nChunks = aIn->nChunks; cx.outBytes = aIn->outBytes; cx.blockFill = aIn->blockFill;
-    }
-    else {
-        cur.frame = 0;
-        cur.srcJiffies = 0;
-        seek_silence(cx, cur, 0);
-        core::codec_source_init(source, sp.chunk_frames, sp.codec_read_frames, cx.frameBytes, cx.jps, sp.total_frames);
-        la.head = la.count = 0;
-    }
-    auto leave = [&](uint32_t aPhase) {
-        if (aOut == nullptr || cx.lane != 0) return;
-#if defined(__CUDA_ARCH__)
-#pragma unroll
-#endif
-        for (int i = 0; i < kStages; i++) aOut->st[i] = st[i];
-        aOut->cur = cur; aOut->source = source; aOut->la = la;
-        aOut->nChunks = cx.nChunks; aOut->outBytes = cx.outBytes; aOut->blockFill = cx.blockFill;
-        aOut->phase = aPhase;
-    };
+    la.head = la.count = 0;
     for (;;) {
-        if (cur.frame >= aStopFrame) { // the stages' stacks are empty here: every message fed so far went all the way through
-            leave(1);
-            return kOk;
-        }
         if (BULK) {
             uint32_t e;
             const uint32_t n = source.read == 0 ? bulk_step<EMIT, STRIDE, true>(sp, cx, st, source, la, cur, e)
@@ -1023,7 +966,6 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx, const Walk
         cur.frame += frames;
         cur.srcJiffies += (uint64_t)frames * cx.jps;
     }
-    leave(2);
     return kOk;
 }
 
@@ -1032,8 +974,7 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx, const Walk
 template <bool EMIT, int STRIDE = 1, bool BULK = true>
 OHP_HD uint32_t run_stream(const ohp_stream_spec& sp, const ohp_ramp_event* aEvents, uint64_t aNumEvents,
                            ohp_chunk_desc* aDescs, ohp_chunk_info* aInfo, uint64_t& aNumChunks, uint64_t& aOutBytes,
-                           uint32_t aLane = 0, uint64_t aLimit = ~0ull,
-                           const WalkState* aIn = nullptr, WalkState* aOut = nullptr, uint64_t aStopFrame = ~0ull)
+                           uint32_t aLane = 0, uint64_t aLimit = ~0ull)
 {
     aNumChunks = 0;
     aOutBytes = 0;
@@ -1057,7 +998,7 @@ OHP_HD uint32_t run_stream(const ohp_stream_spec& sp, const ohp_ramp_event* aEve
     cx.descs = EMIT ? aDescs : nullptr;
     cx.info = EMIT ? aInfo : nullptr;
     cx.limit = aLimit;
-    const uint32_t rc = walk_stream<EMIT, STRIDE, BULK>(sp, cx, aIn, aOut, aStopFrame);
+    const uint32_t rc = walk_stream<EMIT, STRIDE, BULK>(sp, cx);
     if (rc != kOk) return rc;
     aNumChunks = cx.nChunks;
     aOutBytes = cx.outBytes;

@@ -270,19 +270,12 @@ def test_whole_stage_for_a_batch_resident_in_hbm(ctx, port, make):
             torch.cuda.synchronize()
 
 
-@pytest.mark.parametrize("mode", ["stretches_1", "stretches_3", "stretches_8", "stretches_16", "one_walk_sliced", "two_pass"])
+@pytest.mark.parametrize("mode", ["one_walk", "two_pass"])
 def test_whole_stage_device_call_in_every_mode(ctx, port, mode, monkeypatch):
-    """ohp_run_streams_device's default is one walk per stream into bounded regions
-    (test_whole_stage_for_a_batch_resident_in_hbm); here that path cut into slices of streams, the walk in stretches of
-    time (stopped and resumed from its saved state, descriptors stretch-major), and the round-1 count + scan + emit path:
-    same bytes, same sizes, same count."""
+    """ohp_run_streams_device's default, one walk per stream into bounded regions, and its fallback, the round-1 count +
+    scan + emit path (OHP_ONE_WALK=0): same bytes, same sizes, same count, with and without the chunk total."""
     import torch
-    if mode.startswith("stretches_"):
-        monkeypatch.setenv("OHP_STRETCHES", mode.split("_")[1])
-    elif mode == "two_pass":
-        monkeypatch.setenv("OHP_ONE_WALK", "0")
-    else:
-        monkeypatch.setenv("OHP_SLICE_CHUNKS", "700")
+    monkeypatch.setenv("OHP_ONE_WALK", "1" if mode == "one_walk" else "0")
     for w in (workloads.config4(n_streams=120, seconds=0.12, seed=3), workloads.elements(4, n_streams=60), workloads.config5(n_streams=90, seconds=0.1)):
         inp = port.fill_pcm(w.in_bytes, w.seed)
         rc, want, chunks, _ = port.run(w.streams, w.events, inp, w.out_bytes)

@@ -175,34 +175,3 @@ def test_closed_form_bound_covers_every_stream():
     bad = W.config5(2, 0.05)
     bad.streams["sample_rate"][1] = 12345
     assert int(capi.schedule_chunk_bounds(bad.streams, bad.events)[1]) == 0
-
-
-@pytest.mark.parametrize("stretches", [2, 8, 16])
-def test_walk_in_stretches_gives_the_same_playables(stretches):
-    """ohp_run_streams_device walks every stream a stretch at a time (so that ramp_convert_kernel can start after the
-    first sixteenth): stopping between two messages and resuming from the saved state must change nothing -- not the
-    playables, not the ramps carried across the stop, not what the reference would ASSERT on."""
-    from ohpipeline_b200 import workloads as W
-    cases = [W.config1(6.2), W.config2(8, 0.5), W.config3(40, 1.0), W.config4(120, 0.25), W.config5(16, 0.25), W.all_rates(),
-             W.mixed(80, 7, 4000), W.steady_edges(3, 48), W.elements(5, 24), W.elements(6, 24, illegal=True)]
-    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "elements_11.npz"))
-    cases.append(type("G", (), {"streams": g["streams"], "events": g["events"], "name": "golden elements"}))
-    compared = 0
-    for w in cases:
-        for k in range(len(w.streams)):
-            st = w.streams[k:k + 1].copy()
-            ev = w.events[int(st[0]["first_event"]):int(st[0]["first_event"]) + int(st[0]["num_events"])].copy()
-            st[0]["first_event"] = 0
-            try:
-                whole = capi.schedule_build(st, ev, walk=True)
-            except capi.OhpError as e:
-                with pytest.raises(capi.OhpError) as e2:
-                    capi.schedule_build(st, ev, stretches=stretches)
-                assert e2.value.status == e.status
-                continue
-            parts = capi.schedule_build(st, ev, stretches=stretches)
-            assert np.array_equal(parts.chunks, whole.chunks), (w.name, k)
-            assert np.array_equal(parts.info, whole.info)
-            assert np.array_equal(parts.stream_out_bytes, whole.stream_out_bytes)
-            compared += 1
-    assert compared > 400
