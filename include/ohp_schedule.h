@@ -109,7 +109,8 @@ int    ohp_schedule_build(const ohp_stream_spec* streams, size_t n_streams,
                           const ohp_ramp_event* events, size_t n_events,
                           int threads, ohp_schedule** out);
 /* Same result from the class-free walk the GPU schedule kernels compile (ohpipeline_b200/host/schedule_walk.h;
- * device entry points in ohp_schedule_device.h): no message objects, two passes (count, emit). */
+ * device entry points in ohp_schedule_device.h): no message objects, two passes (count, emit).  It records the same
+ * starvations as ohp_schedule_build (ohp_schedule_starvations), without the recent audio's pieces. */
 int    ohp_schedule_build_walk(const ohp_stream_spec* streams, size_t n_streams,
                                const ohp_ramp_event* events, size_t n_events,
                                int threads, ohp_schedule** out);
@@ -130,8 +131,9 @@ void   ohp_schedule_free(ohp_schedule* s);
 
 /*
  * What a stream's StarvationRamper stage was doing when its reservoir ran dry (OHP_EV_STARVATION): everything the flywheel
- * ramp it then plays is made from.  ohp_schedule_build records one per starvation event it applies, streams in order
- * (the class-free walk and the device builders do not: starvations are rare, their flywheel work is planned on the host).
+ * ramp it then plays is made from.  ohp_schedule_build records one per starvation event it applies, streams in order, and
+ * so does the class-free walk (ohp_schedule_build_walk; on the device: ohp_run_streams_device_flywheel,
+ * ohp_starvation_device.h), which keeps no recent audio: its ohp_schedule_recent_begin is all zeros.
  * tests/test_elements_vs_reference.py holds the audio planned from these records against what the real StarvationRamper
  * object plays when it is starved at the same position.
  *

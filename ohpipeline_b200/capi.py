@@ -96,6 +96,11 @@ def cuda_lib():
             L.ohp_run_streams_host.restype = C.c_int
             L.ohp_run_streams_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p, C.c_uint64,
                                                C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint64)]
+        if hasattr(L, "ohp_run_streams_device_flywheel"):
+            L.ohp_run_streams_device_flywheel.restype = C.c_int
+            L.ohp_run_streams_device_flywheel.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p,
+                                                          C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p,
+                                                          C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.c_void_p]
         if hasattr(L, "ohp_run_streams_device"):
             L.ohp_run_streams_device.restype = C.c_int
             L.ohp_run_streams_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p, C.c_uint64,
@@ -611,6 +616,21 @@ class Context:
                                                    C.c_void_p(d_in), in_bytes, C.c_void_p(d_out), out_bytes,
                                                    C.c_void_p(d_stream_out_bytes), C.byref(total) if want_total else None,
                                                    C.c_void_p(stream or 0)))
+        return int(total.value) if want_total else None
+
+    def run_streams_device_flywheel(self, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
+                                    d_fly_out, fly_out_bytes, d_fly_off, d_fly_len, d_starvations=0, d_stream_out_bytes=0,
+                                    stream=None, want_total=True):
+        """ohp_run_streams_device_flywheel: run_streams_device, plus the flywheel audio every starving StarvationRamper plays
+        (event e's at d_fly_out + d_fly_off[e], d_fly_len[e] bytes) and, where d_starvations is given, the starvation
+        records (abi.STARVATION, one per event).  Raw device addresses; returns the playables read (None without want_total)."""
+        total = C.c_uint64(0)
+        self._check(self._L.ohp_run_streams_device_flywheel(self._h, C.c_void_p(d_streams), n_streams, C.c_void_p(d_events), n_events,
+                                                            C.c_void_p(d_in), in_bytes, C.c_void_p(d_out), out_bytes,
+                                                            C.c_void_p(d_fly_out), fly_out_bytes, C.c_void_p(d_starvations),
+                                                            C.c_void_p(d_fly_off), C.c_void_p(d_fly_len),
+                                                            C.c_void_p(d_stream_out_bytes), C.byref(total) if want_total else None,
+                                                            C.c_void_p(stream or 0)))
         return int(total.value) if want_total else None
 
     def fill_streams_device(self, d_in, in_bytes, d_streams, n_streams, seed_base, first_stream_id=0, stream=None):

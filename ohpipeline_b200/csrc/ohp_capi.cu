@@ -9,6 +9,7 @@
 #include "ohp_schedule_kernels.cuh"
 #include "ohp_flywheel_kernels.cuh"
 #include "../../include/ohp_schedule_device.h"
+#include "../../include/ohp_starvation_device.h"
 
 #include <cstdio>
 #include <cstdlib>
@@ -83,7 +84,17 @@ struct ohp_context
     uint64_t* d_outb = nullptr; uint64_t d_outb_cap = 0;
     uint64_t* d_counts = nullptr; uint64_t d_counts_cap = 0;  // ohp_run_streams_device: exact playables per stream
     cudaEvent_t sched_event = nullptr;                           // ... recorded behind a copy the host waits for
-    uint64_t* h_regions = nullptr;                               // ... the regions' total (pinned)
+    cudaEvent_t fly_event = nullptr;                             // ohp_run_streams_device_flywheel: behind the planned jobs' count
+    uint64_t* h_regions = nullptr;                               // ... the regions' total (pinned; [4..8): sched::FlySlots)
+    // ohp_run_streams_device_flywheel (grown on demand)
+    ohp_starvation* d_records = nullptr; uint64_t d_records_cap = 0; // when the caller passes no record array
+    uint64_t* d_slot = nullptr; uint64_t d_slot_cap = 0;             // flywheel slots, scanned in place
+    uint32_t* d_owner = nullptr; uint64_t d_owner_cap = 0;           // the stream that holds each event
+    ohp::sched::FlySlots* d_fly_slots = nullptr;
+    ohp_chunk_desc* d_fly_descs = nullptr; uint64_t d_fly_descs_cap = 0; // prep, then blocks, per starvation event
+    ohp_flywheel_job* d_fly_jobs = nullptr; uint64_t d_fly_jobs_cap = 0;
+    uint8_t* d_fly_train = nullptr; uint64_t d_fly_train_cap = 0;    // training blocks
+    uint8_t* d_fly_gen = nullptr; uint64_t d_fly_gen_cap = 0;        // generated audio
     std::vector<uint64_t> h_begin, h_outb;
     cudaEvent_t ev_start = nullptr, ev_stop = nullptr;
     bool timing = false;
@@ -402,6 +413,15 @@ static int grow(ohp_context* ctx, T*& ptr, uint64_t& cap, uint64_t need)
     return OHP_OK;
 }
 
+// Device buffers another stream may still be reading: grown only once the device is idle.
+template <class T>
+static int grow_idle(ohp_context* ctx, T*& ptr, uint64_t& cap, uint64_t need)
+{
+    if (need <= cap) return OHP_OK;
+    OHP_CUDA(ctx, cudaDeviceSynchronize());
+    return grow(ctx, ptr, cap, need);
+}
+
 static int schedule_status(ohp_context* ctx, cudaStream_t st)
 {
     // words [2], [3] of the status block belong to the schedule kernels
@@ -620,6 +640,8 @@ int ohp_create(int device, ohp_context** out_ctx)
         OHP_CREATE(cudaFuncSetAttribute(sched::schedule_kernel<true, 32>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(sched::schedule_kernel<false, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(sched::schedule_kernel<true, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        OHP_CREATE(cudaFuncSetAttribute(sched::schedule_record_kernel<32>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        OHP_CREATE(cudaFuncSetAttribute(sched::schedule_record_kernel<1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(sched::scan_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(ramp_convert_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(ramp_convert_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -650,7 +672,12 @@ int ohp_destroy(ohp_context* ctx)
     if (ctx->d_outb) (void)cudaFree(ctx->d_outb);
     if (ctx->d_counts) (void)cudaFree(ctx->d_counts);
     if (ctx->h_regions) (void)cudaFreeHost(ctx->h_regions);
+    for (void* p : {(void*)ctx->d_records, (void*)ctx->d_slot, (void*)ctx->d_owner, (void*)ctx->d_fly_slots, (void*)ctx->d_fly_descs,
+                    (void*)ctx->d_fly_jobs, (void*)ctx->d_fly_train, (void*)ctx->d_fly_gen}) {
+        if (p) (void)cudaFree(p);
+    }
     if (ctx->sched_event) (void)cudaEventDestroy(ctx->sched_event);
+    if (ctx->fly_event) (void)cudaEventDestroy(ctx->fly_event);
     if (ctx->h_status) (void)cudaFreeHost(ctx->h_status);
     if (ctx->ev_start) (void)cudaEventDestroy(ctx->ev_start);
     if (ctx->ev_stop) (void)cudaEventDestroy(ctx->ev_stop);
@@ -1086,10 +1113,11 @@ int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, siz
 // the only host round trip is for the regions' total (bound + scan are a few microseconds of GPU time).
 // A stream that outgrows its region (none of the shapes this repo generates does, the bound is held against the exact
 // counts in tests/test_schedule_walk.py) sends the whole call through the two-pass path.
+// records (ohp_run_streams_device_flywheel): the emitting walk also leaves the starvation records there.
 static int run_streams_device_two_pass(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
                                        const ohp_ramp_event* d_events, size_t n_events,
                                        const uint8_t* d_in, uint64_t in_bytes, uint8_t* d_out, uint64_t out_bytes,
-                                       uint64_t* d_stream_out_bytes, uint64_t* total_chunks, cudaStream_t st)
+                                       uint64_t* d_stream_out_bytes, uint64_t* total_chunks, ohp_starvation* records, cudaStream_t st)
 {
     int rc;
     uint64_t total = 0;
@@ -1100,14 +1128,103 @@ static int run_streams_device_two_pass(ohp_context* ctx, const ohp_stream_spec* 
         OHP_CUDA(ctx, cudaDeviceSynchronize());
         if ((rc = grow(ctx, ctx->d_descs, ctx->d_descs_cap, total * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
     }
-    if ((rc = ohp_schedule_emit_device(ctx, d_streams, n_streams, d_events, n_events, ctx->d_begin, ctx->d_descs, nullptr, st)) != OHP_OK) return rc;
+    if (!records) {
+        if ((rc = ohp_schedule_emit_device(ctx, d_streams, n_streams, d_events, n_events, ctx->d_begin, ctx->d_descs, nullptr, st)) != OHP_OK) return rc;
+    }
+    else {
+        sched::ScheduleParams p{};
+        p.streams = d_streams; p.n_streams = n_streams; p.events = d_events; p.n_events = n_events;
+        p.chunk_begin = ctx->d_begin; p.descs = ctx->d_descs; p.info = nullptr;
+        p.status = ctx->d_status + 2;
+        p.records = records;
+        if (schedule_team(n_streams) == 32) {
+            sched::schedule_record_kernel<32><<<sched::schedule_grid(n_streams, 32), sched::kScheduleBlock, 0, st>>>(p);
+        } else {
+            p.lanes_per_warp = schedule_lanes(ctx, n_streams);
+            sched::schedule_record_kernel<1><<<sched::schedule_grid(n_streams, 1, p.lanes_per_warp), sched::kScheduleBlock, 0, st>>>(p);
+        }
+        OHP_CUDA(ctx, cudaGetLastError());
+        ctx->launches++;
+    }
     return launch(ctx, ctx->d_descs, (size_t)total, d_in, in_bytes, d_out, out_bytes, st);
 }
 
-int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
-                           const ohp_ramp_event* d_events, size_t n_events,
-                           const uint8_t* d_in, uint64_t in_bytes, uint8_t* d_out, uint64_t out_bytes,
-                           uint64_t* d_stream_out_bytes, uint64_t* total_chunks, void* stream)
+// What ohp_run_streams_device_flywheel adds to the call (null: ohp_run_streams_device).
+struct FlyArgs
+{
+    uint8_t* out;
+    uint64_t out_bytes;
+    ohp_starvation* records; // the caller's, or the context's
+    uint64_t* off;
+    uint64_t* len;
+};
+
+// The slots' total is known (h_regions[4..8)): refuse what the call cannot lay out.
+static int fly_check(ohp_context* ctx, const FlyArgs& fly)
+{
+    const sched::FlySlots& fs = *reinterpret_cast<const sched::FlySlots*>(ctx->h_regions + 4);
+    char buf[160];
+    if (fs.shared != 0) {
+        std::snprintf(buf, sizeof buf, "%llu events lie in the slices of two streams: a starvation record needs one stream per event",
+                      (unsigned long long)fs.shared);
+        return fail(ctx, OHP_E_INVALID_ARG, buf);
+    }
+    if (fs.bytes > fly.out_bytes || fs.bytes > sched::kSlotBytesMask || (fs.bytes && !fly.out)) {
+        std::snprintf(buf, sizeof buf, "flywheel output: the starvation events' slots need %llu bytes, d_fly_out holds %llu",
+                      (unsigned long long)fs.bytes, (unsigned long long)(fly.out ? fly.out_bytes : 0));
+        return fail(ctx, OHP_E_OUT_OF_RANGE, buf);
+    }
+    return OHP_OK;
+}
+
+// Plan every starvation event's flywheel ramp from its record (device: nothing but the planned jobs' count comes back,
+// behind ctx->fly_event) ...
+static int fly_plan(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams, size_t n_events, const FlyArgs& fly,
+                    cudaStream_t st)
+{
+    const sched::FlySlots fs = *reinterpret_cast<const sched::FlySlots*>(ctx->h_regions + 4);
+    if (fs.count == 0) return OHP_OK; // not one starvation event: the call is ohp_run_streams_device's, launch for launch
+    const uint64_t per = OHP_FLYWHEEL_MAX_PREP + flyplan::kMaxBlocks;
+    int rc;
+    if ((rc = grow_idle(ctx, ctx->d_fly_descs, ctx->d_fly_descs_cap, fs.count * per * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
+    if ((rc = grow_idle(ctx, ctx->d_fly_jobs, ctx->d_fly_jobs_cap, fs.count * sizeof(ohp_flywheel_job))) != OHP_OK) return rc;
+    if (!ctx->fly_event) OHP_CUDA(ctx, cudaEventCreateWithFlags(&ctx->fly_event, cudaEventDisableTiming));
+    sched::scan_kernel<<<1, sched::kScanThreads, 0, st>>>(ctx->d_slot, n_events);
+    OHP_CUDA(ctx, cudaGetLastError());
+    sched::PlanParams pp;
+    pp.streams = d_streams; pp.n_streams = n_streams; pp.n_events = n_events; pp.records = fly.records; pp.slot = ctx->d_slot;
+    pp.prep = ctx->d_fly_descs; pp.jobs = ctx->d_fly_jobs; pp.blocks = ctx->d_fly_descs + fs.count * OHP_FLYWHEEL_MAX_PREP;
+    pp.fly_off = fly.off; pp.fly_len = fly.len; pp.slots = ctx->d_fly_slots;
+    sched::plan_kernel<<<(unsigned)((n_events + 127) / 128), 128, 0, st>>>(pp);
+    OHP_CUDA(ctx, cudaGetLastError());
+    ctx->launches += 2;
+    OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_regions + 4, ctx->d_fly_slots, sizeof(sched::FlySlots), cudaMemcpyDeviceToHost, st));
+    OHP_CUDA(ctx, cudaEventRecord(ctx->fly_event, st));
+    return OHP_OK;
+}
+
+// ... and play it: FlywheelInput::Prepare (prep), FlywheelRamperManager::Ramp (the compacted jobs), RampGenerator's blocks.
+static int fly_play(ohp_context* ctx, const uint8_t* d_in, uint64_t in_bytes, const FlyArgs& fly, cudaStream_t st)
+{
+    const sched::FlySlots& fs = *reinterpret_cast<const sched::FlySlots*>(ctx->h_regions + 4);
+    if (fs.count == 0) return OHP_OK;
+    OHP_CUDA(ctx, cudaEventSynchronize(ctx->fly_event));
+    const uint64_t count = fs.count, bytes = fs.bytes, planned = fs.planned;
+    int rc;
+    if ((rc = grow_idle(ctx, ctx->d_fly_train, ctx->d_fly_train_cap, bytes)) != OHP_OK) return rc;
+    if ((rc = grow_idle(ctx, ctx->d_fly_gen, ctx->d_fly_gen_cap, bytes)) != OHP_OK) return rc;
+    const ohp_chunk_desc* prep = ctx->d_fly_descs;
+    const ohp_chunk_desc* blocks = ctx->d_fly_descs + count * OHP_FLYWHEEL_MAX_PREP;
+    if ((rc = launch(ctx, prep, (size_t)(count * OHP_FLYWHEEL_MAX_PREP), d_in, in_bytes, ctx->d_fly_train, bytes, st)) != OHP_OK) return rc;
+    if ((rc = ohp_flywheel_device(ctx, ctx->d_fly_jobs, (size_t)planned, ctx->d_fly_train, bytes, ctx->d_fly_gen, bytes, st)) != OHP_OK) return rc;
+    return launch(ctx, blocks, (size_t)(count * flyplan::kMaxBlocks), ctx->d_fly_gen, bytes, fly.out, fly.out_bytes, st);
+}
+
+// The body of ohp_run_streams_device and, with fly, of ohp_run_streams_device_flywheel.
+static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
+                              const ohp_ramp_event* d_events, size_t n_events,
+                              const uint8_t* d_in, uint64_t in_bytes, uint8_t* d_out, uint64_t out_bytes,
+                              uint64_t* d_stream_out_bytes, uint64_t* total_chunks, void* stream, const FlyArgs* fly)
 {
     if (!ctx) return OHP_E_INVALID_ARG;
     if (total_chunks) *total_chunks = 0;
@@ -1118,15 +1235,63 @@ int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, s
     int rc;
     if ((rc = grow(ctx, ctx->d_begin, ctx->d_begin_cap, (uint64_t)(n_streams + 1) * sizeof(uint64_t))) != OHP_OK) return rc;
     if ((rc = grow(ctx, ctx->d_counts, ctx->d_counts_cap, (uint64_t)n_streams * sizeof(uint64_t))) != OHP_OK) return rc;
+    if (!ctx->h_regions) OHP_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void**>(&ctx->h_regions), 8 * sizeof(uint64_t), cudaHostAllocDefault));
+    if (!ctx->sched_event) OHP_CUDA(ctx, cudaEventCreateWithFlags(&ctx->sched_event, cudaEventDisableTiming));
+    ohp_starvation* records = nullptr;
+    if (fly) {
+        // records (none yet: all ones), slots (none: zero), owners (none: all ones), the slots' totals, where the flywheel
+        // audio goes (nowhere yet)
+        records = fly->records;
+        if (!records && (rc = grow_idle(ctx, ctx->d_records, ctx->d_records_cap, (uint64_t)(n_events ? n_events : 1) * sizeof(ohp_starvation))) != OHP_OK) return rc;
+        if (!records) records = ctx->d_records;
+        if ((rc = grow_idle(ctx, ctx->d_slot, ctx->d_slot_cap, (uint64_t)(n_events + 1) * sizeof(uint64_t))) != OHP_OK) return rc;
+        if ((rc = grow_idle(ctx, ctx->d_owner, ctx->d_owner_cap, (uint64_t)(n_events ? n_events : 1) * sizeof(uint32_t))) != OHP_OK) return rc;
+        if (!ctx->d_fly_slots) OHP_CUDA(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->d_fly_slots), sizeof(sched::FlySlots)));
+        OHP_CUDA(ctx, cudaMemsetAsync(ctx->d_fly_slots, 0, sizeof(sched::FlySlots), st));
+        OHP_CUDA(ctx, cudaMemsetAsync(ctx->d_slot, 0, (n_events + 1) * sizeof(uint64_t), st));
+        if (n_events) {
+            OHP_CUDA(ctx, cudaMemsetAsync(records, 0xff, n_events * sizeof(ohp_starvation), st));
+            OHP_CUDA(ctx, cudaMemsetAsync(ctx->d_owner, 0xff, n_events * sizeof(uint32_t), st));
+            OHP_CUDA(ctx, cudaMemsetAsync(fly->off, 0, n_events * sizeof(uint64_t), st));
+            OHP_CUDA(ctx, cudaMemsetAsync(fly->len, 0, n_events * sizeof(uint64_t), st));
+        }
+    }
+    auto bound = [&]() -> int { // regions: bound per stream (and, with fly, the flywheel slots)
+        if (fly) {
+            sched::bound_slots_kernel<<<(unsigned)((n_streams + 127) / 128), 128, 0, st>>>(d_streams, n_streams, d_events, n_events, ctx->d_begin,
+                                                                                        ctx->d_slot, ctx->d_owner, ctx->d_fly_slots);
+        }
+        else {
+            sched::bound_kernel<<<(unsigned)((n_streams + 127) / 128), 128, 0, st>>>(d_streams, n_streams, d_events, n_events, ctx->d_begin);
+        }
+        OHP_CUDA(ctx, cudaGetLastError());
+        return OHP_OK;
+    };
+    // with fly, the flywheel work follows whichever way the bytes were made (planned in front of ramp_convert_kernel where
+    // the one walk made them, so that the host waits for the planned jobs' count while that kernel runs)
+    bool planned = false;
+    auto finish = [&](int aRc) -> int {
+        if (aRc != OHP_OK || !fly) return aRc;
+        if (!planned && (aRc = fly_plan(ctx, d_streams, n_streams, n_events, *fly, st)) != OHP_OK) return aRc;
+        planned = true;
+        return fly_play(ctx, d_in, in_bytes, *fly, st);
+    };
     const char* one_walk_env = std::getenv("OHP_ONE_WALK"); // OHP_ONE_WALK=0: count + scan + emit as in round 1
     const bool one_walk = !one_walk_env || std::atoi(one_walk_env) != 0;
     if (!one_walk) {
-        return run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
-                                           d_stream_out_bytes, total_chunks, st);
+        if (fly) {
+            // the bounds land in d_begin, which the count overwrites
+            if ((rc = bound()) != OHP_OK) return rc;
+            ctx->launches++;
+            OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_regions + 4, ctx->d_fly_slots, sizeof(sched::FlySlots), cudaMemcpyDeviceToHost, st));
+            OHP_CUDA(ctx, cudaStreamSynchronize(st));
+            if ((rc = fly_check(ctx, *fly)) != OHP_OK) return rc;
+        }
+        return finish(run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
+                                                  d_stream_out_bytes, total_chunks, records, st));
     }
     // 1. regions: bound per stream, exclusive scan
-    sched::bound_kernel<<<(unsigned)((n_streams + 127) / 128), 128, 0, st>>>(d_streams, n_streams, d_events, n_events, ctx->d_begin);
-    OHP_CUDA(ctx, cudaGetLastError());
+    if ((rc = bound()) != OHP_OK) return rc;
     sched::scan_kernel<<<1, sched::kScanThreads, 0, st>>>(ctx->d_begin, n_streams);
     OHP_CUDA(ctx, cudaGetLastError());
     ctx->launches += 2;
@@ -1134,9 +1299,8 @@ int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, s
     //    regions add up to -- the total (8 bytes, pinned) comes back while the walk runs, so the host's round trip costs
     //    the GPU nothing.  The walk writes nothing for a stream whose region would end beyond the buffer; if the total says
     //    the buffer was too small (first call of a shape), it grows and the walk runs again.
-    if (!ctx->h_regions) OHP_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void**>(&ctx->h_regions), sizeof(uint64_t), cudaHostAllocDefault));
-    if (!ctx->sched_event) OHP_CUDA(ctx, cudaEventCreateWithFlags(&ctx->sched_event, cudaEventDisableTiming));
     OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_regions, ctx->d_begin + n_streams, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (fly) OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_regions + 4, ctx->d_fly_slots, sizeof(sched::FlySlots), cudaMemcpyDeviceToHost, st));
     OHP_CUDA(ctx, cudaEventRecord(ctx->sched_event, st));
     const int team = schedule_team(n_streams);
     auto walk = [&]() -> int {
@@ -1147,8 +1311,14 @@ int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, s
         p.status = ctx->d_status + 2;
         p.counts_out = ctx->d_counts; p.out_bytes = d_stream_out_bytes;
         p.lanes_per_warp = schedule_lanes(ctx, n_streams);
-        if (team == 32) sched::schedule_kernel<true, 32><<<sched::schedule_grid(n_streams, 32), sched::kScheduleBlock, 0, st>>>(p);
-        else sched::schedule_kernel<true, 1><<<sched::schedule_grid(n_streams, 1, p.lanes_per_warp), sched::kScheduleBlock, 0, st>>>(p);
+        p.records = records;
+        const unsigned grid = team == 32 ? sched::schedule_grid(n_streams, 32) : sched::schedule_grid(n_streams, 1, p.lanes_per_warp);
+        if (records) {
+            if (team == 32) sched::schedule_record_kernel<32><<<grid, sched::kScheduleBlock, 0, st>>>(p);
+            else sched::schedule_record_kernel<1><<<grid, sched::kScheduleBlock, 0, st>>>(p);
+        }
+        else if (team == 32) sched::schedule_kernel<true, 32><<<grid, sched::kScheduleBlock, 0, st>>>(p);
+        else sched::schedule_kernel<true, 1><<<grid, sched::kScheduleBlock, 0, st>>>(p);
         OHP_CUDA(ctx, cudaGetLastError());
         ctx->launches++;
         return OHP_OK;
@@ -1156,10 +1326,15 @@ int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, s
     if (ctx->d_descs_cap >= sizeof(ohp_chunk_desc) && (rc = walk()) != OHP_OK) return rc; // (no buffer yet: after the total)
     OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_event));
     const uint64_t regions = *ctx->h_regions;
+    if (fly && (rc = fly_check(ctx, *fly)) != OHP_OK) return rc;
     if (regions > ctx->d_descs_cap / sizeof(ohp_chunk_desc)) {
         OHP_CUDA(ctx, cudaDeviceSynchronize()); // the buffer may still be read by a launch enqueued earlier on another stream
         if ((rc = grow(ctx, ctx->d_descs, ctx->d_descs_cap, regions * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
         if ((rc = walk()) != OHP_OK) return rc;
+    }
+    if (fly) {
+        if ((rc = fly_plan(ctx, d_streams, n_streams, n_events, *fly, st)) != OHP_OK) return rc;
+        planned = true;
     }
     if (total_chunks) {
         // the exact number of playables, and what the walk refused: in front of ramp_convert_kernel in the stream, so the
@@ -1170,7 +1345,7 @@ int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, s
         OHP_CUDA(ctx, cudaEventRecord(ctx->sched_event, st));
     }
     if ((rc = launch(ctx, ctx->d_descs, (size_t)regions, d_in, in_bytes, d_out, out_bytes, st)) != OHP_OK) return rc;
-    if (!total_chunks) return OHP_OK;
+    if (!total_chunks) return finish(OHP_OK);
     OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_event));
     const uint32_t bits = ctx->h_status[2];
     if (bits != 0) {
@@ -1180,15 +1355,41 @@ int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, s
         const uint32_t refused = (1u << sched::kErrSpec) | (1u << sched::kErrAssert);
         if ((bits & (1u << sched::kErrBound)) && !(bits & refused)) {
             (void)read_status(ctx, st);
-            return run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
-                                               d_stream_out_bytes, total_chunks, st);
+            return finish(run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
+                                                      d_stream_out_bytes, total_chunks, records, st));
         }
         if (src != OHP_OK) return src;
     }
     uint64_t total = 0;
     for (size_t s = 0; s < n_streams; s++) total += ctx->h_outb[s];
     *total_chunks = total;
-    return OHP_OK;
+    return finish(OHP_OK);
+}
+
+int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
+                           const ohp_ramp_event* d_events, size_t n_events,
+                           const uint8_t* d_in, uint64_t in_bytes, uint8_t* d_out, uint64_t out_bytes,
+                           uint64_t* d_stream_out_bytes, uint64_t* total_chunks, void* stream)
+{
+    return run_streams_device(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
+                              d_stream_out_bytes, total_chunks, stream, nullptr);
+}
+
+int ohp_run_streams_device_flywheel(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
+                                    const ohp_ramp_event* d_events, size_t n_events,
+                                    const uint8_t* d_in, uint64_t in_bytes, uint8_t* d_out, uint64_t out_bytes,
+                                    uint8_t* d_fly_out, uint64_t fly_out_bytes, ohp_starvation* d_starvations,
+                                    uint64_t* d_fly_off, uint64_t* d_fly_len, uint64_t* d_stream_out_bytes,
+                                    uint64_t* total_chunks, void* stream)
+{
+    if (!ctx) return OHP_E_INVALID_ARG;
+    if (n_events && (!d_fly_off || !d_fly_len)) {
+        if (total_chunks) *total_chunks = 0;
+        return fail(ctx, OHP_E_INVALID_ARG, "null device pointer (d_fly_off / d_fly_len)");
+    }
+    const FlyArgs fly{d_fly_out, d_fly_out ? fly_out_bytes : 0, d_starvations, d_fly_off, d_fly_len};
+    return run_streams_device(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
+                              d_stream_out_bytes, total_chunks, stream, &fly);
 }
 
 int ohp_fill_streams_device(ohp_context* ctx, uint8_t* d_in, uint64_t in_bytes, const ohp_stream_spec* d_streams,

@@ -12,6 +12,7 @@
 #include <cuda_runtime.h>
 
 #include "../host/schedule_walk.h"
+#include "../host/flywheel_plan.h"
 
 namespace ohp {
 namespace sched {
@@ -32,6 +33,7 @@ struct ScheduleParams
     uint64_t* counts_out;      // [n_streams] exact playables per stream (null: two-pass mode)
     uint64_t descs_cap;        // descriptors the buffer holds; a stream whose region would end beyond writes nothing (0: no check)
     uint32_t lanes_per_warp;   // TEAM = 1: streams a warp walks (its first lanes, one each; the others idle); 0 = 32
+    ohp_starvation* records;   // schedule_record_kernel: [n_events], the record of event e at [e]
 };
 
 constexpr uint32_t kErrBound = 4u; // a stream has more playables than stream_chunk_bound allowed for: the caller takes two passes
@@ -52,8 +54,8 @@ __global__ void __launch_bounds__(128) bound_kernel(const ohp_stream_spec* __res
 #ifndef OHP_SCHED_MIN_BLOCKS
 #define OHP_SCHED_MIN_BLOCKS 3 /* <= 168 registers.  The walk times of DESIGN 4.2 were measured with this bound; 5 (96 registers) spills. */
 #endif
-template <bool EMIT, int TEAM>
-__global__ void __launch_bounds__(128, OHP_SCHED_MIN_BLOCKS) schedule_kernel(const ScheduleParams p)
+template <bool EMIT, int TEAM, bool RECORD>
+__device__ __forceinline__ void schedule_body(const ScheduleParams p)
 {
     const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     uint64_t s = t / TEAM;
@@ -74,7 +76,8 @@ __global__ void __launch_bounds__(128, OHP_SCHED_MIN_BLOCKS) schedule_kernel(con
     //  second launch that follows when that turns out to be the case)
     if (regions && p.descs_cap != 0 && p.chunk_begin[s + 1] > p.descs_cap) return;
     const uint64_t limit = regions ? p.chunk_begin[s + 1] - p.chunk_begin[s] : ~0ull;
-    uint32_t rc = run_stream<EMIT, TEAM, true>(sp, p.events, p.n_events, descs, info, nChunks, outBytes, lane, limit);
+    uint32_t rc = run_stream<EMIT, TEAM, true, RECORD>(sp, p.events, p.n_events, descs, info, nChunks, outBytes, lane, limit,
+                                                       RECORD ? p.records + sp.first_event : nullptr, s);
     if (regions) {
         if (rc == kOk && nChunks > limit) rc = kErrBound;
         // the rest of the region: zero-byte descriptors (all lanes of the team, two 128-bit stores each)
@@ -95,6 +98,121 @@ __global__ void __launch_bounds__(128, OHP_SCHED_MIN_BLOCKS) schedule_kernel(con
         p.counts_out[s] = rc == kOk ? nChunks : 0;
         if (p.out_bytes) p.out_bytes[s] = outBytes;
     }
+}
+
+template <bool EMIT, int TEAM>
+__global__ void __launch_bounds__(128, OHP_SCHED_MIN_BLOCKS) schedule_kernel(const ScheduleParams p)
+{
+    schedule_body<EMIT, TEAM, false>(p);
+}
+
+// The emitting walk that also leaves a starvation record per OHP_EV_STARVATION it applies (ohp_run_streams_device_flywheel).
+template <int TEAM>
+__global__ void __launch_bounds__(128, OHP_SCHED_MIN_BLOCKS) schedule_record_kernel(const ScheduleParams p)
+{
+    schedule_body<true, TEAM, true>(p);
+}
+
+// FLYWHEEL SLOTS.  Event e's flywheel audio goes to a slot of align16(ToSamples(20 ms) x frame bytes) of its stream; the
+// slots lie back to back in event order.  slot[e] (n_events + 1 entries, zeroed by the caller) is scanned in place into
+// offsets afterwards; it carries the slot's bytes in its low kSlotCountShift bits and a 1 above them for every starvation
+// event, so that the scan also numbers the starvation events (their descriptor regions).
+constexpr int kSlotCountShift = 40;
+constexpr uint64_t kSlotBytesMask = (1ull << kSlotCountShift) - 1;
+
+struct FlySlots
+{
+    uint64_t bytes;     // slots' total
+    uint64_t count;     // starvation events in the streams' slices
+    uint64_t shared;    // events that two streams' slices both hold
+    uint64_t planned;   // plan_kernel: jobs in the compacted job list
+};
+
+OHP_HD uint64_t fly_slot_bytes(const ohp_stream_spec& sp)
+{
+    const uint32_t jps = core::jiffies_per_sample_or_zero(sp.sample_rate);
+    if (jps == 0) return 0; // the walk refuses the stream
+    const uint64_t bytes = (uint64_t)(OHP_FLYWHEEL_RAMP_JIFFIES / jps) * sp.channels * (sp.bit_depth / 8u);
+    return (bytes + 15u) & ~15ull;
+}
+
+// bound_kernel and the slots in one pass over the streams.  owner[e] (all ones from the caller) takes the stream that holds
+// event e: a second stream holding it is counted in slots->shared.
+__global__ void __launch_bounds__(128) bound_slots_kernel(const ohp_stream_spec* __restrict__ streams, uint64_t n_streams,
+                                                          const ohp_ramp_event* __restrict__ events, uint64_t n_events,
+                                                          uint64_t* __restrict__ bound, uint64_t* __restrict__ slot,
+                                                          uint32_t* __restrict__ owner, FlySlots* __restrict__ slots)
+{
+    const uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= n_streams) return;
+    const ohp_stream_spec sp = streams[s];
+    bound[s] = stream_chunk_bound(sp, events, n_events);
+    const uint64_t first = sp.first_event;
+    const uint64_t end = first + sp.num_events < n_events ? first + sp.num_events : n_events;
+    const uint64_t size = fly_slot_bytes(sp);
+    uint64_t bytes = 0, count = 0, shared = 0;
+    for (uint64_t e = first; e < end; e++) {
+        if (atomicCAS(&owner[e], 0xffffffffu, (uint32_t)s) != 0xffffffffu) shared++;
+        if (events[e].op != OHP_EV_STARVATION) continue;
+        slot[e] = (1ull << kSlotCountShift) | size;
+        bytes += size;
+        count++;
+    }
+    if (bytes | count) {
+        atomicAdd(reinterpret_cast<unsigned long long*>(&slots->bytes), (unsigned long long)bytes);
+        atomicAdd(reinterpret_cast<unsigned long long*>(&slots->count), (unsigned long long)count);
+    }
+    if (shared) atomicAdd(reinterpret_cast<unsigned long long*>(&slots->shared), (unsigned long long)shared);
+}
+
+// One thread per event: where its flywheel audio goes (fly_off, fly_len) and, for the k-th starvation event, the
+// descriptors of two of the three launches in fixed regions -- prep[k * OHP_FLYWHEEL_MAX_PREP ...], blocks[k *
+// flyplan::kMaxBlocks ...] -- planned from its record (flyplan::plan); whatever a region does not use is zero (empty
+// descriptors).  Jobs go to a compacted list (slots->planned of them, in no particular order: each writes its own slot),
+// so that a starvation that is not played runs no flywheel job.  The training block and the generated audio take the same
+// offsets in the two scratch arenas as the output in the caller's (a training block is at most a fifth of its slot).
+struct PlanParams
+{
+    const ohp_stream_spec* streams;
+    uint64_t n_streams;
+    uint64_t n_events;
+    const ohp_starvation* records;
+    const uint64_t* slot;      // scanned: [n_events + 1]
+    ohp_chunk_desc* prep;
+    ohp_flywheel_job* jobs;
+    ohp_chunk_desc* blocks;
+    uint64_t* fly_off;
+    uint64_t* fly_len;
+    FlySlots* slots;
+};
+
+__global__ void __launch_bounds__(128) plan_kernel(const PlanParams p)
+{
+    const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= p.n_events) return;
+    const uint64_t here = p.slot[e], next = p.slot[e + 1];
+    const uint64_t off = here & kSlotBytesMask;
+    p.fly_off[e] = off;
+    p.fly_len[e] = 0;
+    if ((next >> kSlotCountShift) == (here >> kSlotCountShift)) return; // not a starvation event of a stream
+    const uint64_t k = here >> kSlotCountShift;
+    ohp_chunk_desc* prep = p.prep + k * OHP_FLYWHEEL_MAX_PREP;
+    ohp_chunk_desc* blocks = p.blocks + k * flyplan::kMaxBlocks;
+    ohp_flywheel_job job;
+    uint32_t nPrep = 0, nBlocks = 0;
+    const ohp_starvation rec = p.records[e];
+    if (rec.event == e && rec.stream < p.n_streams) {
+        const ohp_stream_spec sp = p.streams[rec.stream];
+        if (flyplan::plan(sp, rec, off, off, off, prep, nPrep, job, blocks, nBlocks) == OHP_OK) {
+            p.fly_len[e] = (uint64_t)job.out_frames * sp.channels * (sp.bit_depth / 8u);
+            p.jobs[atomicAdd(reinterpret_cast<unsigned long long*>(&p.slots->planned), 1ull)] = job;
+        }
+        else {
+            nPrep = nBlocks = 0;
+        }
+    }
+    for (uint32_t i = nPrep; i < OHP_FLYWHEEL_MAX_PREP; i++) prep[i] = flyplan::zero_desc();
+    for (uint32_t i = nBlocks; i < flyplan::kMaxBlocks; i++) blocks[i] = flyplan::zero_desc();
 }
 
 // threads per block; grid for n streams

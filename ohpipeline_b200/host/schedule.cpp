@@ -223,6 +223,7 @@ int ohp_schedule_build_walk(const ohp_stream_spec* streams, size_t n_streams, co
     sch->chunkBegin.assign(n_streams + 1, 0);
     sch->outBytes.assign(n_streams, 0);
     std::vector<uint32_t> rcs(n_streams, 0);
+    std::vector<std::vector<ohp_starvation>> starved(n_streams); // the emitting walk's records, stream by stream
     auto run = [&](bool emit) {
         auto worker = [&](int t) {
             const size_t lo = n_streams * (size_t)t / (size_t)threads;
@@ -230,8 +231,12 @@ int ohp_schedule_build_walk(const ohp_stream_spec* streams, size_t n_streams, co
             for (size_t s = lo; s < hi; s++) {
                 uint64_t n = 0, bytes = 0;
                 if (emit) {
-                    rcs[s] = sched::run_stream<true>(streams[s], events, n_events, sch->chunks.data() + sch->chunkBegin[s],
-                                                     sch->info.data() + sch->chunkBegin[s], n, bytes);
+                    starved[s].resize(streams[s].num_events);
+                    uint32_t nRec = 0;
+                    rcs[s] = sched::run_stream<true, 1, true, true>(streams[s], events, n_events, sch->chunks.data() + sch->chunkBegin[s],
+                                                                    sch->info.data() + sch->chunkBegin[s], n, bytes, 0, ~0ull,
+                                                                    starved[s].data(), s, true, &nRec);
+                    starved[s].resize(nRec);
                 }
                 else {
                     rcs[s] = sched::run_stream<false>(streams[s], events, n_events, nullptr, nullptr, n, bytes);
@@ -264,6 +269,10 @@ int ohp_schedule_build_walk(const ohp_stream_spec* streams, size_t n_streams, co
     sch->chunks.resize(sch->chunkBegin[n_streams]);
     sch->info.resize(sch->chunkBegin[n_streams]);
     run(true);
+    for (size_t s = 0; s < n_streams; s++) {
+        sch->starvations.insert(sch->starvations.end(), starved[s].begin(), starved[s].end());
+    }
+    sch->recentBegin.assign(sch->starvations.size() + 1, 0); // records without the recent audio's pieces
     *out = sch;
     return OHP_OK;
 }

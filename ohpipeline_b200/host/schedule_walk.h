@@ -99,6 +99,15 @@ struct Stage
     uint32_t halted;   // Muter::iHalted / StarvationRamper Halted-or-Starting: no PCM has passed since the start or the last halt
 };
 
+// What stage_chain.h keeps per stage for a StarvationRamper's records (RECORD walks only; see note_starvation).
+struct Starve
+{
+    uint64_t pcmJiffies; // PCM that has passed the stage
+    uint64_t pcmRun;     // ... its latest unbroken run: nothing but PCM of one attenuation (pcmRunAtt) since the stream began,
+    uint32_t pcmRunAtt;  // a MsgSilence passed or a flywheel ramp used the recent audio up
+    uint32_t elemRamp;   // what the element's own SetRamp calls last returned (StarvationRamper::iCurrentRampValue)
+};
+
 struct StreamCtx
 {
     const ohp_ramp_event* ev;
@@ -113,6 +122,12 @@ struct StreamCtx
     ohp_chunk_desc* descs; // EMIT: this stream's first descriptor
     ohp_chunk_info* info;  // EMIT, may be null
     uint64_t limit;        // EMIT: descriptors this stream may write (its region when regions come from stream_chunk_bound)
+    // RECORD: one ohp_starvation per OHP_EV_STARVATION applied -- at rec[event] (event: index in this stream's slice), or
+    // appended at rec[nRec++] where recAppend is set (the host twin keeps them in the order ohp_schedule_build does)
+    ohp_starvation* rec;
+    uint32_t recAppend, nRec;
+    uint64_t stream, firstEvent;
+    Starve sv[kStages];
 };
 
 // MsgAudio::Split (+ SplitCompleted): m keeps the first aJiffies, rest gets what follows.
@@ -431,6 +446,27 @@ OHP_HD bool apply_event(Stage& s, uint32_t op, uint32_t arg)
     return true;
 }
 
+// stage_chain.h NoteStarvation(): called in front of every event a stage applies
+OHP_HD void note_starvation(StreamCtx& cx, const Stage& s, uint32_t stage, uint32_t aEvent)
+{
+    if (s.elem != ElemStarvation || cx.ev[aEvent].op != OHP_EV_STARVATION) return;
+    const bool plays = (s.mode == Running && !s.halted) || (s.mode == RampingUp && s.current != core::kRampMin); // as apply_element_event
+    Starve& r = cx.sv[stage];
+    if (cx.lane == 0 && cx.rec) {
+        ohp_starvation o;
+        o.stream = cx.stream;
+        o.pcm_jiffies = r.pcmJiffies;
+        o.event = (uint32_t)(cx.firstEvent + aEvent);
+        o.ramp = r.elemRamp;
+        o.plays = plays ? 1u : 0u;
+        o.recent_jiffies = r.pcmRun > 0xffffffffull ? 0xffffffffu : (uint32_t)r.pcmRun;
+        o.attenuation = r.pcmRunAtt;
+        o.reserved = 0;
+        cx.rec[cx.recAppend ? cx.nRec++ : aEvent] = o;
+    }
+    if (plays) { r.pcmRun = 0; r.elemRamp = core::kRampMin; } // Pull(): FlywheelRamping -> RampingUp from kMin
+}
+
 OHP_HD bool push_msg(Stage& s, Packed* aRow, const Msg& m)
 {
     if (s.depth == (uint32_t)kStackDepth) return false;
@@ -439,9 +475,12 @@ OHP_HD bool push_msg(Stage& s, Packed* aRow, const Msg& m)
 }
 
 // stage_chain.h Process(): one message through one stage; split remainders go onto the stage's stack (aRow).
-OHP_HD uint32_t stage_process(const StreamCtx& cx, Stage& s, uint32_t stage, Packed* aRow, Msg& msg)
+// RECORD: aAttUp is the attenuation the stages in front of this one leave PCM with (their last that is not unity).
+template <bool RECORD>
+OHP_HD uint32_t stage_process(StreamCtx& cx, Stage& s, uint32_t stage, Packed* aRow, Msg& msg, uint32_t aAttUp)
 {
     while (s.nextAt <= s.pos) {
+        if (RECORD) note_starvation(cx, s, stage, s.nextEv);
         const ohp_ramp_event& e = cx.ev[s.nextEv];
         if (!apply_event(s, e.op, e.arg)) return kErrAssert;
         stage_seek(cx, s, stage, s.nextEv + 1);
@@ -451,6 +490,7 @@ OHP_HD uint32_t stage_process(const StreamCtx& cx, Stage& s, uint32_t stage, Pac
         uint32_t at = (uint32_t)(s.nextAt - s.pos);
         if (msg.silence) at -= at % cx.jps; // silence only splits on sample blocks
         if (at == 0) {
+            if (RECORD) note_starvation(cx, s, stage, s.nextEv);
             const ohp_ramp_event& e = cx.ev[s.nextEv];
             if (!apply_event(s, e.op, e.arg)) return kErrAssert;
             stage_seek(cx, s, stage, s.nextEv + 1);
@@ -473,6 +513,7 @@ OHP_HD uint32_t stage_process(const StreamCtx& cx, Stage& s, uint32_t stage, Pac
     if (s.elem != Generic) {
         if (msg.silence) { // the element reacts, the message is handed on untouched
             element_sees_silence(s);
+            if (RECORD) cx.sv[stage].pcmRun = 0;
             s.pos += msg.size;
             return kOk;
         }
@@ -490,6 +531,7 @@ OHP_HD uint32_t stage_process(const StreamCtx& cx, Stage& s, uint32_t stage, Pac
             const uint32_t e = msg_set_ramp(msg, s.current, s.remaining, s.mode == RampingDown ? core::kDirDown : core::kDirUp,
                                             rest, haveSplit, s.current, cx.jps);
             if (e != kOk) return e;
+            if (RECORD) cx.sv[stage].elemRamp = s.current;
             if (haveSplit && !push_msg(s, aRow, rest)) return kErrDepth;
         }
         if (s.remaining == 0) {
@@ -501,6 +543,14 @@ OHP_HD uint32_t stage_process(const StreamCtx& cx, Stage& s, uint32_t stage, Pac
         core::ramp_set_muted(msg.ramp);
     }
     s.pos += msg.size;
+    if (RECORD && !msg.silence && s.elem == ElemStarvation) {
+        // the attenuation the message carries (stage_chain.h Process(): the stages up to this one are as it left them)
+        Starve& r = cx.sv[stage];
+        const uint32_t att = s.attenuation != OHP_UNITY_ATTENUATION ? s.attenuation : aAttUp;
+        if (att != r.pcmRunAtt) { r.pcmRun = 0; r.pcmRunAtt = att; }
+        r.pcmJiffies += msg.size;
+        r.pcmRun += msg.size;
+    }
     return kOk;
 }
 
@@ -604,7 +654,9 @@ OHP_HD uint32_t next_message(core::CodecSource& src, Lookahead& la)
 // Returns n; 0 means "take the general path for the next message".  What the reference would ASSERT on in the stages
 // is left for the general path to find, at the same message; aErr only reports an ASSERT inside MsgPlayable::Split.
 // UNIFORM: src.read == 0 (compiled separately so that the uniform case pays nothing for the ragged one's tests).
-template <bool EMIT, int STRIDE, bool UNIFORM>
+// RECORD: the StarvationRamper stages' PCM counters advance by the run (no event falls inside it, no MsgSilence either);
+// the element's ramp value follows the recurrence where it is the stage that ramps.
+template <bool EMIT, int STRIDE, bool UNIFORM, bool RECORD>
 OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[kStages], core::CodecSource& src, Lookahead& la,
                           Cursor& cur, uint32_t& aErr)
 {
@@ -630,6 +682,7 @@ OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[
     // stages: what mode, which one ramps, what attenuation the messages leave with, how far the next event is
     uint32_t ramping = 0, muted = 0, atten = OHP_UNITY_ATTENUATION;
     uint32_t rMode = Running, rCurrent = 0, rRemaining = 0;
+    uint32_t rLast = 0; // RECORD: what the last message's SetRamp returned (rCurrent before a completed ramp flips it)
     uint64_t eventRoom = kNever;     // jiffies that can pass every stage before its next event
     uint32_t sizeCap = 0xffffffffu;  // the tightest OHP_EV_MAX_MSG_JIFFIES in force
 #if defined(__CUDA_ARCH__)
@@ -742,6 +795,7 @@ OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[
         }
         n = done;
         if (n == 0) return 0;
+        rLast = rCurrent;
     }
     else if (!uniform) {
         const uint32_t dir = rMode == RampingDown ? core::kDirDown : core::kDirUp;
@@ -763,6 +817,7 @@ OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[
                 const uint32_t e = msg_set_ramp(t, rCurrent, remaining, dir, rest, haveSplit, current, cx.jps);
                 if (e != kOk || haveSplit) break;
                 rRemaining = remaining; rCurrent = current;
+                rLast = current;
                 ramp = t.ramp;
             }
             else {
@@ -853,6 +908,20 @@ OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[
     for (int i = 0; i < kStages; i++) {
         Stage& s = st[i];
         s.pos += posJiffies;
+        if (RECORD && s.elem == ElemStarvation) {
+            Starve& r = cx.sv[i];
+            if ((s.mode == RampingDown || s.mode == RampingUp)) r.elemRamp = rLast;
+            uint32_t att = OHP_UNITY_ATTENUATION;
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+            for (int j = 0; j <= i; j++) {
+                if (st[j].attenuation != OHP_UNITY_ATTENUATION) att = st[j].attenuation;
+            }
+            if (att != r.pcmRunAtt) { r.pcmRun = 0; r.pcmRunAtt = att; }
+            r.pcmJiffies += posJiffies;
+            r.pcmRun += posJiffies;
+        }
         if (s.mode == RampingDown || s.mode == RampingUp) { s.mode = rMode; s.current = rCurrent; s.remaining = rRemaining; }
         if (s.elem != Generic) s.halted = 0; // PCM has passed
     }
@@ -864,7 +933,7 @@ OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[
 // the remaining stages (in registers), hand it to the driver, then resume with the top of the deepest non-empty stack.
 // A team of STRIDE threads (device: a warp, or 1; host: 1) walks the stream holding identical state; they differ only
 // in cx.lane, i.e. in which messages of a bulk step they emit.  BULK = false is the message-at-a-time walk alone.
-template <bool EMIT, int STRIDE, bool BULK>
+template <bool EMIT, int STRIDE, bool BULK, bool RECORD>
 OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
 {
     Packed stack[kStages][kStackDepth];
@@ -877,6 +946,7 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
         st[i].attenuation = OHP_UNITY_ATTENUATION; st[i].depth = 0;
         st[i].elem = stage_element(cx, (uint32_t)i);
         st[i].halted = 1;
+        if (RECORD) { cx.sv[i].pcmJiffies = 0; cx.sv[i].pcmRun = 0; cx.sv[i].pcmRunAtt = OHP_UNITY_ATTENUATION; cx.sv[i].elemRamp = core::kRampMax; }
         if (st[i].elem == ElemStarvation) st[i].maxMsg = 5u * OHP_JIFFIES_PER_MS; // kMaxAudioOutJiffies, StarvationRamper.cpp:376
         stage_seek(cx, st[i], (uint32_t)i, 0);
     }
@@ -894,14 +964,16 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
         Msg m = first;
         int from = 0;
         for (;;) {
+            uint32_t attUp = OHP_UNITY_ATTENUATION;
 #if defined(__CUDA_ARCH__)
 #pragma unroll
 #endif
             for (int i = 0; i < kStages; i++) {
                 if (i >= from) {
-                    const uint32_t e = stage_process(cx, st[i], (uint32_t)i, stack[i], m);
+                    const uint32_t e = stage_process<RECORD>(cx, st[i], (uint32_t)i, stack[i], m, attUp);
                     if (e != kOk) return e;
                 }
+                if (RECORD && st[i].attenuation != OHP_UNITY_ATTENUATION) attUp = st[i].attenuation;
             }
             const uint32_t e2 = drive<EMIT>(cx, m);
             if (e2 != kOk) return e2;
@@ -931,8 +1003,8 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
     for (;;) {
         if (BULK) {
             uint32_t e;
-            const uint32_t n = source.read == 0 ? bulk_step<EMIT, STRIDE, true>(sp, cx, st, source, la, cur, e)
-                                                : bulk_step<EMIT, STRIDE, false>(sp, cx, st, source, la, cur, e);
+            const uint32_t n = source.read == 0 ? bulk_step<EMIT, STRIDE, true, RECORD>(sp, cx, st, source, la, cur, e)
+                                                : bulk_step<EMIT, STRIDE, false, RECORD>(sp, cx, st, source, la, cur, e);
             if (e != kOk) return e;
 #ifdef OHP_WALK_STATS
             if (n != 0) { g_bulk_calls++; g_bulk_msgs += n; }
@@ -966,15 +1038,34 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
         cur.frame += frames;
         cur.srcJiffies += (uint64_t)frames * cx.jps;
     }
+    if (RECORD) {
+        // stage_chain.h Run(): a reservoir that runs dry exactly where the stream ends still starves its StarvationRamper
+        // (no message is left for the event to be applied in front of)
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+        for (int i = 0; i < kStages; i++) {
+            Stage& s = st[i];
+            while (s.elem == ElemStarvation && s.nextAt <= s.pos) {
+                note_starvation(cx, s, (uint32_t)i, s.nextEv);
+                const ohp_ramp_event& e = cx.ev[s.nextEv];
+                (void)apply_element_event(s, e.op, e.arg); // OHP_EV_HALT / OHP_EV_STARVATION: state only
+                stage_seek(cx, s, (uint32_t)i, s.nextEv + 1);
+            }
+        }
+    }
     return kOk;
 }
 
 // Fill the per-stream context from a spec and walk it.  aEvents is the WHOLE events array (aNumEvents entries).
 // aLane: this thread's index in its team of STRIDE (0 on the host).
-template <bool EMIT, int STRIDE = 1, bool BULK = true>
+// RECORD: starvation records go to aRec -- the record of the stream's k-th event at aRec[k] (aRec: the stream's first
+// event's place in an array over the whole events array), or, with aAppend, one after the other; aNumRecords counts them.
+template <bool EMIT, int STRIDE = 1, bool BULK = true, bool RECORD = false>
 OHP_HD uint32_t run_stream(const ohp_stream_spec& sp, const ohp_ramp_event* aEvents, uint64_t aNumEvents,
                            ohp_chunk_desc* aDescs, ohp_chunk_info* aInfo, uint64_t& aNumChunks, uint64_t& aOutBytes,
-                           uint32_t aLane = 0, uint64_t aLimit = ~0ull)
+                           uint32_t aLane = 0, uint64_t aLimit = ~0ull,
+                           ohp_starvation* aRec = nullptr, uint64_t aStream = 0, bool aAppend = false, uint32_t* aNumRecords = nullptr)
 {
     aNumChunks = 0;
     aOutBytes = 0;
@@ -998,7 +1089,15 @@ OHP_HD uint32_t run_stream(const ohp_stream_spec& sp, const ohp_ramp_event* aEve
     cx.descs = EMIT ? aDescs : nullptr;
     cx.info = EMIT ? aInfo : nullptr;
     cx.limit = aLimit;
-    const uint32_t rc = walk_stream<EMIT, STRIDE, BULK>(sp, cx);
+    if (RECORD) {
+        cx.rec = aRec;
+        cx.recAppend = aAppend ? 1u : 0u;
+        cx.nRec = 0;
+        cx.stream = aStream;
+        cx.firstEvent = sp.first_event;
+    }
+    const uint32_t rc = walk_stream<EMIT, STRIDE, BULK, RECORD>(sp, cx);
+    if (RECORD && aNumRecords) *aNumRecords = cx.nRec;
     if (rc != kOk) return rc;
     aNumChunks = cx.nChunks;
     aOutBytes = cx.outBytes;
