@@ -9,7 +9,8 @@ import numpy as np
 import pytest
 
 from ohpipeline_b200 import abi, capi
-from flywheel_util import SHAPES, training_block, train_frames
+from flywheel_util import (DEPTHS, RATES, SHAPES, accepted_shapes, every_shape_streams, shape_split, training_block,
+                           train_frames)
 from util import make_desc
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "flywheel.npz")
@@ -103,6 +104,76 @@ def test_host_ramp_chunks_match_oracle(port):
             assert np.array_equal(got, want), (rate, ch, bits, start)
             assert gfinal == wfinal
             assert int(abi.chunk_out_bytes(got).sum()) == int(job["out_frames"][0]) * ch * bits // 8
+
+
+def test_validate_accepts_exactly_what_the_oracle_plays(port):
+    """ohp_flywheel_validate (and the kernel, which shares check_job) against the oracle's own refusals: every rate x depth
+    x 0-10 channels, a training block a frame short or long, and 0 or 1 frames of output."""
+    n = accepted = 0
+    for rate in RATES:
+        for bits in DEPTHS:
+            for ch in range(0, 11):
+                base = capi.flywheel_job(rate, ch, bits)
+                variants = [base]
+                for field, value in (("train_frames", train_frames(rate) - 1), ("train_frames", train_frames(rate) + 1),
+                                     ("out_frames", 0), ("out_frames", 1)):
+                    v = base.copy()
+                    v[field] = value
+                    variants.append(v)
+                for job in variants:
+                    in_bytes = int(job["train_frames"][0]) * 4 * ch
+                    out_bytes = int(job["out_frames"][0]) * ch * bits // 8
+                    ok = capi.flywheel_validate(job, in_bytes, out_bytes)[0] == abi.OK
+                    rc, _ = port.flywheel(job, np.zeros(max(in_bytes, 1), np.uint8)[:in_bytes], out_bytes)
+                    assert ok == (rc == 0), (rate, ch, bits, job)
+                    n += 1
+                    accepted += ok
+    assert n == 18 * 4 * 11 * 5
+    # 550 shapes as StarvationRamper asks for them, and the same shapes with 0 or 1 frames of output
+    assert accepted == 3 * 550
+
+
+def test_host_ramp_chunks_match_oracle_at_every_shape(port):
+    """test_host_ramp_chunks_match_oracle at every shape the flywheel plays: 550 shapes x 7 start values."""
+    for rate, ch, bits in accepted_shapes():
+        job = capi.flywheel_job(rate, ch, bits, src_off=4096, dst_off=123)
+        for start in (abi.RAMP_MAX, 16383, 12345, 4097, 100, 1, 0):
+            want, wfinal = port.flywheel_ramp_chunks(job, start, 4096, 123)
+            assert want is not None, (rate, ch, bits, start)
+            got, gfinal = capi.flywheel_ramp_chunks(job, start, 4096, 123)
+            assert np.array_equal(got, want), (rate, ch, bits, start)
+            assert gfinal == wfinal, (rate, ch, bits, start)
+            assert int(abi.chunk_out_bytes(got).sum()) == int(job["out_frames"][0]) * ch * bits // 8
+
+
+def test_every_shape_streams_records_and_plan(port):
+    """flywheel_util.every_shape_streams(): the class-free walk records what the class model records, field by field; every
+    record plays; the host planner plans exactly the records at accepted shapes, two per shape, splits training blocks
+    across messages, and plans the oracle's ramped blocks."""
+    w = every_shape_streams()
+    assert len(w.streams) == 576
+    want = capi.schedule_build(w.streams, w.events).starvations
+    got = capi.schedule_build(w.streams, w.events, walk=True).starvations
+    assert len(got) == len(want) == 1152
+    for f in abi.STARVATION.names:
+        assert np.array_equal(got[f], want[f]), f
+    assert np.all(want["plays"] == 1)
+    b = capi.flywheel_plan_batch(w.streams, want)
+    assert len(b.planned) == len(b.jobs) == 1100
+    shape = lambda k: tuple(int(w.streams[int(want["stream"][k])][f]) for f in ("sample_rate", "channels", "bit_depth"))  # noqa: E731
+    accepted, refused = shape_split()
+    planned = [shape(int(k)) for k in b.planned]
+    assert sorted(planned) == sorted(accepted * 2)
+    unplanned = sorted(set(range(len(want))) - set(int(k) for k in b.planned))
+    assert sorted(shape(k) for k in unplanned) == sorted(refused * 2)
+    assert len(b.prep) == 2464
+    # the blocks the host planner plans are the oracle's RampGenerator blocks, job by job
+    blocks = []
+    for i, k in enumerate(b.planned):
+        d, _ = port.flywheel_ramp_chunks(b.jobs[i], int(want["ramp"][k]), int(b.jobs[i]["dst_off"]), int(b.out_off[i]))
+        assert d is not None, shape(int(k))
+        blocks.append(d)
+    assert np.array_equal(np.concatenate(blocks), b.blocks)
 
 
 def test_golden_flywheel_vectors(port):

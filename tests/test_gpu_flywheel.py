@@ -7,23 +7,58 @@ import numpy as np
 import pytest
 
 from ohpipeline_b200 import abi, capi
-from flywheel_util import SHAPES, training_block, train_frames
+from flywheel_util import RATES, SHAPES, accepted_shapes, block_frames, shape_split, training_block, train_frames
 from util import make_desc
 
 pytestmark = pytest.mark.gpu
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "flywheel.npz")
+KINDS = ["tone", "noise", "dc", "zero", "step", "max"]
 
 
 def run_jobs(ctx, jobs, inp, out_bytes, fill=0x5A):
+    out, err = launch(ctx, jobs, inp, out_bytes, fill)
+    if err is not None:
+        raise err
+    return out
+
+
+def launch(ctx, jobs, inp, out_bytes, fill):
+    """One flywheel launch -> (output, the OhpError it raised or None); the output is read back either way."""
     import torch
     d_jobs = torch.from_numpy(jobs.view(np.uint8).copy()).cuda()
     d_in = torch.from_numpy(np.ascontiguousarray(inp)).cuda()
     d_out = torch.full((max(out_bytes, 1),), fill, dtype=torch.uint8, device="cuda")
     torch.cuda.synchronize()
-    ctx.flywheel_device(d_jobs.data_ptr(), len(jobs), d_in.data_ptr(), int(inp.size), d_out.data_ptr(), out_bytes)
-    ctx.sync()
-    return d_out.cpu().numpy()[:out_bytes]
+    err = None
+    try:
+        ctx.flywheel_device(d_jobs.data_ptr(), len(jobs), d_in.data_ptr(), int(inp.size), d_out.data_ptr(), out_bytes)
+        ctx.sync()
+    except capi.OhpError as e:
+        err = e
+    return d_out.cpu().numpy()[:out_bytes], err
+
+
+def out_len(job):
+    return int(job["out_frames"]) * int(job["channels"]) * (int(job["bit_depth"]) // 8)
+
+
+def covered(jobs, out_bytes):
+    """The output bytes some job writes."""
+    mask = np.zeros(out_bytes, dtype=bool)
+    for j in jobs:
+        mask[int(j["dst_off"]):int(j["dst_off"]) + out_len(j)] = True
+    return mask
+
+
+def assert_jobs_match(got, want, jobs, mask, what):
+    """Every byte a job writes is the oracle's; naming the job of the first one that is not."""
+    bad = np.nonzero((got != want) & mask)[0]
+    if bad.size:
+        i = int(bad[0])
+        k = next(k for k, j in enumerate(jobs) if int(j["dst_off"]) <= i < int(j["dst_off"]) + out_len(j))
+        raise AssertionError("%s: byte %d differs (got %#x want %#x) in job %d: %s, %d bytes differ in all"
+                             % (what, i, got[i], want[i], k, jobs[k], bad.size))
 
 
 def batch(kinds, shapes, seed, dst_align=1):
@@ -65,6 +100,120 @@ def test_flywheel_kernel_aligned_destinations_and_many_jobs(ctx, port):
     assert rc == 0
     got = run_jobs(ctx, jobs, inp, out_bytes, fill=0)
     assert np.array_equal(got, want)
+
+
+def every_shape_batch(seed):
+    """Every accepted shape x every training-block kind, in an order shuffled with `seed` (so the warps of one CTA hold
+    different shapes).  Destinations alternate between 16-byte aligned (the word stores, the tail loop after them, and
+    the switch to byte stores inside a job whose tiles are not whole words) and ragged (the byte stores), with a gap of
+    1-16 bytes before each; some training blocks start at offsets that are not a multiple of 4."""
+    rng = np.random.default_rng(seed)
+    work = [(kind, shape) for kind in KINDS for shape in accepted_shapes()]
+    jobs, blocks = [], []
+    src = dst = 0
+    for n, i in enumerate(rng.permutation(len(work))):
+        kind, (rate, ch, bits) = work[int(i)]
+        if n % 5 == 2:
+            pad = 1 + n % 3
+            blocks.append(np.full(pad, 0xC3, dtype=np.uint8))
+            src += pad
+        if n % 2 == 0:
+            dst = (dst + 16) // 16 * 16
+        else:
+            dst += 1 + n % 3
+            dst += dst % 4 == 0
+        j = capi.flywheel_job(rate, ch, bits, src_off=src, dst_off=dst)
+        t = training_block(rate, ch, kind, seed + int(i))
+        jobs.append(j)
+        blocks.append(t)
+        src += t.size
+        dst += out_len(j[0])
+    return np.concatenate(jobs), np.concatenate(blocks), dst + 16
+
+
+def test_flywheel_kernel_at_every_accepted_shape(ctx, port):
+    """550 shapes x 6 kinds of training block in one launch: the eight rates whose 1 ms block is shorter than a 32-frame
+    tile, and the 80 shapes (odd channel counts at 8 or 24 bits) whose tiles end inside a 4-byte word."""
+    fill = 0x5A
+    jobs, inp, out_bytes = every_shape_batch(seed=900)
+    assert len(jobs) == 550 * len(KINDS)
+    assert np.any(jobs["src_off"] % 4 != 0)
+    assert np.sum(jobs["dst_off"] % 16 == 0) >= len(jobs) // 2 and np.sum(jobs["dst_off"] % 4 != 0) == len(jobs) // 2
+    assert capi.flywheel_validate(jobs, inp.size, out_bytes)[0] == abi.OK
+    rc, want = port.flywheel(jobs, inp, out_bytes)
+    assert rc == 0
+    got, err = launch(ctx, jobs, inp, out_bytes, fill)
+    assert err is None, err
+    mask = covered(jobs, out_bytes)
+    assert_jobs_match(got, want, jobs, mask, "every shape")
+    assert np.all(got[~mask] == fill)
+
+
+def test_flywheel_kernel_output_lengths_at_tile_and_block_edges(ctx, port):
+    """Any out_frames (StarvationRamper always asks for 20 ms, the API takes any length): 1, 2, a tile -1 / 0 / +1, a
+    1 ms block -1 / 0 / +1, two blocks + 1 and 20 ms, at every rate, 1 and 3 channels x 8 and 24 bits, destinations
+    4-byte aligned."""
+    fill = 0x5A
+    jobs, blocks = [], []
+    src = dst = 0
+    for rate in RATES:
+        b = block_frames(rate)
+        lengths = sorted({1, 2, 31, 32, 33, b - 1, b, b + 1, 2 * b + 1, abi.FLYWHEEL_RAMP_JIFFIES // abi.jiffies_per_sample(rate)})
+        for ch in (1, 3):
+            for bits in (8, 24):
+                for frames in lengths:
+                    j = capi.flywheel_job(rate, ch, bits, src_off=src, dst_off=dst)
+                    j["out_frames"] = frames
+                    t = training_block(rate, ch, "tone", len(jobs))
+                    jobs.append(j)
+                    blocks.append(t)
+                    src += t.size
+                    dst = (dst + out_len(j[0]) + 4) // 4 * 4
+    jobs, inp, out_bytes = np.concatenate(jobs), np.concatenate(blocks), dst
+    assert capi.flywheel_validate(jobs, inp.size, out_bytes)[0] == abi.OK
+    rc, want = port.flywheel(jobs, inp, out_bytes)
+    assert rc == 0
+    got, err = launch(ctx, jobs, inp, out_bytes, fill)
+    assert err is None, err
+    mask = covered(jobs, out_bytes)
+    assert_jobs_match(got, want, jobs, mask, "output lengths")
+    assert np.all(got[~mask] == fill)
+
+
+@pytest.mark.parametrize("index", range(26))
+def test_refused_shape_among_valid_jobs(ctx, port, index):
+    """Each of the 26 shapes ohp_flywheel_validate refuses, as one job among seven valid ones: the launch fails with
+    E_INVALID_DESC naming that job, its destination keeps the fill, every other job writes the oracle's bytes, and the
+    context runs the valid jobs cleanly afterwards.  (With several refused jobs the message names whichever warp got
+    there first, so there is one per launch.)"""
+    fill = 0x5A
+    accepted, refused = shape_split()
+    pos = index % 8
+    shapes = [accepted[(37 * index + 79 * i) % len(accepted)] for i in range(7)]
+    shapes.insert(pos, refused[index])
+    jobs, blocks = [], []
+    src = dst = 0
+    for n, (rate, ch, bits) in enumerate(shapes):
+        j = capi.flywheel_job(rate, ch, bits, src_off=src, dst_off=dst)
+        t = training_block(rate, ch, KINDS[n % len(KINDS)], 40 * index + n)
+        jobs.append(j)
+        blocks.append(t)
+        src += t.size
+        dst = (dst + out_len(j[0]) + 16) // 16 * 16
+    jobs, inp, out_bytes = np.concatenate(jobs), np.concatenate(blocks), dst
+    assert capi.flywheel_validate(jobs, inp.size, out_bytes) == (abi.E_INVALID_DESC, pos)
+    valid = np.delete(jobs, pos)
+    rc, want = port.flywheel(valid, inp, out_bytes)
+    assert rc == 0
+    got, err = launch(ctx, jobs, inp, out_bytes, fill)
+    assert err is not None and err.status == abi.E_INVALID_DESC, err
+    assert "flywheel job %d (invalid)" % pos in str(err), str(err)
+    mask = covered(valid, out_bytes)
+    assert_jobs_match(got, want, valid, mask, "refused %s" % (refused[index],))
+    assert np.all(got[~mask] == fill)  # the refused job's destination and the gaps
+    again, err = launch(ctx, valid, inp, out_bytes, fill)
+    assert err is None, err
+    assert np.array_equal(again, got)
 
 
 def test_flywheel_kernel_reproduces_reference_golden_vectors(ctx):

@@ -1,7 +1,8 @@
 """ohp_run_streams_device_flywheel on the GPU: every stream's bytes as ohp_run_streams_device writes them, the walk's
 starvation records as the class model records them, and the flywheel audio of every starvation that plays as the host
-route plays it (ohp_schedule_build -> ohp_flywheel_plan_batch -> process / flywheel / process on the device) -- and, for
-flywheel_util.starved_streams(), as the reference's own StarvationRamper object plays it (tests/golden)."""
+route plays it (ohp_schedule_build -> ohp_flywheel_plan_batch -> process / flywheel / process on the device) and as the C
+oracle plays it (the same prep descriptors and job layout through oracle/ohp_oracle.c, with the oracle's own RampGenerator
+blocks) -- and, for flywheel_util.starved_streams(), as the reference's own StarvationRamper object plays it (tests/golden)."""
 import os
 import subprocess
 import sys
@@ -11,6 +12,7 @@ import pytest
 
 from ohpipeline_b200 import abi, capi
 from ohpipeline_b200 import workloads as W
+from flywheel_util import every_shape_streams, shape_split
 
 pytestmark = pytest.mark.gpu
 
@@ -93,6 +95,28 @@ def host_route(ctx, w, inp, sv):
     return {int(k): out[int(o):int(o) + int(n)] for k, o, n in zip(b.planned, b.out_off, b.out_len)}
 
 
+def oracle_route(port, w, inp, sv):
+    """What the C oracle plays for each planned record -> {record index: bytes}.  Only the prep descriptors and the job
+    layout come from ohp_flywheel_plan_batch; then ohpo_process_chunks (the training blocks), ohpo_flywheel, the oracle's
+    RampGenerator::EndBlock restatement (ohpo_flywheel_ramp_chunks, not the product's ohp_flywheel_ramp_chunks) and
+    ohpo_process_chunks again."""
+    b = capi.flywheel_plan_batch(w.streams, sv)
+    if len(b.planned) == 0:
+        return {}
+    rc, train = port.process_chunks(b.prep, inp, b.training_bytes)
+    assert rc == 0
+    rc, gen = port.flywheel(b.jobs, train, b.generated_bytes)
+    assert rc == 0
+    blocks = []
+    for i, k in enumerate(b.planned):
+        d, _ = port.flywheel_ramp_chunks(b.jobs[i], int(sv["ramp"][k]), int(b.jobs[i]["dst_off"]), int(b.out_off[i]))
+        assert d is not None, (w.name, int(k))
+        blocks.append(d)
+    rc, out = port.process_chunks(np.concatenate(blocks), gen, b.out_bytes)
+    assert rc == 0
+    return {int(k): out[int(o):int(o) + int(n)] for k, o, n in zip(b.planned, b.out_off, b.out_len)}
+
+
 def check(ctx, w, port, seed=None):
     """The whole comparison for one batch; returns (records, flywheel result)."""
     inp = port.fill_pcm(w.in_bytes, w.seed if seed is None else seed)
@@ -113,13 +137,16 @@ def check(ctx, w, port, seed=None):
     off, size, total = slots(w)
     assert np.array_equal(r["off"], off), w.name
     want = host_route(ctx, w, inp, sv)
-    played = {int(sv["event"][k]): v for k, v in want.items()}
+    oracle = oracle_route(port, w, inp, sv)
+    assert sorted(oracle) == sorted(want), w.name
+    played = {int(sv["event"][k]): (v, oracle[k]) for k, v in want.items()}
     assert sorted(np.nonzero(r["len"])[0].tolist()) == sorted(played), w.name
     covered = np.zeros(total, dtype=bool)
-    for e, v in played.items():
+    for e, (v, o_bytes) in played.items():
         o, n = int(off[e]), int(r["len"][e])
-        assert n == len(v) and n <= int(size[e])
-        assert np.array_equal(r["fly"][o:o + n], v), (w.name, e)
+        assert n == len(v) == len(o_bytes) and n <= int(size[e])
+        assert np.array_equal(r["fly"][o:o + n], o_bytes), (w.name, e, "differs from the oracle route")
+        assert np.array_equal(r["fly"][o:o + n], v), (w.name, e, "differs from the host route")
         covered[o:o + n] = True
     assert np.all(r["fly"][~covered] == FLY_FILL), w.name
     return sv, r
@@ -148,13 +175,40 @@ def test_random_batches_against_the_host_route(ctx, port):
     assert plays > 50
 
 
+def test_every_shape_streams(ctx, port):
+    """flywheel_util.every_shape_streams(): 576 shapes starved twice.  The 1100 records at the 550 accepted shapes play
+    what the oracle route and the host route play; the 52 at the 26 refused shapes play nothing and keep their slots'
+    fill; the streams' bytes are the oracle's end-to-end output."""
+    w = every_shape_streams()
+    sv, r = check(ctx, w, port)
+    accepted, refused = shape_split()
+    shape = lambda s: (int(s["sample_rate"]), int(s["channels"]), int(s["bit_depth"]))  # noqa: E731
+    ev = sv["event"].astype(np.int64)
+    shapes = [shape(w.streams[int(s)]) for s in sv["stream"]]
+    played = {sh for sh, e in zip(shapes, ev) if r["len"][e]}
+    assert played == set(accepted)
+    silent = [e for sh, e in zip(shapes, ev) if sh in set(refused)]
+    assert len(silent) == 52 and int((r["len"][ev] != 0).sum()) == 1100
+    off, size, _ = slots(w)
+    for e in silent:
+        assert r["len"][e] == 0 and np.all(r["fly"][int(off[e]):int(off[e]) + int(size[e])] == FLY_FILL), e
+    inp = port.fill_pcm(w.in_bytes, w.seed)
+    rc, want, chunks, _ = port.run(w.streams, w.events, inp, w.out_bytes)
+    assert rc == 0
+    mask = np.zeros(w.out_bytes, dtype=bool)
+    for d, n in zip(chunks, abi.chunk_out_bytes(chunks)):
+        mask[int(d["dst_off"]):int(d["dst_off"]) + int(n)] = True
+    assert np.array_equal(r["out"][mask], want[mask])
+    assert np.all(r["out"][~mask] == FILL)
+
+
 def child():
     """Runs in a child process with the environment of the parametrization below."""
     from oracle import pyoracle
     port = pyoracle.Port()
     ctx = capi.Context(0)
     try:
-        for w in batches()[:1] + batches()[-1:]:
+        for w in batches()[:1] + batches()[-1:] + [every_shape_streams()]:
             check(ctx, w, port)
     finally:
         ctx.close()

@@ -10,12 +10,10 @@ import pytest
 
 from ohpipeline_b200 import abi, capi
 from ohpipeline_b200 import workloads as W
-from flywheel_util import starved_streams
+from flywheel_util import RATES, every_shape_streams, starved_streams
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MS = abi.JIFFIES_PER_MS
-RATES = [7350, 8000, 11025, 12000, 14700, 16000, 22050, 24000, 29400, 32000, 44100, 48000, 88200, 96000, 176400, 192000,
-         352800, 384000]
 
 
 def records(w):
@@ -117,7 +115,7 @@ def shape_records():
 
 def test_device_planner_equals_the_class_based_plan(tmp_path):
     specs, recs = shape_records()
-    for name, w, _ in starved_streams() + [(w.name, w, 0) for w in edge_cases()] + \
+    for name, w, _ in starved_streams() + [(w.name, w, 0) for w in edge_cases() + [every_shape_streams()]] + \
             [("elements", W.elements(s, n_streams=24, attenuation=bool(s % 2)), 0) for s in range(8)]:
         sv = capi.schedule_build(w.streams, w.events).starvations
         for r in sv:
