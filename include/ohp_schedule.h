@@ -217,6 +217,8 @@ typedef struct ohp_recent_audio {
 } ohp_recent_audio;
 const ohp_recent_audio* ohp_schedule_recent_audio(const ohp_schedule* s);
 const uint64_t* ohp_schedule_recent_begin(const ohp_schedule* s); /* ohp_schedule_num_starvations(s) + 1 entries */
+/* prep descriptors ohp_flywheel_plan_batch_recent (and the device's planner) allow one starvation: more are not planned */
+#define OHP_FLYWHEEL_MAX_PREP_RECENT 64u
 int    ohp_flywheel_plan_recent(const ohp_stream_spec* stream, const ohp_starvation* starvation,
                                 const ohp_recent_audio* recent, size_t n_recent,
                                 uint64_t training_off, uint64_t generated_off, uint64_t out_off,

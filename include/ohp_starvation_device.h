@@ -21,7 +21,8 @@
  * plays nothing (halted, muted, not yet audible), the last millisecond was not PCM of one attenuation, or the shape does
  * not fit the reference's flywheel buffers (ohp_flywheel_plan's refusals).  Only the bytes of played slots are written.
  *   d_starvations ([n_events], may be NULL): the record of event e at [e]; where e left none, every byte of [e] is 0xff
- *     (event = 0xffffffff).  Records carry no recent audio (ohp_flywheel_plan_recent is host-only).
+ *     (event = 0xffffffff).  Records carry no recent audio: ohp_run_streams_device_flywheel_recent (ohp_starvation_recent.h)
+ *     also keeps it and plays the starvations with silence or a change of attenuation in their last millisecond.
  *   d_fly_off, d_fly_len ([n_events] each): required when n_events > 0.
  * Errors: as ohp_run_streams_device; OHP_E_OUT_OF_RANGE when fly_out_bytes is below the slots' total (ohp_last_error names
  * the bytes needed; nothing is written to d_fly_out); OHP_E_INVALID_ARG when two streams' event slices share an event.

@@ -78,6 +78,10 @@ FLYWHEEL_MAX_PREP = 9
 # include/ohp_schedule.h: ohp_recent_audio
 RECENT_AUDIO = np.dtype([("pcm_jiffies", "<u8"), ("jiffies", "<u4"), ("silence", "<u4"), ("attenuation", "<u4"), ("reserved", "<u4")])
 assert RECENT_AUDIO.itemsize == 24
+FLYWHEEL_MAX_PREP_RECENT = 64
+# include/ohp_starvation_recent.h
+DEVICE_RECENT_PIECES = 16              # pieces of recent audio the device walk keeps per StarvationRamper stage
+RECENT_INCOMPLETE = 0xFFFFFFFF         # a record that needs more pieces than that: not played
 
 # include/ohp_flywheel.h
 FLYWHEEL_JOB = np.dtype([

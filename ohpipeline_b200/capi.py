@@ -101,6 +101,12 @@ def cuda_lib():
             L.ohp_run_streams_device_flywheel.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p,
                                                           C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p,
                                                           C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.c_void_p]
+        if hasattr(L, "ohp_run_streams_device_flywheel_recent"):  # include/ohp_starvation_recent.h
+            L.ohp_run_streams_device_flywheel_recent.restype = C.c_int
+            L.ohp_run_streams_device_flywheel_recent.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p,
+                                                                 C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p,
+                                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                                 C.POINTER(C.c_uint64), C.c_void_p]
         if hasattr(L, "ohp_run_streams_device"):
             L.ohp_run_streams_device.restype = C.c_int
             L.ohp_run_streams_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p, C.c_uint64,
@@ -631,6 +637,20 @@ class Context:
                                                             C.c_void_p(d_fly_off), C.c_void_p(d_fly_len),
                                                             C.c_void_p(d_stream_out_bytes), C.byref(total) if want_total else None,
                                                             C.c_void_p(stream or 0)))
+        return int(total.value) if want_total else None
+
+    def run_streams_device_flywheel_recent(self, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
+                                           d_fly_out, fly_out_bytes, d_fly_off, d_fly_len, d_starvations=0, d_stream_out_bytes=0,
+                                           stream=None, want_total=True, d_recent=0, d_recent_count=0):
+        """ohp_run_streams_device_flywheel_recent: run_streams_device_flywheel with every starvation planned from the element's
+        recent audio, silence included; where given, event e's pieces (abi.RECENT_AUDIO) at d_recent + e *
+        abi.DEVICE_RECENT_PIECES and their number (uint32, abi.RECENT_INCOMPLETE: more than the walk keeps) at d_recent_count[e]."""
+        total = C.c_uint64(0)
+        self._check(self._L.ohp_run_streams_device_flywheel_recent(
+            self._h, C.c_void_p(d_streams), n_streams, C.c_void_p(d_events), n_events, C.c_void_p(d_in), in_bytes, C.c_void_p(d_out),
+            out_bytes, C.c_void_p(d_fly_out), fly_out_bytes, C.c_void_p(d_starvations), C.c_void_p(d_fly_off), C.c_void_p(d_fly_len),
+            C.c_void_p(d_stream_out_bytes), C.c_void_p(d_recent), C.c_void_p(d_recent_count),
+            C.byref(total) if want_total else None, C.c_void_p(stream or 0)))
         return int(total.value) if want_total else None
 
     def fill_streams_device(self, d_in, in_bytes, d_streams, n_streams, seed_base, first_stream_id=0, stream=None):

@@ -10,6 +10,7 @@
 #include "ohp_flywheel_kernels.cuh"
 #include "../../include/ohp_schedule_device.h"
 #include "../../include/ohp_starvation_device.h"
+#include "../../include/ohp_starvation_recent.h"
 
 #include <cstdio>
 #include <cstdlib>
@@ -95,6 +96,9 @@ struct ohp_context
     ohp_flywheel_job* d_fly_jobs = nullptr; uint64_t d_fly_jobs_cap = 0;
     uint8_t* d_fly_train = nullptr; uint64_t d_fly_train_cap = 0;    // training blocks
     uint8_t* d_fly_gen = nullptr; uint64_t d_fly_gen_cap = 0;        // generated audio
+    // ohp_run_streams_device_flywheel_recent, when the caller passes no arrays of its own (grown on demand)
+    ohp_recent_audio* d_recent = nullptr; uint64_t d_recent_cap = 0;
+    uint32_t* d_recent_count = nullptr; uint64_t d_recent_count_cap = 0;
     std::vector<uint64_t> h_begin, h_outb;
     cudaEvent_t ev_start = nullptr, ev_stop = nullptr;
     bool timing = false;
@@ -642,6 +646,8 @@ int ohp_create(int device, ohp_context** out_ctx)
         OHP_CREATE(cudaFuncSetAttribute(sched::schedule_kernel<true, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(sched::schedule_record_kernel<32>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(sched::schedule_record_kernel<1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        OHP_CREATE(cudaFuncSetAttribute(sched::schedule_recent_kernel<32>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        OHP_CREATE(cudaFuncSetAttribute(sched::schedule_recent_kernel<1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(sched::scan_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(ramp_convert_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         OHP_CREATE(cudaFuncSetAttribute(ramp_convert_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -673,7 +679,7 @@ int ohp_destroy(ohp_context* ctx)
     if (ctx->d_counts) (void)cudaFree(ctx->d_counts);
     if (ctx->h_regions) (void)cudaFreeHost(ctx->h_regions);
     for (void* p : {(void*)ctx->d_records, (void*)ctx->d_slot, (void*)ctx->d_owner, (void*)ctx->d_fly_slots, (void*)ctx->d_fly_descs,
-                    (void*)ctx->d_fly_jobs, (void*)ctx->d_fly_train, (void*)ctx->d_fly_gen}) {
+                    (void*)ctx->d_fly_jobs, (void*)ctx->d_fly_train, (void*)ctx->d_fly_gen, (void*)ctx->d_recent, (void*)ctx->d_recent_count}) {
         if (p) (void)cudaFree(p);
     }
     if (ctx->sched_event) (void)cudaEventDestroy(ctx->sched_event);
@@ -1113,11 +1119,13 @@ int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, siz
 // the only host round trip is for the regions' total (bound + scan are a few microseconds of GPU time).
 // A stream that outgrows its region (none of the shapes this repo generates does, the bound is held against the exact
 // counts in tests/test_schedule_walk.py) sends the whole call through the two-pass path.
-// records (ohp_run_streams_device_flywheel): the emitting walk also leaves the starvation records there.
+// records (ohp_run_streams_device_flywheel): the emitting walk also leaves the starvation records there; with recent
+// (ohp_run_streams_device_flywheel_recent) their pieces of recent audio too.
 static int run_streams_device_two_pass(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
                                        const ohp_ramp_event* d_events, size_t n_events,
                                        const uint8_t* d_in, uint64_t in_bytes, uint8_t* d_out, uint64_t out_bytes,
-                                       uint64_t* d_stream_out_bytes, uint64_t* total_chunks, ohp_starvation* records, cudaStream_t st)
+                                       uint64_t* d_stream_out_bytes, uint64_t* total_chunks, ohp_starvation* records, cudaStream_t st,
+                                       const sched::RecentOut* recent = nullptr)
 {
     int rc;
     uint64_t total = 0;
@@ -1138,10 +1146,13 @@ static int run_streams_device_two_pass(ohp_context* ctx, const ohp_stream_spec* 
         p.status = ctx->d_status + 2;
         p.records = records;
         if (schedule_team(n_streams) == 32) {
-            sched::schedule_record_kernel<32><<<sched::schedule_grid(n_streams, 32), sched::kScheduleBlock, 0, st>>>(p);
+            if (recent) sched::schedule_recent_kernel<32><<<sched::schedule_grid(n_streams, 32), sched::kScheduleBlock, 0, st>>>(p, *recent);
+            else sched::schedule_record_kernel<32><<<sched::schedule_grid(n_streams, 32), sched::kScheduleBlock, 0, st>>>(p);
         } else {
             p.lanes_per_warp = schedule_lanes(ctx, n_streams);
-            sched::schedule_record_kernel<1><<<sched::schedule_grid(n_streams, 1, p.lanes_per_warp), sched::kScheduleBlock, 0, st>>>(p);
+            const unsigned grid = sched::schedule_grid(n_streams, 1, p.lanes_per_warp);
+            if (recent) sched::schedule_recent_kernel<1><<<grid, sched::kScheduleBlock, 0, st>>>(p, *recent);
+            else sched::schedule_record_kernel<1><<<grid, sched::kScheduleBlock, 0, st>>>(p);
         }
         OHP_CUDA(ctx, cudaGetLastError());
         ctx->launches++;
@@ -1157,6 +1168,10 @@ struct FlyArgs
     ohp_starvation* records; // the caller's, or the context's
     uint64_t* off;
     uint64_t* len;
+    // ohp_run_streams_device_flywheel_recent: planned from the recent audio (the caller's arrays, or the context's)
+    bool with_recent;
+    sched::RecentOut recent;
+    uint64_t prep_per() const { return with_recent ? OHP_FLYWHEEL_MAX_PREP_RECENT : OHP_FLYWHEEL_MAX_PREP; }
 };
 
 // The slots' total is known (h_regions[4..8)): refuse what the call cannot lay out.
@@ -1184,7 +1199,7 @@ static int fly_plan(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n
 {
     const sched::FlySlots fs = *reinterpret_cast<const sched::FlySlots*>(ctx->h_regions + 4);
     if (fs.count == 0) return OHP_OK; // not one starvation event: the call is ohp_run_streams_device's, launch for launch
-    const uint64_t per = OHP_FLYWHEEL_MAX_PREP + flyplan::kMaxBlocks;
+    const uint64_t per = fly.prep_per() + flyplan::kMaxBlocks;
     int rc;
     if ((rc = grow_idle(ctx, ctx->d_fly_descs, ctx->d_fly_descs_cap, fs.count * per * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
     if ((rc = grow_idle(ctx, ctx->d_fly_jobs, ctx->d_fly_jobs_cap, fs.count * sizeof(ohp_flywheel_job))) != OHP_OK) return rc;
@@ -1193,9 +1208,10 @@ static int fly_plan(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n
     OHP_CUDA(ctx, cudaGetLastError());
     sched::PlanParams pp;
     pp.streams = d_streams; pp.n_streams = n_streams; pp.n_events = n_events; pp.records = fly.records; pp.slot = ctx->d_slot;
-    pp.prep = ctx->d_fly_descs; pp.jobs = ctx->d_fly_jobs; pp.blocks = ctx->d_fly_descs + fs.count * OHP_FLYWHEEL_MAX_PREP;
+    pp.prep = ctx->d_fly_descs; pp.jobs = ctx->d_fly_jobs; pp.blocks = ctx->d_fly_descs + fs.count * fly.prep_per();
     pp.fly_off = fly.off; pp.fly_len = fly.len; pp.slots = ctx->d_fly_slots;
-    sched::plan_kernel<<<(unsigned)((n_events + 127) / 128), 128, 0, st>>>(pp);
+    if (fly.with_recent) sched::plan_recent_kernel<<<(unsigned)((n_events + 127) / 128), 128, 0, st>>>(pp, fly.recent.recent, fly.recent.count);
+    else sched::plan_kernel<<<(unsigned)((n_events + 127) / 128), 128, 0, st>>>(pp);
     OHP_CUDA(ctx, cudaGetLastError());
     ctx->launches += 2;
     OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_regions + 4, ctx->d_fly_slots, sizeof(sched::FlySlots), cudaMemcpyDeviceToHost, st));
@@ -1214,8 +1230,8 @@ static int fly_play(ohp_context* ctx, const uint8_t* d_in, uint64_t in_bytes, co
     if ((rc = grow_idle(ctx, ctx->d_fly_train, ctx->d_fly_train_cap, bytes)) != OHP_OK) return rc;
     if ((rc = grow_idle(ctx, ctx->d_fly_gen, ctx->d_fly_gen_cap, bytes)) != OHP_OK) return rc;
     const ohp_chunk_desc* prep = ctx->d_fly_descs;
-    const ohp_chunk_desc* blocks = ctx->d_fly_descs + count * OHP_FLYWHEEL_MAX_PREP;
-    if ((rc = launch(ctx, prep, (size_t)(count * OHP_FLYWHEEL_MAX_PREP), d_in, in_bytes, ctx->d_fly_train, bytes, st)) != OHP_OK) return rc;
+    const ohp_chunk_desc* blocks = ctx->d_fly_descs + count * fly.prep_per();
+    if ((rc = launch(ctx, prep, (size_t)(count * fly.prep_per()), d_in, in_bytes, ctx->d_fly_train, bytes, st)) != OHP_OK) return rc;
     if ((rc = ohp_flywheel_device(ctx, ctx->d_fly_jobs, (size_t)planned, ctx->d_fly_train, bytes, ctx->d_fly_gen, bytes, st)) != OHP_OK) return rc;
     return launch(ctx, blocks, (size_t)(count * flyplan::kMaxBlocks), ctx->d_fly_gen, bytes, fly.out, fly.out_bytes, st);
 }
@@ -1238,6 +1254,7 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
     if (!ctx->h_regions) OHP_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void**>(&ctx->h_regions), 8 * sizeof(uint64_t), cudaHostAllocDefault));
     if (!ctx->sched_event) OHP_CUDA(ctx, cudaEventCreateWithFlags(&ctx->sched_event, cudaEventDisableTiming));
     ohp_starvation* records = nullptr;
+    FlyArgs flyArgs{}; // *fly with the context's scratch in place of the arrays the caller left NULL
     if (fly) {
         // records (none yet: all ones), slots (none: zero), owners (none: all ones), the slots' totals, where the flywheel
         // audio goes (nowhere yet)
@@ -1255,7 +1272,20 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
             OHP_CUDA(ctx, cudaMemsetAsync(fly->off, 0, n_events * sizeof(uint64_t), st));
             OHP_CUDA(ctx, cudaMemsetAsync(fly->len, 0, n_events * sizeof(uint64_t), st));
         }
+        flyArgs = *fly;
+        flyArgs.records = records;
+        if (fly->with_recent) {
+            // piece counts: 0 until a record is written
+            const uint64_t n = n_events ? n_events : 1;
+            if (!flyArgs.recent.recent && (rc = grow_idle(ctx, ctx->d_recent, ctx->d_recent_cap, n * sched::kRecentPieces * sizeof(ohp_recent_audio))) != OHP_OK) return rc;
+            if (!flyArgs.recent.count && (rc = grow_idle(ctx, ctx->d_recent_count, ctx->d_recent_count_cap, n * sizeof(uint32_t))) != OHP_OK) return rc;
+            if (!flyArgs.recent.recent) flyArgs.recent.recent = ctx->d_recent;
+            if (!flyArgs.recent.count) flyArgs.recent.count = ctx->d_recent_count;
+            if (n_events) OHP_CUDA(ctx, cudaMemsetAsync(flyArgs.recent.count, 0, n_events * sizeof(uint32_t), st));
+        }
+        fly = &flyArgs;
     }
+    const sched::RecentOut* recent = fly && fly->with_recent ? &fly->recent : nullptr;
     auto bound = [&]() -> int { // regions: bound per stream (and, with fly, the flywheel slots)
         if (fly) {
             sched::bound_slots_kernel<<<(unsigned)((n_streams + 127) / 128), 128, 0, st>>>(d_streams, n_streams, d_events, n_events, ctx->d_begin,
@@ -1288,7 +1318,7 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
             if ((rc = fly_check(ctx, *fly)) != OHP_OK) return rc;
         }
         return finish(run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
-                                                  d_stream_out_bytes, total_chunks, records, st));
+                                                  d_stream_out_bytes, total_chunks, records, st, recent));
     }
     // 1. regions: bound per stream, exclusive scan
     if ((rc = bound()) != OHP_OK) return rc;
@@ -1313,7 +1343,11 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
         p.lanes_per_warp = schedule_lanes(ctx, n_streams);
         p.records = records;
         const unsigned grid = team == 32 ? sched::schedule_grid(n_streams, 32) : sched::schedule_grid(n_streams, 1, p.lanes_per_warp);
-        if (records) {
+        if (recent) {
+            if (team == 32) sched::schedule_recent_kernel<32><<<grid, sched::kScheduleBlock, 0, st>>>(p, *recent);
+            else sched::schedule_recent_kernel<1><<<grid, sched::kScheduleBlock, 0, st>>>(p, *recent);
+        }
+        else if (records) {
             if (team == 32) sched::schedule_record_kernel<32><<<grid, sched::kScheduleBlock, 0, st>>>(p);
             else sched::schedule_record_kernel<1><<<grid, sched::kScheduleBlock, 0, st>>>(p);
         }
@@ -1356,7 +1390,7 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
         if ((bits & (1u << sched::kErrBound)) && !(bits & refused)) {
             (void)read_status(ctx, st);
             return finish(run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
-                                                      d_stream_out_bytes, total_chunks, records, st));
+                                                      d_stream_out_bytes, total_chunks, records, st, recent));
         }
         if (src != OHP_OK) return src;
     }
@@ -1388,6 +1422,23 @@ int ohp_run_streams_device_flywheel(ohp_context* ctx, const ohp_stream_spec* d_s
         return fail(ctx, OHP_E_INVALID_ARG, "null device pointer (d_fly_off / d_fly_len)");
     }
     const FlyArgs fly{d_fly_out, d_fly_out ? fly_out_bytes : 0, d_starvations, d_fly_off, d_fly_len};
+    return run_streams_device(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
+                              d_stream_out_bytes, total_chunks, stream, &fly);
+}
+
+int ohp_run_streams_device_flywheel_recent(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
+                                           const ohp_ramp_event* d_events, size_t n_events,
+                                           const uint8_t* d_in, uint64_t in_bytes, uint8_t* d_out, uint64_t out_bytes,
+                                           uint8_t* d_fly_out, uint64_t fly_out_bytes, ohp_starvation* d_starvations,
+                                           uint64_t* d_fly_off, uint64_t* d_fly_len, uint64_t* d_stream_out_bytes,
+                                           ohp_recent_audio* d_recent, uint32_t* d_recent_count, uint64_t* total_chunks, void* stream)
+{
+    if (!ctx) return OHP_E_INVALID_ARG;
+    if (n_events && (!d_fly_off || !d_fly_len)) {
+        if (total_chunks) *total_chunks = 0;
+        return fail(ctx, OHP_E_INVALID_ARG, "null device pointer (d_fly_off / d_fly_len)");
+    }
+    const FlyArgs fly{d_fly_out, d_fly_out ? fly_out_bytes : 0, d_starvations, d_fly_off, d_fly_len, true, {d_recent, d_recent_count}};
     return run_streams_device(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
                               d_stream_out_bytes, total_chunks, stream, &fly);
 }

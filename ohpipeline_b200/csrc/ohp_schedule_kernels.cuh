@@ -54,8 +54,9 @@ __global__ void __launch_bounds__(128) bound_kernel(const ohp_stream_spec* __res
 #ifndef OHP_SCHED_MIN_BLOCKS
 #define OHP_SCHED_MIN_BLOCKS 3 /* <= 168 registers.  The walk times of DESIGN 4.2 were measured with this bound; 5 (96 registers) spills. */
 #endif
-template <bool EMIT, int TEAM, bool RECORD>
-__device__ __forceinline__ void schedule_body(const ScheduleParams p)
+// RECENT: the records' pieces of recent audio too, at recent[e * kRecentPieces ...] and recent_count[e] for event e.
+template <bool EMIT, int TEAM, bool RECORD, bool RECENT = false>
+__device__ __forceinline__ void schedule_body(const ScheduleParams p, ohp_recent_audio* recent = nullptr, uint32_t* recent_count = nullptr)
 {
     const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     uint64_t s = t / TEAM;
@@ -76,8 +77,10 @@ __device__ __forceinline__ void schedule_body(const ScheduleParams p)
     //  second launch that follows when that turns out to be the case)
     if (regions && p.descs_cap != 0 && p.chunk_begin[s + 1] > p.descs_cap) return;
     const uint64_t limit = regions ? p.chunk_begin[s + 1] - p.chunk_begin[s] : ~0ull;
-    uint32_t rc = run_stream<EMIT, TEAM, true, RECORD>(sp, p.events, p.n_events, descs, info, nChunks, outBytes, lane, limit,
-                                                       RECORD ? p.records + sp.first_event : nullptr, s);
+    uint32_t rc = run_stream<EMIT, TEAM, true, RECORD, RECENT>(sp, p.events, p.n_events, descs, info, nChunks, outBytes, lane, limit,
+                                                               RECORD ? p.records + sp.first_event : nullptr, s, false, nullptr,
+                                                               RECENT ? recent + (uint64_t)sp.first_event * kRecentPieces : nullptr,
+                                                               RECENT ? recent_count + sp.first_event : nullptr);
     if (regions) {
         if (rc == kOk && nChunks > limit) rc = kErrBound;
         // the rest of the region: zero-byte descriptors (all lanes of the team, two 128-bit stores each)
@@ -111,6 +114,18 @@ template <int TEAM>
 __global__ void __launch_bounds__(128, OHP_SCHED_MIN_BLOCKS) schedule_record_kernel(const ScheduleParams p)
 {
     schedule_body<true, TEAM, true>(p);
+}
+
+// ... that also leaves each record's pieces of recent audio (ohp_run_streams_device_flywheel_recent).
+struct RecentOut
+{
+    ohp_recent_audio* recent;  // [n_events * kRecentPieces]
+    uint32_t* count;           // [n_events]
+};
+template <int TEAM>
+__global__ void __launch_bounds__(128, OHP_SCHED_MIN_BLOCKS) schedule_recent_kernel(const ScheduleParams p, const RecentOut r)
+{
+    schedule_body<true, TEAM, true, true>(p, r.recent, r.count);
 }
 
 // FLYWHEEL SLOTS.  Event e's flywheel audio goes to a slot of align16(ToSamples(20 ms) x frame bytes) of its stream; the
@@ -186,8 +201,12 @@ struct PlanParams
     FlySlots* slots;
 };
 
-__global__ void __launch_bounds__(128) plan_kernel(const PlanParams p)
+// RECENT: planned from the record's pieces of recent audio (flyplan::plan_recent), OHP_FLYWHEEL_MAX_PREP_RECENT prep
+// descriptors per starvation event; a record whose pieces the walk could not keep all of (OHP_RECENT_INCOMPLETE) is not.
+template <bool RECENT>
+__device__ __forceinline__ void plan_body(const PlanParams p, const ohp_recent_audio* recent = nullptr, const uint32_t* recent_count = nullptr)
 {
+    constexpr uint32_t kPrep = RECENT ? OHP_FLYWHEEL_MAX_PREP_RECENT : OHP_FLYWHEEL_MAX_PREP;
     const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= p.n_events) return;
     const uint64_t here = p.slot[e], next = p.slot[e + 1];
@@ -196,14 +215,23 @@ __global__ void __launch_bounds__(128) plan_kernel(const PlanParams p)
     p.fly_len[e] = 0;
     if ((next >> kSlotCountShift) == (here >> kSlotCountShift)) return; // not a starvation event of a stream
     const uint64_t k = here >> kSlotCountShift;
-    ohp_chunk_desc* prep = p.prep + k * OHP_FLYWHEEL_MAX_PREP;
+    ohp_chunk_desc* prep = p.prep + k * kPrep;
     ohp_chunk_desc* blocks = p.blocks + k * flyplan::kMaxBlocks;
     ohp_flywheel_job job;
     uint32_t nPrep = 0, nBlocks = 0;
     const ohp_starvation rec = p.records[e];
     if (rec.event == e && rec.stream < p.n_streams) {
         const ohp_stream_spec sp = p.streams[rec.stream];
-        if (flyplan::plan(sp, rec, off, off, off, prep, nPrep, job, blocks, nBlocks) == OHP_OK) {
+        int status;
+        if constexpr (RECENT) {
+            const uint32_t n = recent_count[e];
+            status = n <= kRecentPieces ? flyplan::plan_recent(sp, rec, recent + e * kRecentPieces, n, off, off, off, prep, nPrep, job, blocks, nBlocks)
+                                        : OHP_E_INVALID_ARG;
+        }
+        else {
+            status = flyplan::plan(sp, rec, off, off, off, prep, nPrep, job, blocks, nBlocks);
+        }
+        if (status == OHP_OK) {
             p.fly_len[e] = (uint64_t)job.out_frames * sp.channels * (sp.bit_depth / 8u);
             p.jobs[atomicAdd(reinterpret_cast<unsigned long long*>(&p.slots->planned), 1ull)] = job;
         }
@@ -211,8 +239,19 @@ __global__ void __launch_bounds__(128) plan_kernel(const PlanParams p)
             nPrep = nBlocks = 0;
         }
     }
-    for (uint32_t i = nPrep; i < OHP_FLYWHEEL_MAX_PREP; i++) prep[i] = flyplan::zero_desc();
+    for (uint32_t i = nPrep; i < kPrep; i++) prep[i] = flyplan::zero_desc();
     for (uint32_t i = nBlocks; i < flyplan::kMaxBlocks; i++) blocks[i] = flyplan::zero_desc();
+}
+
+__global__ void __launch_bounds__(128) plan_kernel(const PlanParams p)
+{
+    plan_body<false>(p);
+}
+
+__global__ void __launch_bounds__(128) plan_recent_kernel(const PlanParams p, const ohp_recent_audio* __restrict__ recent,
+                                                          const uint32_t* __restrict__ recent_count)
+{
+    plan_body<true>(p, recent, recent_count);
 }
 
 // threads per block; grid for n streams

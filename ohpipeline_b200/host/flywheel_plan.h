@@ -148,5 +148,135 @@ OHP_HD int plan(const ohp_stream_spec& sp, const ohp_starvation& sv, uint64_t aT
     return rc;
 }
 
+// ohp_flywheel_plan_recent on the record's pieces of recent audio (pieces[0..aNumPieces), oldest first), with room for
+// OHP_FLYWHEEL_MAX_PREP_RECENT prep descriptors: the same status, and on OHP_OK the same descriptors.  The pieces are walked
+// three times (the cut, the frames FlywheelInput reads, the descriptors) instead of being collected.
+OHP_HD int plan_recent(const ohp_stream_spec& sp, const ohp_starvation& sv, const ohp_recent_audio* pieces, uint32_t aNumPieces,
+                       uint64_t aTrainingOff, uint64_t aGeneratedOff, uint64_t aOutOff,
+                       ohp_chunk_desc* prep, uint32_t& aNumPrep, ohp_flywheel_job& job, ohp_chunk_desc* blocks, uint32_t& aNumBlocks)
+{
+    aNumPrep = 0;
+    aNumBlocks = 0;
+    const uint32_t jps = core::jiffies_per_sample_or_zero(sp.sample_rate);
+    const uint32_t B = sp.bit_depth / 8u;
+    const uint32_t C = sp.channels;
+    const uint32_t frameBytes = C * B;
+    if (jps == 0 || frameBytes == 0 || !(sp.bit_depth == 8 || sp.bit_depth == 16 || sp.bit_depth == 24 || sp.bit_depth == 32)) return OHP_E_INVALID_ARG;
+    if (C > OHP_FLYWHEEL_MAX_CHANNELS) return OHP_E_INVALID_DESC;
+    if (!sv.plays) return OHP_E_INVALID_ARG;
+    const uint32_t train = OHP_FLYWHEEL_TRAINING_JIFFIES / jps;
+    {
+        const uint32_t decimation = (sp.sample_rate == 192000u || sp.sample_rate == 176400u) ? 4u
+                                  : (sp.sample_rate == 88200u || sp.sample_rate == 96000u) ? 2u : 1u;
+        const uint32_t blockFrames = OHP_FLYWHEEL_BLOCK_JIFFIES / jps;
+        if (train < 2 || train / decimation < OHP_FLYWHEEL_DEGREE + 1u || train * 4u * C > OHP_FLYWHEEL_MAX_INPUT_BYTES
+            || blockFrames * frameBytes > OHP_FLYWHEEL_MAX_BLOCK_BYTES) {
+            return OHP_E_INVALID_DESC;
+        }
+    }
+    // StartFlywheelRamp's cut: whole pieces go from the front while more than kTrainingJiffies is left, the piece under the
+    // cut is split (head: that piece after the cut)
+    uint64_t total = 0;
+    for (uint32_t i = 0; i < aNumPieces; i++) total += pieces[i].jiffies;
+    if (total < OHP_FLYWHEEL_TRAINING_JIFFIES) return OHP_E_INVALID_ARG;
+    uint64_t excess = total - OHP_FLYWHEEL_TRAINING_JIFFIES;
+    uint32_t first = 0;
+    ohp_recent_audio head = {0, 0, 0, 0, 0};
+    while (first < aNumPieces) {
+        head = pieces[first];
+        if (excess == 0) break;
+        if (head.jiffies > excess) {
+            if (head.silence && excess % jps != 0) return OHP_E_INVALID_DESC; // the cut that never ends
+            head.jiffies -= (uint32_t)excess;
+            if (!head.silence) head.pcm_jiffies += excess;
+            excess = 0;
+            break;
+        }
+        excess -= head.jiffies;
+        first++;
+    }
+    // piece i (from `first`) through CreatePlayable: silence, first frame, frames, attenuation
+    auto run = [&](uint32_t i, bool& aSilence, uint64_t& aFirstFrame, uint32_t& aFrames, uint32_t& aAtt) {
+        const ohp_recent_audio& p = i == first ? head : pieces[i];
+        aSilence = p.silence != 0;
+        aAtt = p.silence ? OHP_UNITY_ATTENUATION : p.attenuation;
+        if (p.silence) {
+            aFirstFrame = 0;
+            aFrames = p.jiffies / jps;
+        }
+        else {
+            aFirstFrame = p.pcm_jiffies / jps;
+            aFrames = (uint32_t)((p.pcm_jiffies + p.jiffies) / jps - aFirstFrame);
+        }
+        return p.silence || (p.pcm_jiffies + p.jiffies) / jps <= sp.total_frames;
+    };
+    uint64_t got = 0;
+    uint32_t firstRun = aNumPieces, lastRun = aNumPieces; // the first and last pieces that give frames
+    for (uint32_t i = first; i < aNumPieces; i++) {
+        bool silence; uint64_t firstFrame; uint32_t frames, att;
+        if (!run(i, silence, firstFrame, frames, att)) return OHP_E_INVALID_ARG; // a piece outside the stream
+        if (frames == 0) continue;
+        if (firstRun == aNumPieces) firstRun = i;
+        lastRun = i;
+        got += frames;
+    }
+    if (got < train || got > (uint64_t)train + 1u) return OHP_E_INVALID_ARG;
+    const uint8_t le = (uint8_t)((sp.in_little_endian && B > 1) ? OHP_F_IN_LITTLE_ENDIAN : 0);
+    bool full = false;
+    // frames [aFrom, aFrom + aCount) of piece i, channels [aCh, aCh + aChannels), to slot aSlot of plane aCh and on
+    auto emit = [&](uint32_t i, uint32_t aFrom, uint32_t aCount, uint32_t aCh, uint32_t aChannels, uint64_t aSlot) {
+        if (aNumPrep == OHP_FLYWHEEL_MAX_PREP_RECENT) { full = true; return; }
+        bool silence; uint64_t firstFrame; uint32_t frames, att;
+        (void)run(i, silence, firstFrame, frames, att);
+        ohp_chunk_desc d = zero_desc();
+        d.src_off = silence ? 0 : sp.src_base + (firstFrame + aFrom) * frameBytes + (uint64_t)aCh * B;
+        d.dst_off = aTrainingOff + aSlot * 4u;
+        d.bytes = aCount * aChannels * B;
+        d.ramp_start = (uint16_t)core::kRampMax;
+        d.ramp_end = (uint16_t)core::kRampMax;
+        d.attenuation = (uint16_t)att;
+        d.bit_depth = (uint8_t)sp.bit_depth;
+        d.channels = (uint8_t)aChannels;
+        d.flags = (uint8_t)(silence ? OHP_F_SILENCE : le);
+        d.out_fmt = OHP_OUT_PLANAR32_BE;
+        d.aux = (uint16_t)train;
+        prep[aNumPrep++] = d;
+    };
+    // frames [lo, hi) of those read go out whole; with a frame too many and more than one channel, every plane's first slot
+    // is written last by another frame (as ohp_flywheel_plan_recent)
+    const bool over = got == (uint64_t)train + 1u;
+    const uint64_t lo = (over && C > 1) ? 1 : 0, hi = train;
+    uint64_t at = 0;
+    for (uint32_t i = first; i < aNumPieces; i++) {
+        bool silence; uint64_t firstFrame; uint32_t frames, att;
+        (void)run(i, silence, firstFrame, frames, att);
+        if (frames == 0) continue;
+        const uint64_t a = at > lo ? at : lo, b = (at + frames) < hi ? (at + frames) : hi;
+        if (b > a) emit(i, (uint32_t)(a - at), (uint32_t)(b - a), 0, C, a);
+        at += frames;
+    }
+    if (over && C > 1) {
+        bool silence; uint64_t firstFrame; uint32_t frames, att;
+        (void)run(lastRun, silence, firstFrame, frames, att);
+        emit(firstRun, 0, 1, 0, 1, 0);
+        for (uint32_t c = 1; c < C; c++) emit(lastRun, frames - 1, 1, c - 1, 1, (uint64_t)c * train);
+    }
+    if (full) {
+        aNumPrep = 0;
+        return OHP_E_INVALID_ARG;
+    }
+    job.src_off = aTrainingOff;
+    job.dst_off = aGeneratedOff;
+    job.sample_rate = sp.sample_rate;
+    job.out_frames = OHP_FLYWHEEL_RAMP_JIFFIES / jps;
+    job.train_frames = (uint16_t)train;
+    job.channels = (uint8_t)C;
+    job.bit_depth = (uint8_t)sp.bit_depth;
+    job.reserved = 0;
+    const int rc = ramp_chunks(job, sv.ramp, aGeneratedOff, aOutOff, blocks, aNumBlocks);
+    if (rc != OHP_OK) aNumPrep = 0;
+    return rc;
+}
+
 } // namespace flyplan
 } // namespace ohp

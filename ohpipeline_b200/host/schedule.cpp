@@ -585,7 +585,7 @@ static int plan_batch(const ohp_stream_spec* streams, size_t n_streams, const oh
             return OHP_E_INVALID_ARG;
         }
         const ohp_stream_spec& sp = streams[sv.stream];
-        ohp_chunk_desc prep[64];
+        ohp_chunk_desc prep[OHP_FLYWHEEL_MAX_PREP_RECENT];
         ohp_chunk_desc blocks[OHP_FLYWHEEL_RAMP_JIFFIES / OHP_FLYWHEEL_BLOCK_JIFFIES + 1];
         ohp_flywheel_job job;
         size_t n_prep = 0, n_blocks = 0;

@@ -17,6 +17,7 @@
 #include <cstdint>
 
 #include "../../include/ohp_schedule.h"
+#include "../../include/ohp_starvation_recent.h"
 #include "ramp_core.h"
 #include "codec_source.h"
 
@@ -107,6 +108,89 @@ struct Starve
     uint32_t pcmRunAtt;  // a MsgSilence passed or a flywheel ramp used the recent audio up
     uint32_t elemRamp;   // what the element's own SetRamp calls last returned (StarvationRamper::iCurrentRampValue)
 };
+
+// RECENT walks: the recent audio a StarvationRamper keeps (stage_chain.h NoteRecent / TrimRecent) in a ring of
+// kRecentPieces per stage.  A piece is 16 bytes: where its PCM begins (kSilencePiece: a MsgSilence), jiffies, attenuation.
+constexpr uint32_t kRecentPieces = OHP_DEVICE_RECENT_PIECES;
+static_assert((kRecentPieces & (kRecentPieces - 1)) == 0, "the ring wraps with a mask");
+constexpr uint64_t kSilencePiece = ~0ull;
+
+struct RecentPiece
+{
+    uint64_t pcm;
+    uint32_t jiffies;
+    uint32_t attenuation;
+};
+
+struct RecentRing
+{
+    RecentPiece p[kRecentPieces];
+    uint64_t total;      // jiffies of the pieces held
+    uint32_t head, count;
+    uint32_t dropped;    // a push found the ring full since it was last emptied
+};
+
+// What a walk keeps for the recent audio: nothing, or the rings and where the records' pieces go (record of the stream's
+// k-th event: count[k], pieces out[k * kRecentPieces ...]).
+template <bool RECENT> struct RecentCtx {};
+template <> struct RecentCtx<true>
+{
+    ohp_recent_audio* out;
+    uint32_t* count;
+    uint32_t stride;     // team size: lane i writes pieces i, i + stride, ...
+    RecentRing ring[kStages];
+};
+
+OHP_HD void recent_clear(RecentRing& r)
+{
+    r.total = 0; r.head = 0; r.count = 0; r.dropped = 0;
+}
+
+// TrimRecent: pieces the last millisecond no longer needs go; a lone run of PCM keeps its last 2 ms
+OHP_HD void recent_trim(RecentRing& r)
+{
+    while (r.count > 1 && r.total - r.p[r.head].jiffies >= OHP_FLYWHEEL_TRAINING_JIFFIES) {
+        r.total -= r.p[r.head].jiffies;
+        r.head = (r.head + 1) & (kRecentPieces - 1);
+        r.count--;
+    }
+    RecentPiece& front = r.p[r.head];
+    if (r.count == 1 && front.pcm != kSilencePiece && front.jiffies > 4u * OHP_FLYWHEEL_TRAINING_JIFFIES) {
+        const uint32_t drop = front.jiffies - 2u * OHP_FLYWHEEL_TRAINING_JIFFIES;
+        front.pcm += drop;
+        front.jiffies -= drop;
+        r.total -= drop;
+    }
+}
+
+// NoteRecent: a piece joins the last one where it continues it, else the ring.  A push into a full ring drops the oldest
+// piece.  That loses something only where the class model would keep it -- where the pieces behind it add up to less
+// than 1 ms -- and then the ring holds less than 1 ms until it is emptied: see note_starvation.
+OHP_HD void recent_note(RecentRing& r, uint64_t aPcm, uint32_t aJiffies, uint32_t aAttenuation)
+{
+    if (aJiffies == 0) return;
+    if (aPcm != kSilencePiece && r.count != 0) {
+        RecentPiece& last = r.p[(r.head + r.count - 1) & (kRecentPieces - 1)];
+        if (last.pcm != kSilencePiece && last.attenuation == aAttenuation && last.pcm + last.jiffies == aPcm
+            && (uint64_t)last.jiffies + aJiffies <= 0x7fffffffu) {
+            last.jiffies += aJiffies;
+            r.total += aJiffies;
+            recent_trim(r);
+            return;
+        }
+    }
+    if (r.count == kRecentPieces) {
+        r.total -= r.p[r.head].jiffies;
+        r.head = (r.head + 1) & (kRecentPieces - 1);
+        r.count--;
+        r.dropped = 1;
+    }
+    RecentPiece& p = r.p[(r.head + r.count) & (kRecentPieces - 1)];
+    p.pcm = aPcm; p.jiffies = aJiffies; p.attenuation = aAttenuation;
+    r.count++;
+    r.total += aJiffies;
+    recent_trim(r);
+}
 
 struct StreamCtx
 {
@@ -446,8 +530,9 @@ OHP_HD bool apply_event(Stage& s, uint32_t op, uint32_t arg)
     return true;
 }
 
-// stage_chain.h NoteStarvation(): called in front of every event a stage applies
-OHP_HD void note_starvation(StreamCtx& cx, const Stage& s, uint32_t stage, uint32_t aEvent)
+// stage_chain.h NoteStarvation(): called in front of every event a stage applies.  RECENT: the record's pieces too.
+template <bool RECENT>
+OHP_HD void note_starvation(StreamCtx& cx, RecentCtx<RECENT>& rs, const Stage& s, uint32_t stage, uint32_t aEvent)
 {
     if (s.elem != ElemStarvation || cx.ev[aEvent].op != OHP_EV_STARVATION) return;
     const bool plays = (s.mode == Running && !s.halted) || (s.mode == RampingUp && s.current != core::kRampMin); // as apply_element_event
@@ -464,6 +549,24 @@ OHP_HD void note_starvation(StreamCtx& cx, const Stage& s, uint32_t stage, uint3
         o.reserved = 0;
         cx.rec[cx.recAppend ? cx.nRec++ : aEvent] = o;
     }
+    if constexpr (RECENT) {
+        // the class model's record holds more than kRecentPieces pieces exactly where the ring dropped one and holds less
+        // than 1 ms (recent_note): such a record is incomplete, and the planner refuses it
+        RecentRing& g = rs.ring[stage];
+        const bool incomplete = g.dropped && g.total < OHP_FLYWHEEL_TRAINING_JIFFIES;
+        if (cx.lane == 0) rs.count[aEvent] = incomplete ? OHP_RECENT_INCOMPLETE : g.count;
+        for (uint32_t i = cx.lane; !incomplete && i < g.count; i += rs.stride) {
+            const RecentPiece& q = g.p[(g.head + i) & (kRecentPieces - 1)];
+            ohp_recent_audio a;
+            a.pcm_jiffies = q.pcm == kSilencePiece ? 0 : q.pcm;
+            a.jiffies = q.jiffies;
+            a.silence = q.pcm == kSilencePiece ? 1u : 0u;
+            a.attenuation = q.attenuation;
+            a.reserved = 0;
+            rs.out[(uint64_t)aEvent * kRecentPieces + i] = a;
+        }
+        if (plays) recent_clear(g);
+    }
     if (plays) { r.pcmRun = 0; r.elemRamp = core::kRampMin; } // Pull(): FlywheelRamping -> RampingUp from kMin
 }
 
@@ -476,11 +579,11 @@ OHP_HD bool push_msg(Stage& s, Packed* aRow, const Msg& m)
 
 // stage_chain.h Process(): one message through one stage; split remainders go onto the stage's stack (aRow).
 // RECORD: aAttUp is the attenuation the stages in front of this one leave PCM with (their last that is not unity).
-template <bool RECORD>
-OHP_HD uint32_t stage_process(StreamCtx& cx, Stage& s, uint32_t stage, Packed* aRow, Msg& msg, uint32_t aAttUp)
+template <bool RECORD, bool RECENT>
+OHP_HD uint32_t stage_process(StreamCtx& cx, RecentCtx<RECENT>& rs, Stage& s, uint32_t stage, Packed* aRow, Msg& msg, uint32_t aAttUp)
 {
     while (s.nextAt <= s.pos) {
-        if (RECORD) note_starvation(cx, s, stage, s.nextEv);
+        if (RECORD) note_starvation<RECENT>(cx, rs, s, stage, s.nextEv);
         const ohp_ramp_event& e = cx.ev[s.nextEv];
         if (!apply_event(s, e.op, e.arg)) return kErrAssert;
         stage_seek(cx, s, stage, s.nextEv + 1);
@@ -490,7 +593,7 @@ OHP_HD uint32_t stage_process(StreamCtx& cx, Stage& s, uint32_t stage, Packed* a
         uint32_t at = (uint32_t)(s.nextAt - s.pos);
         if (msg.silence) at -= at % cx.jps; // silence only splits on sample blocks
         if (at == 0) {
-            if (RECORD) note_starvation(cx, s, stage, s.nextEv);
+            if (RECORD) note_starvation<RECENT>(cx, rs, s, stage, s.nextEv);
             const ohp_ramp_event& e = cx.ev[s.nextEv];
             if (!apply_event(s, e.op, e.arg)) return kErrAssert;
             stage_seek(cx, s, stage, s.nextEv + 1);
@@ -514,6 +617,9 @@ OHP_HD uint32_t stage_process(StreamCtx& cx, Stage& s, uint32_t stage, Packed* a
         if (msg.silence) { // the element reacts, the message is handed on untouched
             element_sees_silence(s);
             if (RECORD) cx.sv[stage].pcmRun = 0;
+            if constexpr (RECENT) {
+                if (s.elem == ElemStarvation) recent_note(rs.ring[stage], kSilencePiece, msg.size, OHP_UNITY_ATTENUATION);
+            }
             s.pos += msg.size;
             return kOk;
         }
@@ -548,6 +654,7 @@ OHP_HD uint32_t stage_process(StreamCtx& cx, Stage& s, uint32_t stage, Packed* a
         Starve& r = cx.sv[stage];
         const uint32_t att = s.attenuation != OHP_UNITY_ATTENUATION ? s.attenuation : aAttUp;
         if (att != r.pcmRunAtt) { r.pcmRun = 0; r.pcmRunAtt = att; }
+        if constexpr (RECENT) recent_note(rs.ring[stage], r.pcmJiffies, msg.size, att);
         r.pcmJiffies += msg.size;
         r.pcmRun += msg.size;
     }
@@ -656,10 +763,12 @@ OHP_HD uint32_t next_message(core::CodecSource& src, Lookahead& la)
 // UNIFORM: src.read == 0 (compiled separately so that the uniform case pays nothing for the ragged one's tests).
 // RECORD: the StarvationRamper stages' PCM counters advance by the run (no event falls inside it, no MsgSilence either);
 // the element's ramp value follows the recurrence where it is the stage that ramps.
-template <bool EMIT, int STRIDE, bool UNIFORM, bool RECORD>
-OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[kStages], core::CodecSource& src, Lookahead& la,
-                          Cursor& cur, uint32_t& aErr)
+// RECENT: the run joins the recent audio as one piece.
+template <bool EMIT, int STRIDE, bool UNIFORM, bool RECORD, bool RECENT>
+OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, RecentCtx<RECENT>& rs, Stage (&st)[kStages], core::CodecSource& src,
+                          Lookahead& la, Cursor& cur, uint32_t& aErr)
 {
+    (void)rs;
     aErr = kOk;
     if (!(cx.bits == 8 || cx.bits == 16 || cx.bits == 24 || cx.bits == 32)) return 0;
     constexpr bool uniform = UNIFORM;
@@ -919,6 +1028,7 @@ OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[
                 if (st[j].attenuation != OHP_UNITY_ATTENUATION) att = st[j].attenuation;
             }
             if (att != r.pcmRunAtt) { r.pcmRun = 0; r.pcmRunAtt = att; }
+            if constexpr (RECENT) recent_note(rs.ring[i], r.pcmJiffies, (uint32_t)posJiffies, att);
             r.pcmJiffies += posJiffies;
             r.pcmRun += posJiffies;
         }
@@ -933,9 +1043,10 @@ OHP_HD uint32_t bulk_step(const ohp_stream_spec& sp, StreamCtx& cx, Stage (&st)[
 // the remaining stages (in registers), hand it to the driver, then resume with the top of the deepest non-empty stack.
 // A team of STRIDE threads (device: a warp, or 1; host: 1) walks the stream holding identical state; they differ only
 // in cx.lane, i.e. in which messages of a bulk step they emit.  BULK = false is the message-at-a-time walk alone.
-template <bool EMIT, int STRIDE, bool BULK, bool RECORD>
-OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
+template <bool EMIT, int STRIDE, bool BULK, bool RECORD, bool RECENT>
+OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx, RecentCtx<RECENT>& rs)
 {
+    static_assert(RECORD || !RECENT, "the recent audio goes with the records");
     Packed stack[kStages][kStackDepth];
     Stage st[kStages];
 #if defined(__CUDA_ARCH__)
@@ -947,6 +1058,7 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
         st[i].elem = stage_element(cx, (uint32_t)i);
         st[i].halted = 1;
         if (RECORD) { cx.sv[i].pcmJiffies = 0; cx.sv[i].pcmRun = 0; cx.sv[i].pcmRunAtt = OHP_UNITY_ATTENUATION; cx.sv[i].elemRamp = core::kRampMax; }
+        if constexpr (RECENT) recent_clear(rs.ring[i]);
         if (st[i].elem == ElemStarvation) st[i].maxMsg = 5u * OHP_JIFFIES_PER_MS; // kMaxAudioOutJiffies, StarvationRamper.cpp:376
         stage_seek(cx, st[i], (uint32_t)i, 0);
     }
@@ -970,7 +1082,7 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
 #endif
             for (int i = 0; i < kStages; i++) {
                 if (i >= from) {
-                    const uint32_t e = stage_process<RECORD>(cx, st[i], (uint32_t)i, stack[i], m, attUp);
+                    const uint32_t e = stage_process<RECORD, RECENT>(cx, rs, st[i], (uint32_t)i, stack[i], m, attUp);
                     if (e != kOk) return e;
                 }
                 if (RECORD && st[i].attenuation != OHP_UNITY_ATTENUATION) attUp = st[i].attenuation;
@@ -1003,8 +1115,8 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
     for (;;) {
         if (BULK) {
             uint32_t e;
-            const uint32_t n = source.read == 0 ? bulk_step<EMIT, STRIDE, true, RECORD>(sp, cx, st, source, la, cur, e)
-                                                : bulk_step<EMIT, STRIDE, false, RECORD>(sp, cx, st, source, la, cur, e);
+            const uint32_t n = source.read == 0 ? bulk_step<EMIT, STRIDE, true, RECORD, RECENT>(sp, cx, rs, st, source, la, cur, e)
+                                                : bulk_step<EMIT, STRIDE, false, RECORD, RECENT>(sp, cx, rs, st, source, la, cur, e);
             if (e != kOk) return e;
 #ifdef OHP_WALK_STATS
             if (n != 0) { g_bulk_calls++; g_bulk_msgs += n; }
@@ -1047,7 +1159,7 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
         for (int i = 0; i < kStages; i++) {
             Stage& s = st[i];
             while (s.elem == ElemStarvation && s.nextAt <= s.pos) {
-                note_starvation(cx, s, (uint32_t)i, s.nextEv);
+                note_starvation<RECENT>(cx, rs, s, (uint32_t)i, s.nextEv);
                 const ohp_ramp_event& e = cx.ev[s.nextEv];
                 (void)apply_element_event(s, e.op, e.arg); // OHP_EV_HALT / OHP_EV_STARVATION: state only
                 stage_seek(cx, s, (uint32_t)i, s.nextEv + 1);
@@ -1061,11 +1173,14 @@ OHP_HD uint32_t walk_stream(const ohp_stream_spec& sp, StreamCtx& cx)
 // aLane: this thread's index in its team of STRIDE (0 on the host).
 // RECORD: starvation records go to aRec -- the record of the stream's k-th event at aRec[k] (aRec: the stream's first
 // event's place in an array over the whole events array), or, with aAppend, one after the other; aNumRecords counts them.
-template <bool EMIT, int STRIDE = 1, bool BULK = true, bool RECORD = false>
+// RECENT (not with aAppend): the k-th event's record also leaves its pieces of recent audio at aRecent[k * kRecentPieces ...]
+// and their number at aRecentCount[k] (both at the stream's first event's place, as aRec).
+template <bool EMIT, int STRIDE = 1, bool BULK = true, bool RECORD = false, bool RECENT = false>
 OHP_HD uint32_t run_stream(const ohp_stream_spec& sp, const ohp_ramp_event* aEvents, uint64_t aNumEvents,
                            ohp_chunk_desc* aDescs, ohp_chunk_info* aInfo, uint64_t& aNumChunks, uint64_t& aOutBytes,
                            uint32_t aLane = 0, uint64_t aLimit = ~0ull,
-                           ohp_starvation* aRec = nullptr, uint64_t aStream = 0, bool aAppend = false, uint32_t* aNumRecords = nullptr)
+                           ohp_starvation* aRec = nullptr, uint64_t aStream = 0, bool aAppend = false, uint32_t* aNumRecords = nullptr,
+                           ohp_recent_audio* aRecent = nullptr, uint32_t* aRecentCount = nullptr)
 {
     aNumChunks = 0;
     aOutBytes = 0;
@@ -1096,7 +1211,10 @@ OHP_HD uint32_t run_stream(const ohp_stream_spec& sp, const ohp_ramp_event* aEve
         cx.stream = aStream;
         cx.firstEvent = sp.first_event;
     }
-    const uint32_t rc = walk_stream<EMIT, STRIDE, BULK, RECORD>(sp, cx);
+    RecentCtx<RECENT> rs;
+    if constexpr (RECENT) { rs.out = aRecent; rs.count = aRecentCount; rs.stride = (uint32_t)STRIDE; }
+    else { (void)aRecent; (void)aRecentCount; }
+    const uint32_t rc = walk_stream<EMIT, STRIDE, BULK, RECORD, RECENT>(sp, cx, rs);
     if (RECORD && aNumRecords) *aNumRecords = cx.nRec;
     if (rc != kOk) return rc;
     aNumChunks = cx.nChunks;

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""ohp_run_streams_device_flywheel on a scaled `elements` batch (default 4096 streams x 1 s, every stream with a
+"""ohp_run_streams_device_flywheel and ohp_run_streams_device_flywheel_recent on a scaled `elements` batch (default 4096 streams x 1 s, every stream with a
 StarvationRamper stage): what recording, planning and the three flywheel launches cost on top of ohp_run_streams_device
-on the same batch, and the same work through the host route (ohp_schedule_build on every host core ->
+on the same batch (the recent-audio call alternating with the other two: it also keeps the recent audio in the walk and
+plays the starvations with silence in their last millisecond), and the same work through the host route (ohp_schedule_build on every host core ->
 ohp_flywheel_plan_batch -> upload -> process / flywheel / process) in wall clock.  Both device calls are timed as host
 wall clock around call + stream synchronise, alternating, after warm-up; the card's name and power limit are read in
 the same run.  With --out DIR the result is also written to DIR/starvation_bench.json.
@@ -53,6 +54,9 @@ def main():
     d_off = torch.zeros(ne, dtype=torch.int64, device="cuda")
     d_len = torch.zeros(ne, dtype=torch.int64, device="cuda")
     d_rec = torch.zeros(ne * abi.STARVATION.itemsize, dtype=torch.uint8, device="cuda")
+    d_len_r = torch.zeros(ne, dtype=torch.int64, device="cuda")
+    d_recent = torch.zeros(ne * abi.DEVICE_RECENT_PIECES * abi.RECENT_AUDIO.itemsize, dtype=torch.uint8, device="cuda")
+    d_count = torch.zeros(ne, dtype=torch.int32, device="cuda")
     args = (d_streams.data_ptr(), len(w.streams), d_events.data_ptr(), ne, d_in.data_ptr(), w.in_bytes, d_out.data_ptr(), w.out_bytes)
 
     def plain():
@@ -62,6 +66,11 @@ def main():
     def fly():
         ctx.run_streams_device_flywheel(*args, d_fly.data_ptr(), fly_bytes, d_off.data_ptr(), d_len.data_ptr(), d_rec.data_ptr(),
                                         want_total=False)
+        ctx.sync()
+
+    def fly_recent():
+        ctx.run_streams_device_flywheel_recent(*args, d_fly.data_ptr(), fly_bytes, d_off.data_ptr(), d_len_r.data_ptr(), d_rec.data_ptr(),
+                                               want_total=False, d_recent=d_recent.data_ptr(), d_recent_count=d_count.data_ptr())
         ctx.sync()
 
     def host_route():
@@ -83,22 +92,29 @@ def main():
         return (time.perf_counter() - t) * 1e3, r
 
     for _ in range(3):
-        plain(); fly()  # noqa: E702
-    tp, tf = [], []
+        plain(); fly(); fly_recent()  # noqa: E702
+    tp, tf, tr = [], [], []
     for _ in range(a.reps):
         tp.append(timed(plain)[0])
         tf.append(timed(fly)[0])
+        tr.append(timed(fly_recent)[0])
     th = []
     for _ in range(3):
         ms, (n_records, n_planned) = timed(host_route)
         th.append(ms)
     played = int((d_len.cpu().numpy() != 0).sum())
+    played_recent = int((d_len_r.cpu().numpy() != 0).sum())
+    sched = capi.schedule_build(w.streams, w.events)
+    n_planned_recent = len(capi.flywheel_plan_batch(w.streams, sched.starvations, recent=sched.recent,
+                                                    recent_begin=sched.recent_begin).planned)
     res = {
         "card": card(), "streams": len(w.streams), "seconds": a.seconds, "events": ne,
         "starvation_events": int((w.events["op"] == abi.EV_STARVATION).sum()), "records": n_records,
-        "planned_host": n_planned, "played_device": played, "fly_bytes": fly_bytes, "in_bytes": w.in_bytes, "out_bytes": w.out_bytes,
+        "planned_host": n_planned, "played_device": played, "planned_host_recent": n_planned_recent,
+        "played_device_recent": played_recent, "fly_bytes": fly_bytes, "in_bytes": w.in_bytes, "out_bytes": w.out_bytes,
         "run_streams_device_ms": {"median": float(np.median(tp)), "min": float(np.min(tp)), "max": float(np.max(tp))},
         "run_streams_device_flywheel_ms": {"median": float(np.median(tf)), "min": float(np.min(tf)), "max": float(np.max(tf))},
+        "run_streams_device_flywheel_recent_ms": {"median": float(np.median(tr)), "min": float(np.min(tr)), "max": float(np.max(tr))},
         "host_route_ms": {"median": float(np.median(th)), "min": float(np.min(th)), "max": float(np.max(th))},
         "host_cores": os.cpu_count(),
     }
