@@ -149,7 +149,8 @@ int         ohp_process_host(ohp_context* ctx, const ohp_chunk_desc* h_descs, si
                              const uint8_t* h_in, uint64_t in_bytes,
                              uint8_t* h_out, uint64_t out_bytes);
 /* Wait for everything enqueued on the context's stream (or `stream`) and report device-side
- * descriptor errors. */
+ * descriptor errors.  An error is reported once, by the first call or ohp_sync that reads it;
+ * ohp_last_error names every error found. */
 int         ohp_sync(ohp_context* ctx, void* stream);
 
 /*

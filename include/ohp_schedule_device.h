@@ -73,7 +73,11 @@ int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, siz
  *     stream ever have more playables than its region holds (none of this repo's generators produces one; the bound is
  *     held against exact counts in the tests) -- redo the batch through count + emit.  Without it that case is an
  *     OHP_E_NO_MEMORY from the next ohp_sync.
- * One call at a time per context.  Environment (tests): OHP_ONE_WALK=0 takes count + scan + emit.
+ * Calls on one context may follow one another on any streams without an ohp_sync in between: a call that uses the
+ * context's scratch (this one, its flywheel variants, ohp_process_host, ohp_run_streams_host) waits on the device for
+ * the previous such call's work.  One host thread at a time per context.  The status block is the context's: when the
+ * work of two calls on two streams fails at once, the first ohp_sync of either reports both.
+ * Environment (tests): OHP_ONE_WALK=0 takes count + scan + emit.
  * Errors as ohp_run_streams_host.
  */
 int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,

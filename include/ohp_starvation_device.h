@@ -12,7 +12,8 @@
  *      RampGenerator's ramped 1 ms blocks (INTEGRATION.md 1b) as three launches.
  * Everything is enqueued on `stream` (NULL = the context's own); the host waits only for what ohp_run_streams_device waits
  * for, which now also carries the flywheel slots' total.  A batch without starvation events launches what
- * ohp_run_streams_device launches.  One call at a time per context.
+ * ohp_run_streams_device launches.  Calls may follow one another on any streams without an ohp_sync in between, one host
+ * thread at a time per context (ohp_schedule_device.h).
  *
  * FLYWHEEL OUTPUT.  Event e of the events array gets a slot of d_fly_out at d_fly_off[e] = the sum, over the
  * OHP_EV_STARVATION events before it in the array, of align16(Jiffies::ToSamples(20 ms, rate) x frame bytes) of the stream

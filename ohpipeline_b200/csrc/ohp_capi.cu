@@ -86,6 +86,7 @@ struct ohp_context
     uint64_t* d_counts = nullptr; uint64_t d_counts_cap = 0;  // ohp_run_streams_device: exact playables per stream
     cudaEvent_t sched_event = nullptr;                           // ... recorded behind a copy the host waits for
     cudaEvent_t fly_event = nullptr;                             // ohp_run_streams_device_flywheel: behind the planned jobs' count
+    cudaEvent_t scratch_done = nullptr;                          // behind the last call that used the scratch (ScratchTurn)
     uint64_t* h_regions = nullptr;                               // ... the regions' total (pinned; [4..8): sched::FlySlots)
     // ohp_run_streams_device_flywheel (grown on demand)
     ohp_starvation* d_records = nullptr; uint64_t d_records_cap = 0; // when the caller passes no record array
@@ -172,6 +173,32 @@ struct DrainOnExit
     }
     DrainOnExit(const DrainOnExit&) = delete;
     DrainOnExit& operator=(const DrainOnExit&) = delete;
+};
+
+// The context's scratch (the staging arenas, d_descs, d_begin, d_counts, the flywheel and recent-audio buffers) is shared
+// by every call that stages through it -- ohp_process_host, ohp_run_streams_host, ohp_run_streams_device and its flywheel
+// variants -- and the asynchronous ones return while their kernels still read it.  Each such call holds a ScratchTurn:
+// on entry the caller's stream, the compute stream and the H2D stream wait (on the device, not the host) for the
+// previous call's work, and however the call returns its own work is recorded behind it.  So calls may follow one another
+// on any streams without an ohp_sync in between; a never-recorded event is no wait at all.
+struct ScratchTurn
+{
+    ohp_context* ctx;
+    cudaStream_t st;
+    int rc = OHP_OK; // OHP_E_CUDA when a wait could not be enqueued: the call must not go on
+    ScratchTurn(ohp_context* c, cudaStream_t s) : ctx(c), st(s)
+    {
+        for (cudaStream_t w : {s, c->stream, c->copy_in}) {
+            const cudaError_t e = cudaStreamWaitEvent(w, c->scratch_done, 0);
+            if (e != cudaSuccess) { rc = fail(c, OHP_E_CUDA, "cudaStreamWaitEvent (context scratch)", e); break; }
+        }
+    }
+    ~ScratchTurn()
+    {
+        if (cudaEventRecord(ctx->scratch_done, st) != cudaSuccess) (void)cudaGetLastError();
+    }
+    ScratchTurn(const ScratchTurn&) = delete;
+    ScratchTurn& operator=(const ScratchTurn&) = delete;
 };
 
 // What a host-buffer call copies back.  Only bytes some chunk writes belong to the call: everything else in h_out is
@@ -426,58 +453,80 @@ static int grow_idle(ohp_context* ctx, T*& ptr, uint64_t& cap, uint64_t need)
     return grow(ctx, ptr, cap, need);
 }
 
+// What words [2], [3] of the status block (the schedule kernels') say, bits != 0: the status, and the message in buf.
+static int schedule_error(uint32_t bits, uint32_t stream_word, char* buf, size_t size)
+{
+    const uint32_t stream_index = 0xffffffffu - stream_word;
+    if (bits & (1u << sched::kErrSpec)) {
+        std::snprintf(buf, size, "stream %u: spec not representable (rate, frame size, chunk size, event slice or sink)", stream_index);
+        return OHP_E_INVALID_ARG;
+    }
+    if (bits & (1u << sched::kErrAssert)) {
+        std::snprintf(buf, size, "stream %u: the reference would ASSERT on this schedule", stream_index);
+        return OHP_E_INVALID_DESC;
+    }
+    if (bits & (1u << sched::kErrBound)) {
+        std::snprintf(buf, size, "stream %u: more playables than its descriptor region holds", stream_index);
+        return OHP_E_NO_MEMORY;
+    }
+    std::snprintf(buf, size, "stream %u: more than %d pending message splits in one stage", stream_index, sched::kStackDepth);
+    return OHP_E_NO_MEMORY;
+}
+
+// ohp_schedule_count_device: only the schedule kernels have run on the caller's buffers
 static int schedule_status(ohp_context* ctx, cudaStream_t st)
 {
-    // words [2], [3] of the status block belong to the schedule kernels
     OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_status, ctx->d_status, 16 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     OHP_CUDA(ctx, cudaStreamSynchronize(st));
     const uint32_t bits = ctx->h_status[2];
     if (bits == 0) return OHP_OK;
-    const uint32_t stream_index = 0xffffffffu - ctx->h_status[3];
+    const uint32_t stream_word = ctx->h_status[3];
     OHP_CUDA(ctx, cudaMemsetAsync(ctx->d_status + 2, 0, 2 * sizeof(uint32_t), st));
     OHP_CUDA(ctx, cudaStreamSynchronize(st));
     char buf[160];
-    if (bits & (1u << sched::kErrSpec)) {
-        std::snprintf(buf, sizeof buf, "stream %u: spec not representable (rate, frame size, chunk size, event slice or sink)", stream_index);
-        return fail(ctx, OHP_E_INVALID_ARG, buf);
-    }
-    if (bits & (1u << sched::kErrAssert)) {
-        std::snprintf(buf, sizeof buf, "stream %u: the reference would ASSERT on this schedule", stream_index);
-        return fail(ctx, OHP_E_INVALID_DESC, buf);
-    }
-    if (bits & (1u << sched::kErrBound)) {
-        std::snprintf(buf, sizeof buf, "stream %u: more playables than its descriptor region holds", stream_index);
-        return fail(ctx, OHP_E_NO_MEMORY, buf);
-    }
-    std::snprintf(buf, sizeof buf, "stream %u: more than %d pending message splits in one stage", stream_index, sched::kStackDepth);
-    return fail(ctx, OHP_E_NO_MEMORY, buf);
+    const int status = schedule_error(bits, stream_word, buf, sizeof buf);
+    return fail(ctx, status, buf);
 }
 
+// Every error word of the status block -- [0], [1] the chunk kernels', [2], [3] the schedule kernels', [12], [13] the
+// flywheel kernel's -- is read and cleared together, so that an error is reported once, by the first call or ohp_sync that
+// reads it, and never again by a later one.  The status is the first of: a flywheel job, a stream the walk refused, a chunk
+// descriptor (or the watchdog); ohp_last_error names every error found, in that order.
 static int read_status(ohp_context* ctx, cudaStream_t st)
 {
     OHP_CUDA(ctx, cudaMemcpyAsync(ctx->h_status, ctx->d_status, 16 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     OHP_CUDA(ctx, cudaStreamSynchronize(st));
-    const uint32_t fly_bits = ctx->h_status[12];
-    if (fly_bits != 0) {
-        // words [12], [13] belong to the flywheel kernel
-        const uint32_t job = ctx->h_status[13];
-        OHP_CUDA(ctx, cudaMemsetAsync(ctx->d_status + 12, 0, 2 * sizeof(uint32_t), st));
-        OHP_CUDA(ctx, cudaStreamSynchronize(st));
-        char fbuf[128];
-        std::snprintf(fbuf, sizeof fbuf, "device rejected flywheel job %u (%s)", job - 1, (fly_bits & 1u) ? "invalid" : "out of range");
-        return fail(ctx, (fly_bits & 1u) ? OHP_E_INVALID_DESC : OHP_E_OUT_OF_RANGE, fbuf);
-    }
-    if (ctx->h_status[2] != 0) return schedule_status(ctx, st); // a walk enqueued by ohp_run_streams_device refused a stream
-    const uint32_t bits = ctx->h_status[0];
-    if (bits == 0) return OHP_OK;
-    const uint32_t first = ctx->h_status[1];
-    OHP_CUDA(ctx, cudaMemsetAsync(ctx->d_status, 0, 16 * sizeof(uint32_t), st));
+    const uint32_t fly_bits = ctx->h_status[12], job = ctx->h_status[13];
+    const uint32_t sched_bits = ctx->h_status[2], stream_word = ctx->h_status[3];
+    const uint32_t bits = ctx->h_status[0], first = ctx->h_status[1];
+    if (fly_bits == 0 && sched_bits == 0 && bits == 0) return OHP_OK;
+    OHP_CUDA(ctx, cudaMemsetAsync(ctx->d_status, 0, 4 * sizeof(uint32_t), st));
+    OHP_CUDA(ctx, cudaMemsetAsync(ctx->d_status + 12, 0, 2 * sizeof(uint32_t), st));
     OHP_CUDA(ctx, cudaStreamSynchronize(st));
-    char buf[128];
-    if (bits & kErrWatchdog) return fail(ctx, OHP_E_CUDA, "kernel watchdog: a pipeline barrier never completed");
-    std::snprintf(buf, sizeof buf, "device rejected chunk descriptor %u (%s)", first - 1,
-                  (bits & kErrInvalidDesc) ? "invalid" : "out of range");
-    return fail(ctx, (bits & kErrInvalidDesc) ? OHP_E_INVALID_DESC : OHP_E_OUT_OF_RANGE, buf);
+    int status = OHP_OK;
+    std::string msg;
+    auto note = [&](int s, const char* what) {
+        if (status == OHP_OK) status = s;
+        if (!msg.empty()) msg += "; ";
+        msg += what;
+    };
+    char buf[160];
+    if (fly_bits != 0) {
+        std::snprintf(buf, sizeof buf, "device rejected flywheel job %u (%s)", job - 1, (fly_bits & 1u) ? "invalid" : "out of range");
+        note((fly_bits & 1u) ? OHP_E_INVALID_DESC : OHP_E_OUT_OF_RANGE, buf);
+    }
+    if (sched_bits != 0) { // a walk enqueued by ohp_run_streams_device refused a stream
+        const int s = schedule_error(sched_bits, stream_word, buf, sizeof buf);
+        note(s, buf);
+    }
+    if (bits & kErrWatchdog) {
+        note(OHP_E_CUDA, "kernel watchdog: a pipeline barrier never completed");
+    } else if (bits != 0) {
+        std::snprintf(buf, sizeof buf, "device rejected chunk descriptor %u (%s)", first - 1,
+                      (bits & kErrInvalidDesc) ? "invalid" : "out of range");
+        note((bits & kErrInvalidDesc) ? OHP_E_INVALID_DESC : OHP_E_OUT_OF_RANGE, buf);
+    }
+    return fail(ctx, status, msg.c_str());
 }
 
 } // namespace ohp
@@ -620,6 +669,7 @@ int ohp_create(int device, ohp_context** out_ctx)
     OHP_CREATE(cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking));
     OHP_CREATE(cudaEventCreate(&ctx->ev_start));
     OHP_CREATE(cudaEventCreate(&ctx->ev_stop));
+    OHP_CREATE(cudaEventCreateWithFlags(&ctx->scratch_done, cudaEventDisableTiming));
     OHP_CREATE(cudaMalloc(reinterpret_cast<void**>(&ctx->d_table2), sizeof(uint16_t) * OHP_RAMP_TABLE_ENTRIES));
     OHP_CREATE(cudaMalloc(reinterpret_cast<void**>(&ctx->d_status), 16 * sizeof(uint32_t)));
     OHP_CREATE(cudaMallocHost(reinterpret_cast<void**>(&ctx->h_status), 16 * sizeof(uint32_t)));
@@ -666,6 +716,7 @@ int ohp_destroy(ohp_context* ctx)
     if (ctx->copy_in) (void)cudaStreamSynchronize(ctx->copy_in);
     if (ctx->stream) (void)cudaStreamSynchronize(ctx->stream);
     if (ctx->copy_out) (void)cudaStreamSynchronize(ctx->copy_out);
+    if (ctx->scratch_done) (void)cudaEventSynchronize(ctx->scratch_done); // the last call may have been on the caller's stream
     (void)cudaGetLastError();
     if (ctx->d_in) (void)cudaFree(ctx->d_in);
     if (ctx->d_out) (void)cudaFree(ctx->d_out);
@@ -684,6 +735,7 @@ int ohp_destroy(ohp_context* ctx)
     }
     if (ctx->sched_event) (void)cudaEventDestroy(ctx->sched_event);
     if (ctx->fly_event) (void)cudaEventDestroy(ctx->fly_event);
+    if (ctx->scratch_done) (void)cudaEventDestroy(ctx->scratch_done);
     if (ctx->h_status) (void)cudaFreeHost(ctx->h_status);
     if (ctx->ev_start) (void)cudaEventDestroy(ctx->ev_start);
     if (ctx->ev_stop) (void)cudaEventDestroy(ctx->ev_stop);
@@ -740,6 +792,8 @@ int ohp_process_host(ohp_context* ctx, const ohp_chunk_desc* h_descs, size_t n, 
         return fail(ctx, vrc, buf);
     }
     OHP_CUDA(ctx, cudaSetDevice(ctx->device));
+    const ScratchTurn turn(ctx, ctx->stream);
+    if (turn.rc != OHP_OK) return turn.rc;
     int rc;
     if ((rc = grow(ctx, ctx->d_in, ctx->d_in_cap, in_bytes + 16)) != OHP_OK) return rc;
     if ((rc = grow(ctx, ctx->d_out, ctx->d_out_cap, out_bytes + 16)) != OHP_OK) return rc;
@@ -1005,6 +1059,8 @@ static int run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, 
     if (n_streams == 0) return OHP_OK;
     if (!h_streams || !h_out || (!h_in && in_bytes) || (n_events && !h_events)) return fail(ctx, OHP_E_INVALID_ARG, "null host pointer");
     OHP_CUDA(ctx, cudaSetDevice(ctx->device));
+    const ScratchTurn turn(ctx, ctx->stream);
+    if (turn.rc != OHP_OK) return turn.rc;
     int rc;
     if ((rc = grow(ctx, ctx->d_specs, ctx->d_specs_cap, (uint64_t)n_streams * sizeof(ohp_stream_spec))) != OHP_OK) return rc;
     if ((rc = grow(ctx, ctx->d_events, ctx->d_events_cap, (uint64_t)(n_events ? n_events : 1) * sizeof(ohp_ramp_event))) != OHP_OK) return rc;
@@ -1248,6 +1304,8 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
     if (!d_streams || !d_out || (!d_in && in_bytes) || (n_events && !d_events)) return fail(ctx, OHP_E_INVALID_ARG, "null device pointer");
     OHP_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    const ScratchTurn turn(ctx, st);
+    if (turn.rc != OHP_OK) return turn.rc;
     int rc;
     if ((rc = grow(ctx, ctx->d_begin, ctx->d_begin_cap, (uint64_t)(n_streams + 1) * sizeof(uint64_t))) != OHP_OK) return rc;
     if ((rc = grow(ctx, ctx->d_counts, ctx->d_counts_cap, (uint64_t)n_streams * sizeof(uint64_t))) != OHP_OK) return rc;
@@ -1383,12 +1441,13 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
     OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_event));
     const uint32_t bits = ctx->h_status[2];
     if (bits != 0) {
-        const int src = schedule_status(ctx, st); // waits for ramp_convert_kernel too: the call has failed anyway
-        // a stream outgrew its region and none was refused for what it is (schedule_status reports those first): nothing
+        // waits for ramp_convert_kernel too (the call has failed anyway) and clears whatever that kernel reports beside the
+        // walk's refusal: the error is this call's, no later ohp_sync reports it again
+        const int src = read_status(ctx, st);
+        // a stream outgrew its region and none was refused for what it is (read_status reports those first): nothing
         // wrong with the batch, take the exact two-pass path
         const uint32_t refused = (1u << sched::kErrSpec) | (1u << sched::kErrAssert);
         if ((bits & (1u << sched::kErrBound)) && !(bits & refused)) {
-            (void)read_status(ctx, st);
             return finish(run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
                                                       d_stream_out_bytes, total_chunks, records, st, recent));
         }

@@ -256,16 +256,24 @@ def test_whole_stage_for_a_batch_resident_in_hbm(ctx, port, make):
         assert np.array_equal(got[mask], want[mask])
         assert (got[~mask] == 0x5A).all(), "bytes no chunk covers were written"
         if round_ == 0:
-            other = workloads.config5(n_streams=300, seconds=0.05)   # more chunks: the descriptor buffer has to grow
-            o_in = torch.zeros(other.in_bytes + 16, dtype=torch.uint8, device="cuda")
-            o_out = torch.zeros(other.out_bytes + 16, dtype=torch.uint8, device="cuda")
+            # more chunks: the walk into the existing buffer stops short, the buffer grows and the walk runs again
+            other = workloads.config5(n_streams=300, seconds=0.05)
+            o_inp = port.fill_pcm(other.in_bytes, other.seed)
+            rc, o_want, o_chunks, _ = port.run(other.streams, other.events, o_inp, other.out_bytes)
+            assert rc == 0
+            o_in = torch.from_numpy(np.concatenate([o_inp, np.zeros(16, np.uint8)])).cuda()
+            o_out = torch.full((other.out_bytes + 16,), 0x5A, dtype=torch.uint8, device="cuda")
             o_s = torch.from_numpy(other.streams.view(np.uint8).copy()).cuda()
             o_e = torch.from_numpy(other.events.view(np.uint8).copy()).cuda()
             torch.cuda.synchronize()
             n_other = ctx.run_streams_device(o_s.data_ptr(), len(other.streams), o_e.data_ptr(), len(other.events),
                                              o_in.data_ptr(), other.in_bytes, o_out.data_ptr(), other.out_bytes)
             ctx.sync()
-            assert n_other == len(capi.schedule_build(other.streams, other.events).chunks)
+            assert n_other == len(o_chunks)
+            o_got = o_out.cpu().numpy()[:other.out_bytes]
+            o_mask = covered_mask(o_chunks, other.out_bytes)
+            assert np.array_equal(o_got[o_mask], o_want[o_mask]), "bytes of the batch that regrew the descriptor buffer"
+            assert (o_got[~o_mask] == 0x5A).all()
             d_out.fill_(0x5A)
             torch.cuda.synchronize()
 
