@@ -95,7 +95,7 @@ typedef struct ohp_chunk_desc {
     uint16_t ramp_end;    /* Ramp::iEnd,   0..16384                                                        */
     uint16_t attenuation; /* MsgPlayablePcm::iAttenuation; 256 = unity; !=256 requires bit_depth 16        */
     uint8_t  bit_depth;   /* 8, 16, 24, 32                                                                 */
-    uint8_t  channels;    /* 1..32 (DecodedAudio::kMaxNumChannels is 8; silence is exercised at 10)        */
+    uint8_t  channels;    /* 1..32 (DecodedAudio::kMaxNumChannels is 8; every sink and mode is tested at 1..32) */
     uint8_t  flags;       /* OHP_F_*                                                                       */
     uint8_t  out_fmt;     /* ohp_out_fmt                                                                   */
     uint16_t aux;         /* per-format parameter, see ohp_out_fmt                                         */
