@@ -72,12 +72,15 @@ int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, siz
  *     ramp + convert kernel), report a stream the walk refuses here instead of at the next ohp_sync, and -- should a
  *     stream ever have more playables than its region holds (none of this repo's generators produces one; the bound is
  *     held against exact counts in the tests) -- redo the batch through count + emit.  Without it that case is an
- *     OHP_E_NO_MEMORY from the next ohp_sync.
+ *     OHP_E_NO_MEMORY from the next ohp_sync naming the lowest such stream; such a stream writes no byte of d_out and
+ *     reports 0 in d_stream_out_bytes, the other streams' bytes and sizes are exact.  A call that asks for the total
+ *     after such a call on another stream finishes its own work and then returns that call's OHP_E_NO_MEMORY.
  * Calls on one context may follow one another on any streams without an ohp_sync in between: a call that uses the
  * context's scratch (this one, its flywheel variants, ohp_process_host, ohp_run_streams_host) waits on the device for
  * the previous such call's work.  One host thread at a time per context.  The status block is the context's: when the
  * work of two calls on two streams fails at once, the first ohp_sync of either reports both.
- * Environment (tests): OHP_ONE_WALK=0 takes count + scan + emit.
+ * Environment (tests): OHP_ONE_WALK=0 takes count + scan + emit.  OHP_REGION_CAP=n gives no stream a region of more
+ * than n descriptors, so that the streams with more than n playables outgrow theirs (both read on every call).
  * Errors as ohp_run_streams_host.
  */
 int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,

@@ -1174,7 +1174,8 @@ int ohp_run_streams_host(ohp_context* ctx, const ohp_stream_spec* h_streams, siz
 // a playable MsgPlayable::Read does nothing for, and costs ramp_convert_kernel a record and a ticket).  No count pass, and
 // the only host round trip is for the regions' total (bound + scan are a few microseconds of GPU time).
 // A stream that outgrows its region (none of the shapes this repo generates does, the bound is held against the exact
-// counts in tests/test_schedule_walk.py) sends the whole call through the two-pass path.
+// counts in tests/test_schedule_walk.py and tests/test_chunk_bound.py) sends the whole call through the two-pass path;
+// tests/test_gpu_region_overflow.py makes streams outgrow regions capped by OHP_REGION_CAP.
 // records (ohp_run_streams_device_flywheel): the emitting walk also leaves the starvation records there; with recent
 // (ohp_run_streams_device_flywheel_recent) their pieces of recent audio too.
 static int run_streams_device_two_pass(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,
@@ -1344,13 +1345,16 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
         fly = &flyArgs;
     }
     const sched::RecentOut* recent = fly && fly->with_recent ? &fly->recent : nullptr;
+    const char* cap_env = std::getenv("OHP_REGION_CAP"); // OHP_REGION_CAP=n: regions of at most n descriptors (tests)
+    const uint64_t region_cap = cap_env ? std::strtoull(cap_env, nullptr, 10) : ~0ull;
     auto bound = [&]() -> int { // regions: bound per stream (and, with fly, the flywheel slots)
         if (fly) {
             sched::bound_slots_kernel<<<(unsigned)((n_streams + 127) / 128), 128, 0, st>>>(d_streams, n_streams, d_events, n_events, ctx->d_begin,
-                                                                                        ctx->d_slot, ctx->d_owner, ctx->d_fly_slots);
+                                                                                        ctx->d_slot, ctx->d_owner, ctx->d_fly_slots, region_cap);
         }
         else {
-            sched::bound_kernel<<<(unsigned)((n_streams + 127) / 128), 128, 0, st>>>(d_streams, n_streams, d_events, n_events, ctx->d_begin);
+            sched::bound_kernel<<<(unsigned)((n_streams + 127) / 128), 128, 0, st>>>(d_streams, n_streams, d_events, n_events, ctx->d_begin,
+                                                                                  region_cap);
         }
         OHP_CUDA(ctx, cudaGetLastError());
         return OHP_OK;
@@ -1419,9 +1423,12 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
     OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_event));
     const uint64_t regions = *ctx->h_regions;
     if (fly && (rc = fly_check(ctx, *fly)) != OHP_OK) return rc;
-    if (regions > ctx->d_descs_cap / sizeof(ohp_chunk_desc)) {
+    // (at least one descriptor: with none, regions that add up to 0 -- every stream refused, or outgrowing a region of 0 --
+    //  would leave the walk unlaunched, and what it reports unreported)
+    const uint64_t need = regions ? regions : 1;
+    if (need > ctx->d_descs_cap / sizeof(ohp_chunk_desc)) {
         OHP_CUDA(ctx, cudaDeviceSynchronize()); // the buffer may still be read by a launch enqueued earlier on another stream
-        if ((rc = grow(ctx, ctx->d_descs, ctx->d_descs_cap, regions * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
+        if ((rc = grow(ctx, ctx->d_descs, ctx->d_descs_cap, need * sizeof(ohp_chunk_desc))) != OHP_OK) return rc;
         if ((rc = walk()) != OHP_OK) return rc;
     }
     if (fly) {
@@ -1440,6 +1447,13 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
     if (!total_chunks) return finish(OHP_OK);
     OHP_CUDA(ctx, cudaEventSynchronize(ctx->sched_event));
     const uint32_t bits = ctx->h_status[2];
+    uint64_t total = 0;
+    bool outgrown = false; // a stream of THIS call outgrew its region (the status bit may be an earlier call's)
+    for (size_t s = 0; s < n_streams; s++) {
+        outgrown |= ctx->h_outb[s] == sched::kOutgrown;
+        total += ctx->h_outb[s];
+    }
+    int earlier = OHP_OK;
     if (bits != 0) {
         // waits for ramp_convert_kernel too (the call has failed anyway) and clears whatever that kernel reports beside the
         // walk's refusal: the error is this call's, no later ohp_sync reports it again
@@ -1447,16 +1461,18 @@ static int run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams
         // a stream outgrew its region and none was refused for what it is (read_status reports those first): nothing
         // wrong with the batch, take the exact two-pass path
         const uint32_t refused = (1u << sched::kErrSpec) | (1u << sched::kErrAssert);
-        if ((bits & (1u << sched::kErrBound)) && !(bits & refused)) {
+        if (outgrown && !(bits & refused)) {
             return finish(run_streams_device_two_pass(ctx, d_streams, n_streams, d_events, n_events, d_in, in_bytes, d_out, out_bytes,
                                                       d_stream_out_bytes, total_chunks, records, st, recent));
         }
-        if (src != OHP_OK) return src;
+        // only an earlier call without the total outgrew a region: this call's work is whole, and reports that error
+        // once it is done (as that call's ohp_sync would have)
+        if (bits != (1u << sched::kErrBound)) return src;
+        earlier = src;
     }
-    uint64_t total = 0;
-    for (size_t s = 0; s < n_streams; s++) total += ctx->h_outb[s];
     *total_chunks = total;
-    return finish(OHP_OK);
+    rc = finish(OHP_OK);
+    return rc != OHP_OK ? rc : earlier;
 }
 
 int ohp_run_streams_device(ohp_context* ctx, const ohp_stream_spec* d_streams, size_t n_streams,

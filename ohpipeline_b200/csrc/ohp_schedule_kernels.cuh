@@ -30,21 +30,26 @@ struct ScheduleParams
     ohp_chunk_info* info;      // EMIT, may be null
     uint32_t* status;          // [0] error bits (1 << code), [1] 0xffffffff - lowest failing stream (atomicMax; 0 = none)
     // ONE-WALK mode (regions from stream_chunk_bound): EMIT also reports what COUNT would have, and fills each region's tail
-    uint64_t* counts_out;      // [n_streams] exact playables per stream (null: two-pass mode)
+    uint64_t* counts_out;      // [n_streams] exact playables per stream, kOutgrown for one that outgrew its region, 0 for one
+                               // refused (null: two-pass mode)
     uint64_t descs_cap;        // descriptors the buffer holds; a stream whose region would end beyond writes nothing (0: no check)
     uint32_t lanes_per_warp;   // TEAM = 1: streams a warp walks (its first lanes, one each; the others idle); 0 = 32
     ohp_starvation* records;   // schedule_record_kernel: [n_events], the record of event e at [e]
 };
 
 constexpr uint32_t kErrBound = 4u; // a stream has more playables than stream_chunk_bound allowed for: the caller takes two passes
+constexpr uint64_t kOutgrown = ~0ull; // counts_out of such a stream: tells this call's overflow from an earlier call's status bit
 
 // Regions for the one-walk mode: bound[s] playables at most for stream s (scanned into region offsets afterwards).
+// cap: at most this many (~0 but for tests, which make chosen streams outgrow their regions: OHP_REGION_CAP).
 __global__ void __launch_bounds__(128) bound_kernel(const ohp_stream_spec* __restrict__ streams, uint64_t n_streams,
-                                                    const ohp_ramp_event* __restrict__ events, uint64_t n_events, uint64_t* __restrict__ bound)
+                                                    const ohp_ramp_event* __restrict__ events, uint64_t n_events, uint64_t* __restrict__ bound,
+                                                    uint64_t cap)
 {
     const uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_streams) return;
-    bound[s] = stream_chunk_bound(streams[s], events, n_events);
+    const uint64_t b = stream_chunk_bound(streams[s], events, n_events);
+    bound[s] = b < cap ? b : cap;
 }
 
 
@@ -98,8 +103,9 @@ __device__ __forceinline__ void schedule_body(const ScheduleParams p, ohp_recent
         if (p.out_bytes) p.out_bytes[s] = outBytes;
     }
     else if (regions) {
-        p.counts_out[s] = rc == kOk ? nChunks : 0;
-        if (p.out_bytes) p.out_bytes[s] = outBytes;
+        // (an outgrown stream wrote no byte: 0 output bytes)
+        p.counts_out[s] = rc == kOk ? nChunks : (rc == kErrBound ? kOutgrown : 0);
+        if (p.out_bytes) p.out_bytes[s] = rc == kOk ? outBytes : 0;
     }
 }
 
@@ -156,12 +162,13 @@ OHP_HD uint64_t fly_slot_bytes(const ohp_stream_spec& sp)
 __global__ void __launch_bounds__(128) bound_slots_kernel(const ohp_stream_spec* __restrict__ streams, uint64_t n_streams,
                                                           const ohp_ramp_event* __restrict__ events, uint64_t n_events,
                                                           uint64_t* __restrict__ bound, uint64_t* __restrict__ slot,
-                                                          uint32_t* __restrict__ owner, FlySlots* __restrict__ slots)
+                                                          uint32_t* __restrict__ owner, FlySlots* __restrict__ slots, uint64_t cap)
 {
     const uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_streams) return;
     const ohp_stream_spec sp = streams[s];
-    bound[s] = stream_chunk_bound(sp, events, n_events);
+    const uint64_t b = stream_chunk_bound(sp, events, n_events);
+    bound[s] = b < cap ? b : cap;
     const uint64_t first = sp.first_event;
     const uint64_t end = first + sp.num_events < n_events ? first + sp.num_events : n_events;
     const uint64_t size = fly_slot_bytes(sp);
